@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- edges/sec of the K-layer credibility-weighted LightGCN training step on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one full training step of the reference loop (lightgcn_cu.py:608-654 /
 Version-2/lighgcn_cu_pop.py:826-866) on one batch of 4096 users: on-device triple sampling, K-layer forward, fused
@@ -45,6 +45,8 @@ def parse():
     ap.add_argument("--no-flush", action="store_true", help="do not flush L2 between timed steps")
     ap.add_argument("--hot-mb", type=float, default=None,
                     help="MiB of hot (high-degree) rows the SpMM keeps L2-resident (default: CredGraph.HOT_BYTES)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (one GPU only)")
     return ap.parse_args()
 
 
@@ -294,7 +296,30 @@ def traffic_per_step(name):
     return float(j["bytes_per_step"]), j.get("source")
 
 
-def run_single(args, name, dev, steps, warmup, clocks, with_cpu, with_extras):
+DUMP_ROWS = 8192        # rows kept of each table: 6 tables x 8192 rows x d = 128 x 4 B = 25 MB per workload at most
+
+
+def dump_last_step(out_dir, prefix, loss, step):
+    """--dump-outputs: what the last timed TrainStep.step() computed, as float32 .npy files that two builds can be
+    compared by -- the loss it returned, the embedding tables Adam updated in place, and the final embeddings and
+    gradients it leaves on the step and the parameters.  Tables longer than DUMP_ROWS rows are cut to the same seeded
+    sample of rows in every run."""
+    out = pathlib.Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / f"{prefix}loss.npy", loss.detach().float().reshape(1).cpu().numpy())
+    m = step.model
+    for side, emb, final in (("user", m.user_emb.weight, step.f_u), ("item", m.item_emb.weight, step.f_i)):
+        n = emb.shape[0]
+        rows = None
+        if n > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+            rows = torch.from_numpy(rows).to(emb.device)
+        for what, t in (("emb", emb), ("final", final), ("grad", emb.grad)):
+            t = t.detach() if rows is None else t.detach().index_select(0, rows)
+            np.save(out / f"{prefix}{side}_{what}.npy", t.float().cpu().numpy())
+
+
+def run_single(args, name, dev, steps, warmup, clocks, with_cpu, with_extras, dump_prefix=None):
     from credgcn import _lib, graph, model, sampler, synth
     shp = synth.SHAPES[name]
     t0 = time.time()
@@ -358,10 +383,12 @@ def run_single(args, name, dev, steps, warmup, clocks, with_cpu, with_extras):
             if not args.no_flush:
                 flush_buf.fill_(s & 0xff)
             starts[s].record()
-            step.step(dev_batches[s % n_batches])
+            loss_dev = step.step(dev_batches[s % n_batches])
             ends[s].record()
         torch.cuda.synchronize()
         step_ms = [a.elapsed_time(b) for a, b in zip(starts, ends)]
+        if dump_prefix is not None:
+            dump_last_step(args.dump_outputs, dump_prefix, loss_dev, step)
         # (b) `e2e`: the same call with PINNED HOST batches -- H2D of the batch, replay, D2H of the loss, every step
         for s in range(2):
             float(step.step(pinned[s % n_batches]).item())
@@ -539,6 +566,10 @@ def extras_small(args, sg, shp, gr, net, dev):
 
 def main():
     args = parse()
+    if args.dump_outputs is not None and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        raise SystemExit("--dump-outputs writes the training step of --impl ours on one GPU")
+    if args.dump_outputs is not None and args.steps < 1:
+        raise SystemExit("--dump-outputs writes the last timed step: it needs --steps 1 or more")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -562,11 +593,13 @@ def main():
     if name == "C5":
         print("[bench] C5 on ONE GPU: 50M x 10M x 1B edges needs ~165 GB of the 180 GB", file=sys.stderr)
     clocks = ClockSampler(local)
+    dump = args.dump_outputs is not None
     line = run_single(args, name, dev, args.steps, args.warmup, clocks, with_cpu=not args.no_cpu_baseline,
-                      with_extras=True)
+                      with_extras=True, dump_prefix="" if dump else None)
     if args.workload is None and not args.no_extra:
         # the L2-resident BASELINE config (configs[1]) measured the same way, as an extra object
-        c2 = run_single(args, "C2", dev, max(args.steps, 50), args.warmup, clocks, with_cpu=False, with_extras=True)
+        c2 = run_single(args, "C2", dev, args.steps, args.warmup, clocks, with_cpu=False, with_extras=True,
+                        dump_prefix="c2_" if dump else None)
         line["c2"] = {k: c2[k] for k in ("value", "unit", "ms_per_step", "config", "e2e", "roofline", "phases_ms",
                                          "graph_build_ms", "steps_per_epoch", "epoch_ms", "epoch_ms_kind",
                                          "eval_full_rank", "torch_gpu_baseline", "train_edges") if k in c2}

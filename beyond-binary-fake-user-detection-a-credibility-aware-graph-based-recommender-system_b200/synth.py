@@ -241,8 +241,8 @@ def make_graph_device(name: str = "C4", device="cuda", *, num_users=None, num_it
     n = edges.shape[1]
     n_tr, n_va = int(n * split[0]), int(n * split[1])
 
-    g1 = torch._standard_gamma(torch.where(is_fake, 1.0, 5.0).to(torch.float32))
-    g2 = torch._standard_gamma(torch.where(is_fake, 8.0, 2.0).to(torch.float32))
+    g1 = torch._standard_gamma(torch.where(is_fake, 1.0, 5.0).to(torch.float32), generator=gen)
+    g2 = torch._standard_gamma(torch.where(is_fake, 8.0, 2.0).to(torch.float32), generator=gen)
     cred = (g1 / (g1 + g2)).clamp(0.0, 1.0).to(torch.float32)
     cred[0], cred[-1] = 1.0, 0.0
     return SynthGraph(name=name, num_users=U, num_items=I, train_edges=edges[:, :n_tr].contiguous(),

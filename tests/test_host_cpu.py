@@ -73,6 +73,12 @@ def test_synthetic_generator_is_seeded_and_shaped():
     assert abs(a.is_fake.mean() - 0.05) < 0.01
     assert a.cred[a.is_fake].mean() < a.cred[~a.is_fake].mean()           # fake users are the low-credibility ones
     assert not np.array_equal(synth.make_graph("C1", seed=1).train_edges, a.train_edges)
+    # the torch generator of the C4 / C5 shapes is seeded in the same way, credibilities included
+    import torch
+    da, db = (synth.make_graph_device("C4", "cpu", num_users=20_000, num_items=4_000, num_edges=100_000)
+              for _ in range(2))
+    for k in ("train_edges", "val_edges", "test_edges", "cred", "is_fake"):
+        assert torch.equal(getattr(da, k), getattr(db, k)), k
 
 
 def test_metric_assembly_from_device_sums_equals_host_metrics():

@@ -223,6 +223,65 @@ def train_step_grads(ops, e0_u, e0_i, users, pos, neg, num_layers, order, reg_we
     return loss, (b_u + d_e0u).astype(F32), (b_i + d_e0i).astype(F32), f_u, f_i
 
 
+def bpr_rows_f64(f_u, f_i, e0_u, e0_i, users, pos, neg, reg_weight, fair_weight=0.0, pop=None, batch_total=0):
+    """The fused loss of `bpr_loss` in float64 throughout, with the means over `batch_total` triples (a shard of a
+    larger batch; 0 = len(users)).  Besides the loss and d f_u / d f_i it returns, per gradient element, the sum of
+    the absolute values of the terms that make it up (S_u, S_i): the scale an fp32 sum of those terms is accurate
+    to, row by row, whatever the other rows hold.  `mult_u` / `mult_i`: how many plan entries each row has (the
+    L2 gradient of a row is mult * 2 reg / batch_total * e0)."""
+    users, pos, neg = (np.asarray(x, np.int64) for x in (users, pos, neg))
+    Bt = float(batch_total or len(users))
+    fu, fp, fn = (np.asarray(x, np.float64) for x in (f_u[users], f_i[pos], f_i[neg]))
+    y_pos, y_neg = (fu * fp).sum(1), (fu * fn).sum(1)
+    sig = 1.0 / (1.0 + np.exp(-(y_pos - y_neg)))
+    pw = fair_weight * np.asarray(pop, np.float64)[pos] if (pop is not None and fair_weight) else np.zeros(len(users))
+    l2 = sum((np.asarray(e[r], np.float64) ** 2).sum(1) for e, r in ((e0_u, users), (e0_i, pos), (e0_i, neg)))
+    terms = -np.log(sig + 1e-12) + pw * y_pos + reg_weight * l2
+    gx = -(sig * (1.0 - sig)) / (sig + 1e-12) / Bt
+    cp, cn = gx + pw / Bt, -gx
+    d_fu, s_u = np.zeros(f_u.shape), np.zeros(f_u.shape)
+    d_fi, s_i = np.zeros(f_i.shape), np.zeros(f_i.shape)
+    for d, s, rows, a, b in ((d_fu, s_u, users, cp[:, None] * fp, cn[:, None] * fn), (d_fi, s_i, pos, cp[:, None] * fu, 0),
+                             (d_fi, s_i, neg, cn[:, None] * fu, 0)):
+        np.add.at(d, rows, a + b)
+        np.add.at(s, rows, np.abs(a) + np.abs(b))
+    mult_u = np.bincount(users, minlength=f_u.shape[0])
+    mult_i = np.bincount(pos, minlength=f_i.shape[0]) + np.bincount(neg, minlength=f_i.shape[0])
+    return dict(loss=float(terms.sum() / Bt), loss_abs=float(np.abs(terms).sum() / Bt), d_fu=d_fu, d_fi=d_fi,
+                s_u=s_u, s_i=s_i, mult_u=mult_u, mult_i=mult_i)
+
+
+# --------------------------------------------------------------------------------------
+# Adam (torch.optim.Adam defaults: no weight decay, no amsgrad) and a multi-step driver
+# --------------------------------------------------------------------------------------
+def adam_step_f64(p, g, m, v, t, lr=1e-3, betas=(0.9, 0.999), eps=1e-8):
+    """Step t (1-based) of torch.optim.Adam in float64 on one table; returns the new (p, m, v)."""
+    b1, b2 = betas
+    g = np.asarray(g, np.float64)
+    m = b1 * m + (1.0 - b1) * g
+    v = b2 * v + (1.0 - b2) * g * g
+    step = lr / (1.0 - b1 ** t) * m / (np.sqrt(v) / math.sqrt(1.0 - b2 ** t) + eps)
+    return np.asarray(p, np.float64) - step, m, v
+
+
+def train_steps(ops, e0_u, e0_i, batches, num_layers, order, reg_weight, fair_weight=0.0, pop=None, lr=1e-3):
+    """Reference for a run of training steps (CU:608-652 repeated): per (users, pos, neg) batch, loss and gradients
+    from `train_step_grads` at the current parameters, then `adam_step_f64` on both tables.  The parameters are
+    rounded to float32 after every step, as the stored tables are.  Returns one dict per step: the loss, the
+    gradients and the parameters after the step."""
+    p = [np.array(e0_u, F32), np.array(e0_i, F32)]
+    mv = [[np.zeros(x.shape), np.zeros(x.shape)] for x in p]
+    out = []
+    for t, (users, pos, neg) in enumerate(batches, start=1):
+        loss, g_u, g_i, _, _ = train_step_grads(ops, p[0], p[1], users, pos, neg, num_layers, order, reg_weight,
+                                                fair_weight, pop)
+        for k, g in enumerate((g_u, g_i)):
+            q, mv[k][0], mv[k][1] = adam_step_f64(p[k], g, mv[k][0], mv[k][1], t, lr)
+            p[k] = q.astype(F32)
+        out.append(dict(loss=loss, g_u=g_u, g_i=g_i, p_u=p[0].copy(), p_i=p[1].copy()))
+    return out
+
+
 # --------------------------------------------------------------------------------------
 # a12 / a13 / a14. samplers (sequential, NumPy Generator -- same draw order as the reference)
 # --------------------------------------------------------------------------------------

@@ -262,6 +262,7 @@ __global__ void __launch_bounds__(SP_THREADS, MINB) k_spmm(const int32_t* __rest
                                                            float4* ACC_OUT, float acc_scale, float4* partial,
                                                            const uint8_t* __restrict__ nz,
                                                            const uint8_t* __restrict__ acc_nz,
+                                                           const uint8_t* __restrict__ out_rows,
                                                            const int4* __restrict__ work, const SpmmPush ps_in) {
   // PUSH = false: a compile-time "off", so that the ordinary instantiations carry no trace of the push path
   const SpmmPush ps = PUSH ? ps_in : SpmmPush{0ull, 0, 0};
@@ -289,6 +290,14 @@ __global__ void __launch_bounds__(SP_THREADS, MINB) k_spmm(const int32_t* __rest
     wf = ld_val<HOT>(val + lane);
   }
   asm volatile("griddepcontrol.wait;" ::: "memory");
+  // out_rows (nullable; written by an earlier kernel, so read after the wait): a row with out_rows[row] == 0 is not
+  // computed and none of its outputs is written.  Every chunk of a long row reads the same flag, so either all of
+  // them arrive or none does, and the arrival counter stays 0 between launches.  Only the row-sparse (NZ) products
+  // take a mask (spmm_dispatch): in the other instantiations the check would cost registers at the 64-register cap
+  // (-Xptxas -v: spills in the d = 64 and d = 128 gather loops).
+  if (NZ && !PUSH && out_rows != nullptr &&
+      __ldg(out_rows + (item >= sc.n_chunks ? wd.w : __ldg(sc.perm + wd.w))) == 0)
+    return;
   gather_batches<G, V, UNR, NZ, HOT>(idx, val, wd.z, X, lane, mask, cf, wf, acc, nz);
   if (item >= sc.n_chunks) {
     // (loading ACC_IN[row] before the gathers, to take it off the dependency chain, was measured SLOWER: the
@@ -323,11 +332,13 @@ template <int G, int V>
 __global__ void __launch_bounds__(SP_THREADS) k_spmm_finish(SpmmSched sc, const float4* __restrict__ partial,
                                                             float4* __restrict__ Y, const float4* ACC_IN,
                                                             float4* ACC_OUT, float acc_scale,
-                                                            const uint8_t* __restrict__ acc_nz, const SpmmPush ps) {
+                                                            const uint8_t* __restrict__ acc_nz,
+                                                            const uint8_t* __restrict__ out_rows, const SpmmPush ps) {
   constexpr int GROUPS = SP_THREADS / G;
   constexpr int ROW4 = G * V;
   __shared__ float4 red[GROUPS][ROW4];
   const int k = blockIdx.x;
+  if (out_rows != nullptr && __ldg(out_rows + __ldg(sc.perm + k)) == 0) return;   // the whole CTA: row not computed
   const int lane = threadIdx.x & (G - 1), grp = threadIdx.x / G;
   const int c0 = __ldg(sc.chunk_ptr + k), c1 = __ldg(sc.chunk_ptr + k + 1);
   float4 acc[V];
@@ -376,7 +387,8 @@ static int row_flags(const float* X, int64_t n_rows, int32_t d, uint8_t* flags, 
 template <int G, int V, int UNR, int MINB, bool NZ, bool PUSH, bool HOT>
 static int launch_spmm(const cgx_csr* m, const float* val, const float* X, float* Y, const float* ACC_IN,
                        float* ACC_OUT, float acc_scale, void* workspace, size_t workspace_bytes,
-                       cudaStream_t stream, const uint8_t* nz, const uint8_t* acc_nz, const SpmmPush ps) {
+                       cudaStream_t stream, const uint8_t* nz, const uint8_t* acc_nz, const uint8_t* out_rows,
+                       const SpmmPush ps) {
   constexpr int GROUPS = SP_THREADS / G;
   float4* partial = nullptr;
   if (m->n_long > 0) {
@@ -400,18 +412,18 @@ static int launch_spmm(const cgx_csr* m, const float* val, const float* X, float
   CGX_CUDA(cudaLaunchKernelEx(&cfg, k_spmm<G, V, UNR, MINB, NZ, PUSH, HOT>, HOT ? m->idx_hint : m->idx, val, items, sc,
                               reinterpret_cast<const float4*>(X), reinterpret_cast<float4*>(Y),
                               reinterpret_cast<const float4*>(ACC_IN), reinterpret_cast<float4*>(ACC_OUT), acc_scale,
-                              partial, nz, acc_nz, static_cast<const int4*>(m->work), ps));
+                              partial, nz, acc_nz, out_rows, static_cast<const int4*>(m->work), ps));
   CGX_LAUNCH_CHECK();
   if (m->n_huge > 0) {
     k_spmm_finish<G, V><<<(unsigned)m->n_huge, SP_THREADS, 0, stream>>>(
         sc, partial, reinterpret_cast<float4*>(Y), reinterpret_cast<const float4*>(ACC_IN),
-        reinterpret_cast<float4*>(ACC_OUT), acc_scale, acc_nz, ps);
+        reinterpret_cast<float4*>(ACC_OUT), acc_scale, acc_nz, out_rows, ps);
     CGX_LAUNCH_CHECK();
   }
   return CGX_OK;
 }
 
-#define CGX_SPMM_ARGS m, val, X, Y, ACC_IN, ACC_OUT, acc_scale, ws, ws_bytes, stream, nz, acc_nz, ps
+#define CGX_SPMM_ARGS m, val, X, Y, ACC_IN, ACC_OUT, acc_scale, ws, ws_bytes, stream, nz, acc_nz, out_rows, ps
 
 // Group geometry by regime (profiles/r1_spmm_variants.txt; the sweep itself lives in the round-1 history).
 // Gathered table in L2 (C2/C3: latency-bound): d/4 lanes per row, one float4 per lane, 8 gathers in flight.
@@ -422,7 +434,8 @@ static int launch_spmm(const cgx_csr* m, const float* val, const float* X, float
 template <int G, int V, int UNR>
 static int spmm_flavour(const cgx_csr* m, const float* val, const float* X, float* Y, const float* ACC_IN,
                         float* ACC_OUT, float acc_scale, void* ws, size_t ws_bytes, cudaStream_t stream,
-                        const uint8_t* nz, const uint8_t* acc_nz, const SpmmPush ps, bool hot) {
+                        const uint8_t* nz, const uint8_t* acc_nz, const uint8_t* out_rows, const SpmmPush ps,
+                        bool hot) {
   const bool push = ps.rows_per > 0;
   if constexpr (V == 2) {
     if (hot && nz == nullptr) {
@@ -438,16 +451,18 @@ static int spmm_flavour(const cgx_csr* m, const float* val, const float* X, floa
   return launch_spmm<G, V, UNR, 4, false, false, false>(CGX_SPMM_ARGS);
 }
 
-#define CGX_FLAVOUR_ARGS m, val, X, Y, ACC_IN, ACC_OUT, acc_scale, ws, ws_bytes, stream, nz, acc_nz, ps, hot
+#define CGX_FLAVOUR_ARGS m, val, X, Y, ACC_IN, ACC_OUT, acc_scale, ws, ws_bytes, stream, nz, acc_nz, out_rows, ps, hot
 
 static int spmm_dispatch(const cgx_csr* m, int use_bwd, int32_t d, const float* X, float* Y, const float* ACC_IN,
                          float* ACC_OUT, float acc_scale, void* ws, size_t ws_bytes, cudaStream_t stream,
                          const uint8_t* nz = nullptr, const SpmmPush ps = SpmmPush{0ull, 0, 0},
-                         const uint8_t* acc_nz = nullptr) {
+                         const uint8_t* acc_nz = nullptr, const uint8_t* out_rows = nullptr) {
   CGX_REQUIRE(m && m->perm && m->work && (m->nnz == 0 || (m->idx && m->val_fwd && m->val_bwd)) && X, CGX_ERR_ARG,
               "spmm: NULL pointer (cgx_csr needs idx, both value arrays and the cgx_row_schedule* outputs)");
   CGX_REQUIRE(m->n_long == 0 || (m->chunk_ptr && m->arrive), CGX_ERR_ARG, "spmm: chunk tables missing");
   CGX_REQUIRE(Y || ACC_OUT || ps.rows_per > 0, CGX_ERR_ARG, "spmm: no output requested");
+  CGX_REQUIRE(out_rows == nullptr || (nz != nullptr && ps.rows_per == 0), CGX_ERR_ARG,
+              "spmm: an output-row mask needs gather flags and no push mode");
   const float* val = use_bwd ? m->val_bwd : m->val_fwd;
   if (m->n_rows == 0) return CGX_OK;
   const bool beyond_l2 = int64_t(m->n_cols) * int64_t(d) * 4 > option(CGX_OPT_L2_TABLE_BYTES);
@@ -565,6 +580,40 @@ extern "C" int cgx_row_flags(const float* X, int64_t n_rows, int32_t d, uint8_t*
   return row_flags(X, n_rows, d, flags, static_cast<cudaStream_t>(stream));
 }
 
+// Item frontier of a triple batch: flags[i] = 1 for i in pos, neg and the by_user rows of the batch users.  One warp
+// per triple; duplicate users walk their row twice (the stores are idempotent).  Out-of-range ids are clamped to 0,
+// as cgx_bpr_plan does, so the frontier covers every row that cgx_bpr_mark_rows flags.
+__device__ __forceinline__ int64_t clamp_row(int64_t x, int64_t n) { return (x < 0 || x >= n) ? 0 : x; }
+__global__ void k_batch_frontier(const int64_t* __restrict__ indptr, const int32_t* __restrict__ idx,
+                                 const int64_t* __restrict__ users, const int64_t* __restrict__ pos,
+                                 const int64_t* __restrict__ neg, int64_t B, int32_t U, int32_t I,
+                                 uint8_t* __restrict__ flags) {
+  const int64_t t = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) / 32;
+  const int lane = threadIdx.x & 31;
+  if (t >= B) return;
+  if (lane == 0) {
+    flags[clamp_row(pos[t], I)] = 1;
+    flags[clamp_row(neg[t], I)] = 1;
+  }
+  const int64_t u = clamp_row(users[t], U);
+  const int64_t end = indptr[u + 1];
+  for (int64_t j = indptr[u] + lane; j < end; j += 32) flags[idx[j]] = 1;
+}
+
+extern "C" int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64_t* pos,
+                                  const int64_t* neg, int64_t B, uint8_t* flags_i, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  CGX_REQUIRE(by_user && by_user->indptr && (by_user->nnz == 0 || by_user->idx) && users && pos && neg && flags_i,
+              CGX_ERR_ARG, "batch_frontier: NULL pointer");
+  CGX_REQUIRE(B > 0 && B < (int64_t(1) << 29) && by_user->n_rows > 0 && by_user->n_cols > 0, CGX_ERR_ARG,
+              "batch_frontier: bad batch size %lld or empty graph", (long long)B);
+  CGX_CUDA(cudaMemsetAsync(flags_i, 0, size_t(by_user->n_cols), stream));
+  k_batch_frontier<<<(unsigned)ceil_div(B * 32, 256), 256, 0, stream>>>(
+      by_user->indptr, by_user->idx, users, pos, neg, B, by_user->n_rows, by_user->n_cols, flags_i);
+  CGX_LAUNCH_CHECK();
+  return CGX_OK;
+}
+
 // Layer buffers: the Jacobi order reads layer k of BOTH sides while it writes layer k + 1, so it needs two buffers
 // per side; in Gauss-Seidel order every buffer is dead by the time it is overwritten (the item product reads u_k
 // and writes i_{k+1}, the user product reads i_{k+1} and writes u_{k+1}), so one per side is enough -- 15 GB less
@@ -649,6 +698,14 @@ extern "C" int cgx_propagate_bwd_flagged(const cgx_csr* by_user, const cgx_csr* 
                                          int32_t d, const float* g_u, const float* g_i, const uint8_t* g_u_rows,
                                          const uint8_t* g_i_rows, float* d_e0_u, float* d_e0_i, void* workspace,
                                          size_t workspace_bytes, void* stream_) {
+  return cgx_propagate_bwd_frontier(by_user, by_item, order, K, d, g_u, g_i, g_u_rows, g_i_rows, nullptr, d_e0_u,
+                                    d_e0_i, workspace, workspace_bytes, stream_);
+}
+
+extern "C" int cgx_propagate_bwd_frontier(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t K,
+                                          int32_t d, const float* g_u, const float* g_i, const uint8_t* g_u_rows,
+                                          const uint8_t* g_i_rows, const uint8_t* front_i, float* d_e0_u,
+                                          float* d_e0_i, void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE((g_u_rows == nullptr) == (g_i_rows == nullptr), CGX_ERR_ARG,
               "propagate_bwd_flagged: pass both row-flag arrays or neither");
@@ -682,6 +739,11 @@ extern "C" int cgx_propagate_bwd_flagged(const cgx_csr* by_user, const cgx_csr* 
   // Work with the unscaled adjoints bu' = bu / s, bi' = bi / s (the recurrences are linear):
   //   Jacobi: (bu', bi') <- (g_u + C^T bi', g_i + A^T bu');  Gauss-Seidel: bi' = g_i + A^T bu'; bu' = g_u + C^T bi'
   // and fold s into the last product's epilogue.
+  // Item frontier (front_i, nullable): the first item-side adjoint g_i + A^T g_u is non-zero only on front_i.  When
+  // that product writes scratch, it computes only the rows of front_i, and the one product that gathers it skips
+  // every other row.  Invariant: every row outside front_i of the masked buffer is stale and is never read.  No
+  // product that writes d_e0_u / d_e0_i is masked.  (A mask needs the row-sparse first product: spmm_dispatch.)
+  const uint8_t* front = sparse ? front_i : nullptr;
   if (order == CGX_ORDER_JACOBI) {
     const float* bu = g_u;
     const float* bi = g_i;
@@ -696,10 +758,12 @@ extern "C" int cgx_propagate_bwd_flagged(const cgx_csr* by_user, const cgx_csr* 
       const float sc = last ? s : 1.0f;
       const bool sp = sparse && k == 0;
       const SpmmPush nops{0ull, 0, 0};
-      CGX_TRY(spmm_dispatch(by_user, 1, d, bi, nullptr, g_u, nu, sc, lw, lws, stream, sp ? nz_i : nullptr, nops,
+      // bi of k = 1 is the masked output of k = 0's item product (scratch, K >= 2): gather only its frontier rows
+      const uint8_t* bi_nz = sp ? nz_i : (k == 1 ? front : nullptr);
+      CGX_TRY(spmm_dispatch(by_user, 1, d, bi, nullptr, g_u, nu, sc, lw, lws, stream, bi_nz, nops,
                             sparse ? nz_u : nullptr));                                             // g_u + C^T bi
       CGX_TRY(spmm_dispatch(by_item, 1, d, bu, nullptr, g_i, ni, sc, lw, lws, stream, sp ? nz_u : nullptr, nops,
-                            sparse ? nz_i : nullptr));                                             // g_i + A^T bu
+                            sparse ? nz_i : nullptr, k == 0 && !last ? front : nullptr));       // g_i + A^T bu
       bu = nu;
       bi = ni;
     }
@@ -712,11 +776,12 @@ extern "C" int cgx_propagate_bwd_flagged(const cgx_csr* by_user, const cgx_csr* 
     const SpmmPush nops{0ull, 0, 0};
     for (int k = 0; k < K; ++k) {
       const bool last = k == K - 1;
-      float* ni = ib[0];
+      float* ni = ib[0];   // scratch at every k: d_e0_i = s * g_i is written below
       float* nu = last ? d_e0_u : ub[k & 1];
+      const uint8_t* f0 = k == 0 ? front : nullptr;
       CGX_TRY(spmm_dispatch(by_item, 1, d, bu, nullptr, g_i, ni, 1.0f, lw, lws, stream,
-                            sparse && k == 0 ? nz_u : nullptr, nops, sparse ? nz_i : nullptr));       // bi'
-      CGX_TRY(spmm_dispatch(by_user, 1, d, ni, nullptr, g_u, nu, last ? s : 1.0f, lw, lws, stream, nullptr, nops,
+                            sparse && k == 0 ? nz_u : nullptr, nops, sparse ? nz_i : nullptr, f0));      // bi'
+      CGX_TRY(spmm_dispatch(by_user, 1, d, ni, nullptr, g_u, nu, last ? s : 1.0f, lw, lws, stream, f0, nops,
                             sparse ? nz_u : nullptr));                                                // bu'
       bu = nu;
     }

@@ -102,6 +102,19 @@ def bpr_plan(graph: CredGraph, users, pos, neg, plan=None):
     return plan
 
 
+def batch_frontier(graph: CredGraph, users, pos, neg, flags=None):
+    """uint8[I]: 1 on the items of pos, neg and the train rows of the batch users (cgx_batch_frontier), the only
+    rows where the first item-side adjoint of the batch's loss can be non-zero."""
+    dev = graph.device
+    users, pos, neg = _i64c(users, dev), _i64c(pos, dev), _i64c(neg, dev)
+    if flags is None:
+        flags = torch.empty(graph.num_items, dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().cgx_batch_frontier(graph.by_user.ref(), ptr(users), ptr(pos), ptr(neg), users.numel(), ptr(flags),
+                                       stream_ptr(dev)))
+    return flags
+
+
 def bpr_fused(graph: CredGraph, f_u, f_i, e0_u, e0_i, users, pos, neg, reg_weight, fair_weight=0.0, pop=None,
               g_u=None, g_i=None, plan=None, bufs=None, batch_total=0):
     """Loss value + gradients w.r.t. the propagated tables + compact ego (L2) gradient.
@@ -363,11 +376,12 @@ class TrainStep:
         self.g_u, self.g_i = torch.zeros_like(eu), torch.zeros_like(ei)
         self.nz_u = torch.zeros(eu.shape[0], dtype=torch.uint8, device=dev)
         self.nz_i = torch.zeros(ei.shape[0], dtype=torch.uint8, device=dev)
+        self.front_i = torch.zeros(ei.shape[0], dtype=torch.uint8, device=dev)   # item frontier of the batch
         eu.grad, ei.grad = torch.empty_like(eu), torch.empty_like(ei)
         self.opt = optimizer or FusedAdam(eu, ei, lr=lr)
         self.sampler = sampler
         self.phase_events = None      # set to a list to collect (start, fwd_end, loss_end, bwd_end) CUDA events
-        self.side = torch.cuda.Stream(device=dev)     # plan + gradient-buffer clearing overlap the forward
+        self.side = torch.cuda.Stream(device=dev)     # plan (+ item frontier) overlap the forward
         self.tick = torch.zeros(1, dtype=torch.int64, device=dev)   # sampler offset counter (device side)
         self._bufs = {}
         self._graph = None
@@ -392,6 +406,9 @@ class TrainStep:
         dev = eu.device
         users, pos, neg = _i64c(users, dev), _i64c(pos, dev), _i64c(neg, dev)
         plan, bufs = self._batch_bufs(users.numel(), dev)
+        # The item frontier pays only when the item table is beyond L2 (the SpMM's regime switch): inside L2 the
+        # masked gather's per-entry flag lookup costs more than the gathers it saves (C2: +9 us per backward).
+        front = self.front_i if g.num_items * d * 4 > _lib.get_option("L2_TABLE_BYTES") else None
         marks = []
         with torch.cuda.device(dev):
             main = torch.cuda.current_stream(dev)
@@ -399,6 +416,8 @@ class TrainStep:
             self.side.wait_stream(main)                 # the indices are ready
             with torch.cuda.stream(self.side):
                 bpr_plan(g, users, pos, neg, plan)      # scatter plan: beside the forward
+                if front is not None:
+                    batch_frontier(g, users, pos, neg, front)
             st = stream_ptr(dev)
             check(lib().cgx_propagate_fwd(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
                                           ptr(self.f_u), ptr(self.f_i), ptr(ws), ws.numel(), st))
@@ -409,9 +428,9 @@ class TrainStep:
             n_ent = ego_rows.numel()
             check(lib().cgx_bpr_mark_rows(ptr(ego_rows), n_ent, g.num_users, ptr(self.nz_u), ptr(self.nz_i), st))
             self._mark(marks)
-            check(lib().cgx_propagate_bwd_flagged(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(self.g_u),
-                                                  ptr(self.g_i), ptr(self.nz_u), ptr(self.nz_i), ptr(eu.grad),
-                                                  ptr(ei.grad), ptr(ws), ws.numel(), st))
+            check(lib().cgx_propagate_bwd_frontier(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(self.g_u),
+                                                   ptr(self.g_i), ptr(self.nz_u), ptr(self.nz_i), ptr(front),
+                                                   ptr(eu.grad), ptr(ei.grad), ptr(ws), ws.numel(), st))
             self._mark(marks)
             apply_ego(g, ego_rows, ego_coef, eu, ei, eu.grad, ei.grad)
             check(lib().cgx_bpr_clear_rows(ptr(ego_rows), n_ent, g.num_users, d, ptr(self.g_u), ptr(self.g_i),

@@ -233,6 +233,23 @@ int cgx_propagate_bwd_flagged(const cgx_csr* by_user, const cgx_csr* by_item, in
                               int32_t d, const float* g_u, const float* g_i, const uint8_t* g_u_rows,
                               const uint8_t* g_i_rows, float* d_e0_u, float* d_e0_i, void* workspace,
                               size_t workspace_bytes, void* stream);
+/* The same backward of loss.backward() (CU:651, V2:862), told where the first item-side adjoint can be non-zero.
+ * front_i uint8[I] (nullable; NULL = cgx_propagate_bwd_flagged): every item row that is non-zero in g_i, or that
+ * has a non-zero row of g_u among its neighbours, MUST be flagged -- cgx_batch_frontier writes such flags for the
+ * gradient of a triple batch.  The first item-row product g_i + A^T g_u then computes only the flagged rows when
+ * its output is scratch (Gauss-Seidel always, Jacobi for num_layers >= 2), and the product that reads it gathers
+ * only those rows.  Same bits as cgx_propagate_bwd_flagged. */
+int cgx_propagate_bwd_frontier(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t num_layers,
+                               int32_t d, const float* g_u, const float* g_i, const uint8_t* g_u_rows,
+                               const uint8_t* g_i_rows, const uint8_t* front_i, float* d_e0_u, float* d_e0_i,
+                               void* workspace, size_t workspace_bytes, void* stream);
+/* Item frontier of a triple batch for cgx_propagate_bwd_frontier (the items whose rows the first adjoint of
+ * loss.backward(), CU:651 / V2:862, can make non-zero): flags_i uint8[num_items] is zeroed, then set for pos[t],
+ * neg[t] and every column of by_user row users[t], t < batch.  users / pos / neg int64[batch] (device); ids out of
+ * range count as 0, as in cgx_bpr_plan.  Depends on the indices only: it can run on a side stream beside the
+ * forward propagation, as cgx_bpr_plan does. */
+int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64_t* pos, const int64_t* neg,
+                       int64_t batch, uint8_t* flags_i, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * BPR + L2 (+ fairness) on a batch of (user, pos, neg) triples.  Replaces score / l2_reg / the loss

@@ -19,7 +19,8 @@ PRECISIONS = {"fp32": 0, "bf16x3": 1, "bf16": 2}
 # cgx_option (include/credgcn.h).  The library reads no environment variables; for experiments this binding maps
 # CGX_OPT_<NAME>=<int> onto cgx_set_option when the library is loaded.
 OPTIONS = {"L2_TABLE_BYTES": 0, "SPARSE_FIRST_ADJOINT": 1, "PDL": 2, "P2P_ONESHOT_MAX": 3, "P2P_TIMING": 4,
-           "P2P_TIMEOUT_MS": 5, "EVAL_DEBUG": 6, "HOT_ROWS": 7, "EVAL_GROUPS": 8}
+           "P2P_TIMEOUT_MS": 5, "EVAL_DEBUG": 6, "HOT_ROWS": 7, "EVAL_GROUPS": 8,
+           "TOPK_CHUNK_USERS": 9}
 LONG_ROW = 256
 CHUNK = 256
 

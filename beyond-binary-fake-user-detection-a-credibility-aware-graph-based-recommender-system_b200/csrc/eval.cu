@@ -1,6 +1,7 @@
 // Full-rank evaluation: user x item score tiles fused with the train-item mask and a per-row
 // running top-K, plus candidate-list scoring for the sampled protocol.  This file holds the exact
-// fp32 path (CUDA cores); the tensor-core path lives in eval_tc.cu and reuses the selection code.
+// fp32 path (CUDA cores) for K <= 128; the tensor-core path lives in eval_tc.cu and reuses the selection code, and
+// K > 128 runs the candidate-buffer kernels of eval_deep.cu.
 //
 // Replaces (reference, /root/reference): the per-user loop of evaluate_full_ranking,
 // Version-2/lighgcn_cu_pop.py:691-704 (mul+sum scores, scores[train] = -1e9, full argsort) and the
@@ -241,6 +242,11 @@ int eval_topk_tc(const int64_t* users, int64_t n_users, const float* f_u, const 
                  const int64_t* tr_indptr, const int32_t* tr_idx, int32_t K, int precision, int32_t* out_ids,
                  float* out_scores, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 size_t eval_topk_tc_workspace(int64_t n_users, int32_t I, int32_t d, int32_t K, int precision);
+int eval_topk_deep(const int64_t* users, int64_t n_users, const float* f_u, const float* f_i, int32_t I, int32_t d,
+                   const int64_t* tr_indptr, const int32_t* tr_idx, int32_t K, int32_t* out_ids, float* out_scores,
+                   void* workspace, size_t workspace_bytes, cudaStream_t stream);
+size_t eval_topk_deep_workspace(int64_t n_users, int32_t K);
+int eval_topk_deep_max_k();
 
 // exact path on (a subset of) the rows; grid sized for max_rows, CTAs past *n_rows_dev exit at once
 int eval_fp32_rows(const int64_t* users, const int32_t* row_list, const int32_t* n_rows_dev, int64_t max_rows,
@@ -260,6 +266,7 @@ using namespace cgx;
 
 extern "C" size_t cgx_eval_topk_workspace_bytes(int64_t n_users, int32_t num_items, int32_t d, int32_t k,
                                                 int precision) {
+  if (k > 128) return eval_topk_deep_workspace(n_users, k);   // every precision: exact fp32 (eval_deep.cu)
   if (precision == CGX_SCORE_FP32) return 256;
   return eval_topk_tc_workspace(n_users, num_items, d, k, precision);
 }
@@ -270,9 +277,14 @@ extern "C" int cgx_eval_topk(const int64_t* users, int64_t n_users, const float*
                              size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(users && f_u && f_i && train_indptr && out_ids && out_scores, CGX_ERR_ARG, "eval_topk: NULL pointer");
-  CGX_REQUIRE(n_users > 0 && I > 0 && k > 0 && k <= 128 && k <= I, CGX_ERR_ARG,
-              "eval_topk: need 0 < k <= min(128, num_items), got k=%d I=%d", k, I);
+  CGX_REQUIRE(n_users > 0 && I > 0 && k > 0 && k <= eval_topk_deep_max_k() && k <= I, CGX_ERR_ARG,
+              "eval_topk: need 0 < k <= min(%d, num_items), got k=%d I=%d", eval_topk_deep_max_k(), k, I);
   CGX_REQUIRE(cgx_emb_dim_supported(d), CGX_ERR_UNSUPPORTED, "eval_topk: emb_dim %d unsupported", d);
+  CGX_REQUIRE(precision == CGX_SCORE_FP32 || precision == CGX_SCORE_BF16X3 || precision == CGX_SCORE_BF16,
+              CGX_ERR_ARG, "eval_topk: bad precision %d", precision);
+  if (k > 128)   // past the shared-memory list of k_eval_fp32: the deep path, exact fp32 for every precision
+    return eval_topk_deep(users, n_users, f_u, f_i, I, d, train_indptr, train_idx, k, out_ids, out_scores, workspace,
+                          workspace_bytes, stream);
   if (precision != CGX_SCORE_FP32)
     return eval_topk_tc(users, n_users, f_u, f_i, I, d, train_indptr, train_idx, k, precision, out_ids, out_scores,
                         workspace, workspace_bytes, stream);

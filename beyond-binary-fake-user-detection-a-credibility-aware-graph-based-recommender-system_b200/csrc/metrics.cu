@@ -15,7 +15,7 @@
 namespace cgx {
 
 constexpr int MET_MAX_KS = 8;     // distinct cut-offs per call
-constexpr int MET_MAX_K = 256;    // largest cut-off
+constexpr int MET_MAX_K = 4096;   // largest cut-off (the deepest list cgx_eval_topk returns)
 constexpr int MET_SUMS = 7;       // precision, recall, ndcg, log-pop, self-information, high-cred recall, low-cred recall
 constexpr int MET_THREADS = 256;
 
@@ -44,10 +44,11 @@ __global__ void __launch_bounds__(MET_THREADS) k_metrics(const int32_t* __restri
                                                          const uint8_t* __restrict__ group,
                                                          uint32_t* __restrict__ bitmaps, int64_t words,
                                                          double* __restrict__ partial) {
-  __shared__ double disc[MET_MAX_K];
-  __shared__ double idcg[MET_MAX_K + 1];
+  extern __shared__ double met_tab[];   // disc[kmax], idcg[kmax + 1]: sized by the largest cut-off
   __shared__ double red[MET_THREADS / 32][MET_SUMS];
   const int kmax = ks.k[ks.n - 1];
+  double* disc = met_tab;
+  double* idcg = met_tab + kmax;
   for (int r = threadIdx.x; r < kmax; r += MET_THREADS) disc[r] = 1.0 / log2(double(r) + 2.0);
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -202,10 +203,12 @@ extern "C" int cgx_eval_metrics(const int32_t* ranked, int64_t n_users, int32_t 
   Arena ws(workspace, workspace_bytes);
   double* partial = ws.take<double>(size_t(blocks) * n_ks * MET_SUMS);
   CGX_REQUIRE(ws.ok, CGX_ERR_WORKSPACE, "eval_metrics: workspace too small");
-  k_metrics<<<(unsigned)blocks, MET_THREADS, 0, stream>>>(ranked, n_users, ld, users, test_indptr, test_idx, gt_single,
-                                                         num_items, ks, item_pop,
-                                                         double(total_train) + double(num_items), group, bitmaps,
-                                                         words, partial);
+  const size_t tab_smem = size_t(2 * ks.k[n_ks - 1] + 1) * sizeof(double);   // 64 KB at a cut-off of 4096
+  CGX_CUDA(cudaFuncSetAttribute(k_metrics, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tab_smem));
+  k_metrics<<<(unsigned)blocks, MET_THREADS, tab_smem, stream>>>(ranked, n_users, ld, users, test_indptr, test_idx,
+                                                                gt_single, num_items, ks, item_pop,
+                                                                double(total_train) + double(num_items), group,
+                                                                bitmaps, words, partial);
   CGX_LAUNCH_CHECK();
   k_metrics_final<<<n_ks * MET_SUMS, 256, 0, stream>>>(partial, blocks, n_ks, out);
   CGX_LAUNCH_CHECK();

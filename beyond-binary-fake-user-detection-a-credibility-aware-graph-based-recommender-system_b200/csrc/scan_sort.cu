@@ -33,11 +33,12 @@ static const int64_t k_option_defaults[CGX_OPT_COUNT_] = {
     0,                  // CGX_OPT_EVAL_DEBUG
     1,                  // CGX_OPT_HOT_ROWS
     0,                  // CGX_OPT_EVAL_GROUPS
+    0,                  // CGX_OPT_TOPK_CHUNK_USERS
 };
 static std::atomic<int64_t> g_options[CGX_OPT_COUNT_] = {
     {k_option_defaults[0]}, {k_option_defaults[1]}, {k_option_defaults[2]}, {k_option_defaults[3]},
     {k_option_defaults[4]}, {k_option_defaults[5]}, {k_option_defaults[6]}, {k_option_defaults[7]},
-    {k_option_defaults[8]}};
+    {k_option_defaults[8]}, {k_option_defaults[9]}};
 int64_t option(int which) { return g_options[which].load(std::memory_order_relaxed); }
 
 // --------------------------------------------------------------------------------------------

@@ -72,7 +72,9 @@ typedef enum {
                                         insertions / no MMAs / no TMA loads / no merges): WRONG RESULTS, profiles/eval_ablate.py */
   CGX_OPT_HOT_ROWS = 7,              /* [1] cgx_spmm uses the hot-row hints of cgx_csr.idx_hint when present */
   CGX_OPT_EVAL_GROUPS = 8,           /* [0] scanning warp groups of the tensor-core cgx_eval_topk: 0 = library choice, 1, 2 */
-  CGX_OPT_COUNT_ = 9
+  CGX_OPT_TOPK_CHUNK_USERS = 9,      /* [0] users per chunk of cgx_eval_topk for k > 128: 0 = library choice (as many as
+                                        its bounded workspace holds); a smaller value forces more, smaller chunks */
+  CGX_OPT_COUNT_ = 10
 } cgx_option;
 int cgx_set_option(int option, int64_t value, int64_t* previous);
 int64_t cgx_get_option(int option);
@@ -395,6 +397,14 @@ int cgx_comm_timing(uint64_t* out4);
  * Full-rank evaluation.  Replaces the per-user loop of evaluate_full_ranking (V2:691-704):
  * scores of `users` against every item, train items forced to -1e9, best K by
  * (score desc, item id asc).  out_ids int32[n, K], out_scores float[n, K].
+ * 0 < k <= min(4096, num_items); a larger k fails with CGX_ERR_ARG.
+ *   k <= 128   CGX_SCORE_FP32: the exact fp32 kernel.  BF16X3 / BF16: the tcgen05 kernel where
+ *              cgx_eval_topk_uses_tensor_cores says so (BF16X3 with the same ids and score bits as fp32, BF16 a
+ *              single-pass selection re-scored in fp32), else the fp32 kernel.
+ *   k > 128    every precision runs the exact fp32 deep kernel: ids and score bits equal those of FP32, and the
+ *              first 128 columns equal a k = 128 FP32 call (CGX_SCORE_BF16 also gets the exact result).  The
+ *              workspace is bounded (about 1 GiB); users are processed in chunks that fit it
+ *              (CGX_OPT_TOPK_CHUNK_USERS).
  * ------------------------------------------------------------------------------------------ */
 size_t cgx_eval_topk_workspace_bytes(int64_t n_users, int32_t num_items, int32_t d, int32_t k,
                                      int precision);
@@ -403,7 +413,7 @@ int cgx_eval_topk(const int64_t* users, int64_t n_users, const float* f_u, const
                   int32_t k, int precision, int32_t* out_ids, float* out_scores,
                   void* workspace, size_t workspace_bytes, void* stream);
 
-/* 1 when cgx_eval_topk runs the tcgen05 kernel for this (d, k, precision); 0 when it falls back to the exact
+/* 1 when cgx_eval_topk runs the tcgen05 kernel for this (d, k, precision); 0 when it falls back to an exact
  * fp32 kernel (precision FP32, k > 52, or a width whose operands do not fit shared memory: BF16X3 with d = 256). */
 int cgx_eval_topk_uses_tensor_cores(int32_t d, int32_t k, int precision);
 
@@ -429,7 +439,7 @@ int cgx_rank_candidates(const float* scores, const int64_t* cand, int64_t n_user
  * the accumulation loops of evaluate_full_ranking V2:691-752 / evaluate_sampled CU:521-546.
  *   ground truth   gt_single != NULL: one item per row (sampled protocol), else the sorted test rows
  *                  test_idx[test_indptr[users[r]] .. test_indptr[users[r] + 1]) (duplicates counted, as np.diff)
- *   ks_host        HOST array of n_ks <= 8 ascending cut-offs, each <= min(ld, 256)
+ *   ks_host        HOST array of n_ks <= 8 ascending cut-offs, each <= min(ld, 4096)
  *   item_pop       nullable int64[num_items] train popularity (V2:382-388); total_train = its sum
  *   group          nullable uint8[n]: bit 0 = row is in the high-credibility group, bit 1 = in the low one
  *                  (make_cred_groups V2:406-423; a row can be in both when the groups overlap)

@@ -580,36 +580,40 @@ extern "C" int cgx_row_flags(const float* X, int64_t n_rows, int32_t d, uint8_t*
   return row_flags(X, n_rows, d, flags, static_cast<cudaStream_t>(stream));
 }
 
-// Item frontier of a triple batch: flags[i] = 1 for i in pos, neg and the by_user rows of the batch users.  One warp
-// per triple; duplicate users walk their row twice (the stores are idempotent).  Out-of-range ids are clamped to 0,
-// as cgx_bpr_plan does, so the frontier covers every row that cgx_bpr_mark_rows flags.
+// Item frontier of a triple batch: flags[i] = 1 for i in pos, neg and the by_user rows of the batch users, and
+// (flags_u nullable) flags_u[u] = 1 for the batch users.  One warp per triple; duplicate users walk their row twice
+// (the stores are idempotent).  Out-of-range ids are clamped to 0, as cgx_bpr_plan does, so the frontier covers every
+// row that cgx_bpr_mark_rows flags.
 __device__ __forceinline__ int64_t clamp_row(int64_t x, int64_t n) { return (x < 0 || x >= n) ? 0 : x; }
 __global__ void k_batch_frontier(const int64_t* __restrict__ indptr, const int32_t* __restrict__ idx,
                                  const int64_t* __restrict__ users, const int64_t* __restrict__ pos,
                                  const int64_t* __restrict__ neg, int64_t B, int32_t U, int32_t I,
-                                 uint8_t* __restrict__ flags) {
+                                 uint8_t* __restrict__ flags, uint8_t* __restrict__ flags_u) {
   const int64_t t = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) / 32;
   const int lane = threadIdx.x & 31;
   if (t >= B) return;
+  const int64_t u = clamp_row(users[t], U);
   if (lane == 0) {
     flags[clamp_row(pos[t], I)] = 1;
     flags[clamp_row(neg[t], I)] = 1;
+    if (flags_u != nullptr) flags_u[u] = 1;
   }
-  const int64_t u = clamp_row(users[t], U);
   const int64_t end = indptr[u + 1];
   for (int64_t j = indptr[u] + lane; j < end; j += 32) flags[idx[j]] = 1;
 }
 
 extern "C" int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64_t* pos,
-                                  const int64_t* neg, int64_t B, uint8_t* flags_i, void* stream_) {
+                                  const int64_t* neg, int64_t B, uint8_t* flags_i, uint8_t* flags_u,
+                                  void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(by_user && by_user->indptr && (by_user->nnz == 0 || by_user->idx) && users && pos && neg && flags_i,
               CGX_ERR_ARG, "batch_frontier: NULL pointer");
   CGX_REQUIRE(B > 0 && B < (int64_t(1) << 29) && by_user->n_rows > 0 && by_user->n_cols > 0, CGX_ERR_ARG,
               "batch_frontier: bad batch size %lld or empty graph", (long long)B);
   CGX_CUDA(cudaMemsetAsync(flags_i, 0, size_t(by_user->n_cols), stream));
+  if (flags_u != nullptr) CGX_CUDA(cudaMemsetAsync(flags_u, 0, size_t(by_user->n_rows), stream));
   k_batch_frontier<<<(unsigned)ceil_div(B * 32, 256), 256, 0, stream>>>(
-      by_user->indptr, by_user->idx, users, pos, neg, B, by_user->n_rows, by_user->n_cols, flags_i);
+      by_user->indptr, by_user->idx, users, pos, neg, B, by_user->n_rows, by_user->n_cols, flags_i, flags_u);
   CGX_LAUNCH_CHECK();
   return CGX_OK;
 }
@@ -636,10 +640,23 @@ extern "C" size_t cgx_propagate_workspace_bytes_for(const cgx_csr* by_user, cons
 
 extern "C" int cgx_propagate_fwd(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t K, int32_t d,
                                  const float* e0_u, const float* e0_i, float* out_u, float* out_i,
-                                 void* workspace, size_t workspace_bytes, void* stream_) {
+                                 void* workspace, size_t workspace_bytes, void* stream) {
+  return cgx_propagate_fwd_layers(by_user, by_item, order, K, d, e0_u, e0_i, out_u, out_i, 0, K, nullptr, nullptr,
+                                  nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int cgx_propagate_fwd_layers(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t K,
+                                        int32_t d, const float* e0_u, const float* e0_i, float* out_u, float* out_i,
+                                        int32_t layer_begin, int32_t layer_end, const uint8_t* rows_u,
+                                        const uint8_t* rows_i, const uint8_t* all_rows, void* workspace,
+                                        size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(by_user && by_item && e0_u && e0_i && out_u && out_i, CGX_ERR_ARG, "propagate_fwd: NULL pointer");
   CGX_REQUIRE(K >= 1, CGX_ERR_ARG, "propagate_fwd: num_layers must be >= 1");
+  CGX_REQUIRE(0 <= layer_begin && layer_begin <= layer_end && layer_end <= K, CGX_ERR_ARG,
+              "propagate_fwd: layers [%d, %d) outside [0, %d)", layer_begin, layer_end, K);
+  CGX_REQUIRE((rows_u == nullptr && rows_i == nullptr) || all_rows != nullptr, CGX_ERR_ARG,
+              "propagate_fwd: output-row masks need all_rows");
   CGX_REQUIRE(order == CGX_ORDER_JACOBI || order == CGX_ORDER_GS, CGX_ERR_ARG, "propagate_fwd: bad order");
   CGX_REQUIRE(by_user->n_rows == by_item->n_cols && by_user->n_cols == by_item->n_rows, CGX_ERR_ARG,
               "propagate_fwd: operator shapes disagree");
@@ -658,23 +675,28 @@ extern "C" int cgx_propagate_fwd(const cgx_csr* by_user, const cgx_csr* by_item,
   void* lw = ws.take<char>(lws);
   CGX_REQUIRE(ws.ok, CGX_ERR_WORKSPACE, "propagate_fwd: workspace too small");
   const float s = 1.0f / float(K + 1);
-  const float* cu = e0_u;  // layer k tables
-  const float* ci = e0_i;
-  for (int k = 0; k < K; ++k) {
+  const SpmmPush nops{0ull, 0, 0};
+  // The last layer writes only the output rows its masks flag (rows_u / rows_i, nullable).  A mask needs the
+  // row-sparse instantiation (spmm_dispatch); its gather flags are all_rows, all ones, so no entry is dropped and the
+  // sum is the unmasked one.  Layer k - 1's buffers are what layer k gathers, and the last layer writes no user
+  // buffer (and, in Jacobi order, no item buffer): a later call for the rows left out finds its inputs intact.
+  for (int k = layer_begin; k < layer_end; ++k) {
     const bool first = k == 0, last = k == K - 1;
+    const float* cu = first ? e0_u : ub[(k - 1) & 1];   // layer k tables
+    const float* ci = first ? e0_i : ib[(k - 1) & 1];
     float* nu = ub[k & 1];
     float* ni = ib[k & 1];
     const float sc = last ? s : 1.0f;
+    const uint8_t* mu = last ? rows_u : nullptr;
+    const uint8_t* mi = last ? rows_i : nullptr;
     // item side: i_{k+1} = C u_k
     const bool need_ni = !last || order == CGX_ORDER_GS;
     CGX_TRY(spmm_dispatch(by_item, 0, d, cu, need_ni ? ni : nullptr, first ? e0_i : out_i, out_i, sc, lw, lws,
-                          stream));
+                          stream, mi ? all_rows : nullptr, nops, nullptr, mi));
     // user side: u_{k+1} = A i_k (Jacobi) or A i_{k+1} (Gauss-Seidel)
     const float* src = order == CGX_ORDER_JACOBI ? ci : ni;
     CGX_TRY(spmm_dispatch(by_user, 0, d, src, last ? nullptr : nu, first ? e0_u : out_u, out_u, sc, lw, lws,
-                          stream));
-    cu = nu;
-    ci = ni;
+                          stream, mu ? all_rows : nullptr, nops, nullptr, mu));
   }
   return CGX_OK;
 }

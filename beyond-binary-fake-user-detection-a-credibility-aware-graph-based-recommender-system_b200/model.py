@@ -102,16 +102,17 @@ def bpr_plan(graph: CredGraph, users, pos, neg, plan=None):
     return plan
 
 
-def batch_frontier(graph: CredGraph, users, pos, neg, flags=None):
+def batch_frontier(graph: CredGraph, users, pos, neg, flags=None, flags_u=None):
     """uint8[I]: 1 on the items of pos, neg and the train rows of the batch users (cgx_batch_frontier), the only
-    rows where the first item-side adjoint of the batch's loss can be non-zero."""
+    rows where the first item-side adjoint of the batch's loss can be non-zero.  flags_u (uint8[U], optional) is
+    set to 1 on the batch users."""
     dev = graph.device
     users, pos, neg = _i64c(users, dev), _i64c(pos, dev), _i64c(neg, dev)
     if flags is None:
         flags = torch.empty(graph.num_items, dtype=torch.uint8, device=dev)
     with torch.cuda.device(dev):
         check(lib().cgx_batch_frontier(graph.by_user.ref(), ptr(users), ptr(pos), ptr(neg), users.numel(), ptr(flags),
-                                       stream_ptr(dev)))
+                                       ptr(flags_u), stream_ptr(dev)))
     return flags
 
 
@@ -360,7 +361,19 @@ class TrainStep:
     `step(users)` samples on device and updates the parameters; `forward_backward(users, pos, neg)` runs
     on an injected triple list and leaves the gradients in `.grad` (parity tests).  `capture(batch)` records
     the whole step as ONE CUDA graph (sampler offsets and the Adam step count are device-side counters), which
-    removes the ~25 per-step launch calls from the host's critical path."""
+    removes the ~25 per-step launch calls from the host's critical path.
+
+    `f_u` / `f_i` are the final embeddings of the last step.  The loss reads only the batch users' rows of f_u and
+    the pos / neg rows of f_i, so when the item table is beyond L2 (the SpMM's regime switch), num_layers >= 2 and
+    the device has room for a second forward workspace ((U + I) d floats) with DEFER_HEADROOM to spare, the step
+    computes the last layer's products only on the batch users and on the item frontier (pos, neg and the
+    batch users' train items: all that the batch users' last-layer rows gather).  The first read of `f_u` or `f_i`
+    after a step computes the other rows, on the current stream, with the same bits as an eager forward.  The
+    properties return the same tensor objects every time: a reference held across a later step() is not completed
+    by it; read the attribute again."""
+
+    # free device memory that must remain after the deferred path's own forward workspace, else the step stays eager
+    DEFER_HEADROOM = 2 << 30
 
     def __init__(self, model: _Base, lr=1e-3, reg_weight=1e-4, fair_weight=0.0, pop=None, optimizer=None,
                  sampler=None):
@@ -369,7 +382,7 @@ class TrainStep:
         dev = model.user_emb.weight.device
         self.pop = None if pop is None else torch.as_tensor(pop, dtype=torch.float32, device=dev).contiguous()
         eu, ei = model.user_emb.weight, model.item_emb.weight
-        self.f_u, self.f_i = torch.empty_like(eu), torch.empty_like(ei)
+        self._f_u, self._f_i = torch.empty_like(eu), torch.empty_like(ei)
         # dL/d(final tables): dense, but kept ALL-ZERO between steps -- the loss writes <= 3 * batch rows, flags them
         # for the adjoint (cgx_bpr_mark_rows) and the rows are zeroed again after use (cgx_bpr_clear_rows): no fill of
         # (U + I) d floats and no scan for non-zero rows per step
@@ -377,6 +390,7 @@ class TrainStep:
         self.nz_u = torch.zeros(eu.shape[0], dtype=torch.uint8, device=dev)
         self.nz_i = torch.zeros(ei.shape[0], dtype=torch.uint8, device=dev)
         self.front_i = torch.zeros(ei.shape[0], dtype=torch.uint8, device=dev)   # item frontier of the batch
+        self.batch_u = torch.zeros(eu.shape[0], dtype=torch.uint8, device=dev)   # users of the batch
         eu.grad, ei.grad = torch.empty_like(eu), torch.empty_like(ei)
         self.opt = optimizer or FusedAdam(eu, ei, lr=lr)
         self.sampler = sampler
@@ -385,6 +399,62 @@ class TrainStep:
         self.tick = torch.zeros(1, dtype=torch.int64, device=dev)   # sampler offset counter (device side)
         self._bufs = {}
         self._graph = None
+        # Deferred last layer: decided by the first forward (_defers_final).  Its layer buffers must survive the
+        # backward, which overwrites the graph's shared workspace, so the deferred path owns a forward workspace.
+        self._defer_final = None
+        self._fws = self._all_rows = None
+        self._pending = False         # f_u / f_i lack the rows outside the last step's masks
+        self._final_error = None      # a failed completion: f_u / f_i are unusable until the next step
+
+    @property
+    def f_u(self) -> torch.Tensor:
+        """[U, d] final user embeddings of the last step."""
+        self._complete_final()
+        return self._f_u
+
+    @property
+    def f_i(self) -> torch.Tensor:
+        """[I, d] final item embeddings of the last step."""
+        self._complete_final()
+        return self._f_i
+
+    def _defers_final(self, d, order, beyond_l2):
+        """Whether steps restrict the last layer (see the class doc).  Inside L2 the masked products' per-entry flag
+        lookup costs more than the rows they skip (C2: 0.479 ms per step with it against 0.463 without); and the
+        deferred path needs (U + I) d floats more device memory, which C5 on one GPU does not have."""
+        if self.model.num_layers < 2 or not beyond_l2:
+            return False
+        g = self.graph
+        need = lib().cgx_propagate_workspace_bytes_for(g.by_user.ref(), g.by_item.ref(), d, order)
+        free, _ = torch.cuda.mem_get_info(g.device)
+        return free >= need + self.DEFER_HEADROOM
+
+    @torch.no_grad()
+    def _complete_final(self):
+        """The last layer's products on the rows the last step left out: the complement of its masks, as the
+        epilogue adds into f_u / f_i in place (a row computed twice would be added twice)."""
+        if self._final_error is not None:
+            raise self._final_error
+        if not self._pending:
+            return
+        m, g = self.model, self.graph
+        eu, ei = m.user_emb.weight, m.item_emb.weight
+        d, K, order = eu.shape[1], m.num_layers, _lib.ORDERS[m.ORDER]
+        dev = eu.device
+        with torch.cuda.device(dev):
+            rest_u = torch.eq(self.batch_u, 0).view(torch.uint8)
+            rest_i = torch.eq(self.front_i, 0).view(torch.uint8)
+            try:
+                check(lib().cgx_propagate_fwd_layers(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
+                                                     ptr(self._f_u), ptr(self._f_i), K - 1, K, ptr(rest_u),
+                                                     ptr(rest_i), ptr(self._all_rows), ptr(self._fws),
+                                                     self._fws.numel(), stream_ptr(dev)))
+            except _lib.CgxError as e:
+                # part of the rows may have been added already, so a retry could add them twice: every read raises
+                # until the next step recomputes the tables
+                self._final_error = e
+                raise
+        self._pending = False
 
     def _mark(self, marks):
         if self.phase_events is not None:
@@ -408,8 +478,17 @@ class TrainStep:
         plan, bufs = self._batch_bufs(users.numel(), dev)
         # The item frontier pays only when the item table is beyond L2 (the SpMM's regime switch): inside L2 the
         # masked gather's per-entry flag lookup costs more than the gathers it saves (C2: +9 us per backward).
-        front = self.front_i if g.num_items * d * 4 > _lib.get_option("L2_TABLE_BYTES") else None
+        beyond_l2 = g.num_items * d * 4 > _lib.get_option("L2_TABLE_BYTES")
+        if self._defer_final is None:
+            self._defer_final = self._defers_final(d, order, beyond_l2)
+        defer = bool(self._defer_final) and K >= 2     # K = 1: the last layer reads E^0, which Adam overwrites
+        if defer and self._fws is None:
+            self._fws = workspace(lib().cgx_propagate_workspace_bytes_for(g.by_user.ref(), g.by_item.ref(), d, order),
+                                  dev)
+            self._all_rows = torch.ones(max(g.num_users, g.num_items), dtype=torch.uint8, device=dev)
+        front = self.front_i if beyond_l2 or defer else None
         marks = []
+        self._pending, self._final_error = False, None
         with torch.cuda.device(dev):
             main = torch.cuda.current_stream(dev)
             self._mark(marks)
@@ -417,13 +496,27 @@ class TrainStep:
             with torch.cuda.stream(self.side):
                 bpr_plan(g, users, pos, neg, plan)      # scatter plan: beside the forward
                 if front is not None:
-                    batch_frontier(g, users, pos, neg, front)
+                    batch_frontier(g, users, pos, neg, front, self.batch_u if defer else None)
             st = stream_ptr(dev)
-            check(lib().cgx_propagate_fwd(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
-                                          ptr(self.f_u), ptr(self.f_i), ptr(ws), ws.numel(), st))
-            self._mark(marks)
-            main.wait_stream(self.side)
-            loss, _, _, ego_rows, ego_coef = bpr_fused(g, self.f_u, self.f_i, eu, ei, users, pos, neg, self.reg,
+            if defer:
+                # layers 1..K-1 beside the plan and frontier, then layer K on the rows the loss reads
+                fws = self._fws
+                check(lib().cgx_propagate_fwd_layers(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
+                                                     ptr(self._f_u), ptr(self._f_i), 0, K - 1, None, None, None,
+                                                     ptr(fws), fws.numel(), st))
+                main.wait_stream(self.side)
+                check(lib().cgx_propagate_fwd_layers(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
+                                                     ptr(self._f_u), ptr(self._f_i), K - 1, K, ptr(self.batch_u),
+                                                     ptr(self.front_i), ptr(self._all_rows), ptr(fws), fws.numel(),
+                                                     st))
+                self._mark(marks)
+                self._pending = True
+            else:
+                check(lib().cgx_propagate_fwd(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
+                                              ptr(self._f_u), ptr(self._f_i), ptr(ws), ws.numel(), st))
+                self._mark(marks)
+                main.wait_stream(self.side)
+            loss, _, _, ego_rows, ego_coef = bpr_fused(g, self._f_u, self._f_i, eu, ei, users, pos, neg, self.reg,
                                                        self.fair, self.pop, self.g_u, self.g_i, plan, bufs)
             n_ent = ego_rows.numel()
             check(lib().cgx_bpr_mark_rows(ptr(ego_rows), n_ent, g.num_users, ptr(self.nz_u), ptr(self.nz_i), st))
@@ -490,6 +583,7 @@ class TrainStep:
         self._graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._graph):
             self._g_loss = self._sampled_step(self._g_users)
+        self._g_pending = self._pending           # what each replay leaves of f_u / f_i
         self.phase_events = keep
         return self
 
@@ -500,5 +594,6 @@ class TrainStep:
         if self._graph is not None and users.numel() == self._g_users.numel() and self.phase_events is None:
             self._g_users.copy_(users, non_blocking=True)
             self._graph.replay()
+            self._pending, self._final_error = self._g_pending, None
             return self._g_loss
         return self._sampled_step(_i64c(users, self.graph.device))

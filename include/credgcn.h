@@ -223,6 +223,20 @@ size_t cgx_propagate_workspace_bytes_for(const cgx_csr* by_user, const cgx_csr* 
 int cgx_propagate_fwd(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t num_layers,
                       int32_t d, const float* e0_u, const float* e0_i, float* out_u, float* out_i,
                       void* workspace, size_t workspace_bytes, void* stream);
+/* The same forward, layers [layer_begin, layer_end) only (0 <= layer_begin <= layer_end <= num_layers), with
+ * output-row masks for the last layer's products.  A call that starts at layer k > 0 continues the one that ran
+ * layers 0..k-1 on the same out_u / out_i and workspace.  rows_u uint8[U] / rows_i uint8[I] (nullable): the last
+ * layer computes and writes (out_* and its layer buffer) only the flagged rows; the other rows of out_* keep the
+ * running sum of layers 0..K-1.  Masked rows can be computed later by a call for layer K-1 alone with the
+ * complementary masks on the same workspace: the last layer's inputs are not overwritten by it, and the final
+ * tables then carry the bits of cgx_propagate_fwd.  all_rows: uint8[max(U, I)], every entry 1, needed with a mask.
+ * (The last layer adds into out_* in place: computing a row twice adds it twice.)  The completing call picks its
+ * SpMM geometry from the options current when it runs (CGX_OPT_L2_TABLE_BYTES): change none between the two calls,
+ * or the completed rows may differ from cgx_propagate_fwd in the last bits. */
+int cgx_propagate_fwd_layers(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t num_layers,
+                             int32_t d, const float* e0_u, const float* e0_i, float* out_u, float* out_i,
+                             int32_t layer_begin, int32_t layer_end, const uint8_t* rows_u, const uint8_t* rows_i,
+                             const uint8_t* all_rows, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Backward: (g_u, g_i) = dL/d(out_u, out_i) dense -> (d_e0_u, d_e0_i).  SURVEY.md appendix C. */
 int cgx_propagate_bwd(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t num_layers,
@@ -248,10 +262,11 @@ int cgx_propagate_bwd_frontier(const cgx_csr* by_user, const cgx_csr* by_item, i
 /* Item frontier of a triple batch for cgx_propagate_bwd_frontier (the items whose rows the first adjoint of
  * loss.backward(), CU:651 / V2:862, can make non-zero): flags_i uint8[num_items] is zeroed, then set for pos[t],
  * neg[t] and every column of by_user row users[t], t < batch.  users / pos / neg int64[batch] (device); ids out of
- * range count as 0, as in cgx_bpr_plan.  Depends on the indices only: it can run on a side stream beside the
- * forward propagation, as cgx_bpr_plan does. */
+ * range count as 0, as in cgx_bpr_plan.  flags_u uint8[num_users] (nullable) is zeroed and set for users[t]: the
+ * user rows the loss reads.  Depends on the indices only: it can run on a side stream beside the forward
+ * propagation, as cgx_bpr_plan does. */
 int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64_t* pos, const int64_t* neg,
-                       int64_t batch, uint8_t* flags_i, void* stream);
+                       int64_t batch, uint8_t* flags_i, uint8_t* flags_u, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * BPR + L2 (+ fairness) on a batch of (user, pos, neg) triples.  Replaces score / l2_reg / the loss

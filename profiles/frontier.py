@@ -2,15 +2,19 @@
 
     python profiles/frontier.py stats OUT.json [--batches N]        (GPU)  |F|, its edges and its hot-set share
     python profiles/frontier.py kernels OUT.json [--tree DIR]       (GPU)  torch.profiler times of one eager C4 step
-    python profiles/frontier.py traffic STATS.json                  (CPU)  rewrite launches 7 / 8 of r2_traffic.json
+    python profiles/frontier.py reads OUT.json                      (GPU)  what reading TrainStep.f_u costs; C2 deferral
+    python profiles/frontier.py traffic STATS.json                  (CPU)  rewrite launches 5 - 8 of r2_traffic.json
 
 The frontier F of a batch is pos + neg + the train items of the batch users (cgx_batch_frontier): the only rows where
 the first item-side adjoint bi' = g_i + A^T g_u can be non-zero.  `stats` builds the C4 graph and the sampler exactly
 as bench.py does and measures F over bench's first batches.  `kernels` runs eager training steps (no CUDA graph) of
 the package found in --tree (default: this repository) under torch.profiler and lists the SpMM launches of the last
-step in launch order.  `traffic` replaces the two launches of the Gauss-Seidel adjoint at k = 0 in
-profiles/r2_traffic.json (which bench.py divides by the propagation time for roofline.frac) with bytes computed from
-the measured frontier: the ncu capture of those two launches predates the frontier and no longer describes them.
+step in launch order.  `reads` times, with CUDA events and under torch.profiler, the first read of f_u after an eager
+C4 step (the last layer's products on the rows the step left out), and C2 graph replays with the deferred last layer
+forced on and off.  `traffic` replaces the last forward hop (launches 5 and 6, restricted to F and the batch users)
+and the two launches of the Gauss-Seidel adjoint at k = 0 in profiles/r2_traffic.json (which bench.py divides by the
+propagation time for roofline.frac) with bytes computed from the measured frontier: the ncu capture of those four
+launches predates the frontier and no longer describes them.
 """
 import argparse
 import json
@@ -98,6 +102,77 @@ def kernels(args):
         print(" ".join(f"{l['ms']:.2f}" for l in s))
 
 
+def _kname(k):
+    return k.name.split("(")[0].replace("void ", "").replace("cgx::", "")
+
+
+def reads(args):
+    e = c4_setup(HERE.parent, True)
+    torch, step, batches, np = e["torch"], e["step"], e["batches"], e["np"]
+    for s in range(3):
+        step.step(batches[s])
+        step.f_u
+    torch.cuda.synchronize()
+    assert step._defer_final, "C4 should defer the last layer"
+    read_ms = []
+    for s in range(3, 3 + args.steps):
+        step.step(batches[s])
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        step.f_u
+        b.record()
+        torch.cuda.synchronize()
+        read_ms.append(a.elapsed_time(b))
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        step.step(batches[0])
+        torch.cuda.synchronize()
+        step.f_i
+        torch.cuda.synchronize()
+    ev = sorted((k for k in prof.events() if k.device_type == torch.autograd.DeviceType.CUDA),
+                key=lambda k: k.time_range.start)
+    lst = [dict(kernel=_kname(k), ms=round(k.time_range.elapsed_us() / 1e3, 3)) for k in ev]
+    # the read starts with the two torch kernels that invert the masks
+    n_step = next(j for j, x in enumerate(lst) if "elementwise" in x["kernel"])
+    out = dict(gpu=torch.cuda.get_device_name(), first_read_ms_events=read_ms,
+               first_read_ms_median=float(np.median(read_ms)),
+               step_kernels=[x for x in lst[:n_step] if "spmm" in x["kernel"] or "frontier" in x["kernel"]],
+               read_kernels=lst[n_step:])
+    del step, e
+    torch.cuda.empty_cache()
+    # C2 (tables inside L2): graph replays with the deferred last layer forced on / off, alternated
+    from credgcn import graph, model, sampler, synth
+    shp = synth.SHAPES["C2"]
+    sg = synth.make_graph("C2")
+    gr = graph.build_graph(sg.train_edges, sg.num_users, sg.num_items, sg.cred, shp["variant"], "cuda")
+    users = torch.nonzero(gr.deg_u > 0).reshape(-1)[:4096].cuda()
+    sts = {}
+    for defer in (False, True):
+        torch.manual_seed(42)
+        net = model.LightGCN(sg.num_users, sg.num_items, shp["emb_dim"], shp["num_layers"], gr.operator("A"),
+                             gr.operator("C")).cuda()
+        st = model.TrainStep(net, lr=1e-3, reg_weight=1e-4, sampler=sampler.TripleSampler(gr, 0.7, 0.75, 50, seed=42))
+        st._defer_final = defer
+        sts[defer] = st.capture(users.numel())
+    c2 = {False: [], True: []}
+    for rep in range(5):
+        for defer, st in sts.items():
+            for _ in range(20):
+                st.step(users)
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record()
+            for _ in range(200):
+                st.step(users)
+            b.record()
+            torch.cuda.synchronize()
+            c2[defer].append(a.elapsed_time(b) / 200)
+    out["c2_ms_per_step"] = {"eager_last_layer": c2[False], "deferred_last_layer": c2[True],
+                             "median_eager": float(np.median(c2[False])), "median_deferred": float(np.median(c2[True]))}
+    pathlib.Path(args.out).write_text(json.dumps(out, indent=1))
+    print(json.dumps({k: v for k, v in out.items() if k not in ("step_kernels", "read_kernels")}))
+    for x in out["read_kernels"]:
+        print(x)
+
+
 def traffic(args):
     """Compulsory DRAM bytes of the two launches of the first adjoint hop under the frontier, from measured |F|.
     Launch 7 (item rows, masked by F): work descriptors of every item row; idx + val of the rows in F; the first
@@ -118,7 +193,22 @@ def traffic(args):
     data = json.loads(path.read_text())
     c4 = data["C4"]
     src = f"profiles/{pathlib.Path(args.stats).name} (frontier.py traffic)"
-    for i, gb, kind in ((6, l7, "item rows masked by the batch's item frontier F"),
+    # Launches 5 and 6, the last forward hop restricted to F (item rows) and the batch users (user rows).  Launch 5
+    # gathers u_{K-1} along the edges of F's rows: it is charged the captured launch's DRAM bytes per edge net of its
+    # streams (descriptors, three d-wide row streams), times the edges of F; plus every descriptor, the first batch of
+    # column ids / values of the rows outside F, F's three row streams, and the flag arrays (all-ones gather flags
+    # over users, the mask over items).  Launch 6: every descriptor, the first batch of every row outside the batch,
+    # the batch rows' idx + val, gathered rows and two row streams (ACC_IN, ACC_OUT), and the flag arrays.
+    l5_cap = c4["launches"][4].get("captured_before_frontier", c4["launches"][4])
+    desc_i = 16 * (st["item_chunks"] + I - st["item_rows_long"])
+    desc_u = 16 * (st["user_chunks"] + U - st["user_rows_long"])
+    per_edge = (l5_cap["gb"] * 1e9 - desc_i - 3 * row * I) / E
+    l5 = desc_i + 64 * out_items + per_edge * m["front_edges"] + 3 * row * m["front_items"] + U + I
+    bu_edges = B * E / U
+    l6 = desc_u + 64 * (U - B) + (8 + row) * bu_edges + 2 * row * B + U + I
+    for i, gb, kind in ((4, l5, "last forward hop: item rows masked by the batch's item frontier F"),
+                        (5, l6, "last forward hop: user rows masked by the batch users"),
+                        (6, l7, "item rows masked by the batch's item frontier F"),
                         (7, l8, "user rows gathering only the rows of F")):
         old = c4["launches"][i]
         c4["launches"][i] = dict(kernel=old.get("captured_kernel", old["kernel"]), gb=round(gb / 1e9, 3),
@@ -126,16 +216,17 @@ def traffic(args):
                                  captured_before_frontier=dict(ms=old.get("ms"), gb=old.get("gb"),
                                                                l2_hit_pct=old.get("l2_hit_pct"))
                                  if "captured_before_frontier" not in old else old["captured_before_frontier"])
-    c4["launches"][6]["kernel"] = "k_spmm<16, 2, 4, 4, 1, 0, 0>"
-    c4["launches"][7]["kernel"] = "k_spmm<16, 2, 4, 4, 1, 0, 0>"
+    for i in range(4, 8):
+        c4["launches"][i]["kernel"] = "k_spmm<16, 2, 4, 4, 1, 0, 0>"
     c4["bytes_per_step"] = sum(l["gb"] for l in c4["launches"]) * 1e9
     c4["source"] = ("computed: ncu --set full of bench.py's eager step (profiles/r2_ncu_spmm_c4.txt) for launches "
-                    f"1-6 and 9-12, bytes computed from the measured item frontier ({src}) for launches 7 and 8")
-    c4["note"] = ("launches 7 and 8 (the Gauss-Seidel adjoint at k = 0) are computed, not captured: they now touch "
-                  "only the batch's item frontier; their capture before that change is kept under "
-                  "captured_before_frontier")
+                    f"1-4 and 9-12, bytes computed from the measured item frontier ({src}) for launches 5-8")
+    c4["note"] = ("launches 5 and 6 (the last forward hop) and 7 and 8 (the Gauss-Seidel adjoint at k = 0) are "
+                  "computed, not captured: they now touch only the batch's item frontier (and, launch 6, the batch "
+                  "users); their capture before that change is kept under captured_before_frontier")
     path.write_text(json.dumps(data, indent=1))
-    print(f"launch 7: {l7 / 1e9:.3f} GB, launch 8: {l8 / 1e9:.3f} GB, step: {c4['bytes_per_step'] / 1e9:.1f} GB")
+    print(f"launch 5: {l5 / 1e9:.3f} GB, launch 6: {l6 / 1e9:.3f} GB, launch 7: {l7 / 1e9:.3f} GB, "
+          f"launch 8: {l8 / 1e9:.3f} GB, step: {c4['bytes_per_step'] / 1e9:.1f} GB")
 
 
 def main():
@@ -148,10 +239,13 @@ def main():
     a.add_argument("out")
     a.add_argument("--tree", default=str(HERE.parent))
     a.add_argument("--steps", type=int, default=2)
+    a = sub.add_parser("reads")
+    a.add_argument("out")
+    a.add_argument("--steps", type=int, default=5)
     a = sub.add_parser("traffic")
     a.add_argument("stats")
     args = ap.parse_args()
-    dict(stats=stats, kernels=kernels, traffic=traffic)[args.cmd](args)
+    dict(stats=stats, kernels=kernels, reads=reads, traffic=traffic)[args.cmd](args)
 
 
 if __name__ == "__main__":

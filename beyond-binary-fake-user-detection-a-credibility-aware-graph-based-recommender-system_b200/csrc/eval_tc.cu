@@ -12,9 +12,10 @@
 // candidates per user; k_rescore then recomputes their scores exactly as the fp32 kernel does (same
 // fmaf order -> same bits), sorts by (score desc, id asc) and proves the top K complete:
 // if exact_score[K-1] > approx_score[K'-1] + eps(user) no item outside the candidate list can reach
-// the top K.  Rows that fail the proof are redone by the exact fp32 kernel (eval.cu).  The result
-// is therefore identical to CGX_SCORE_FP32.  precision = BF16 is the single-pass variant (K' = d,
-// error ~2^-8 relative, no proof, no redo) for callers that accept approximate ranking.
+// the top K.  Rows that fail the proof are redone by the exact fp32 kernel (k_eval_redo_rows), and so
+// are rows whose lists hold fewer than K real candidates (a user with fewer unseen items than K').  The
+// result is therefore identical to CGX_SCORE_FP32.  precision = BF16 is the single-pass variant (error
+// ~2^-8 relative, no proof; short lists are still redone) for callers that accept approximate ranking.
 //
 // Kernel anatomy (one CTA per 128 users, 17 warps with two scanning groups, 13 with one):
 //   warp 0      TMEM allocation, then one elected lane (elect.sync) issues tcgen05.mma (M=128, N=128, K=16 per
@@ -469,7 +470,7 @@ __global__ void __launch_bounds__(256) k_rescore(const int64_t* __restrict__ use
                                                  const int32_t* __restrict__ tr_idx,
                                                  const int32_t* __restrict__ cand_ids, const float* __restrict__ cand_thr,
                                                  const float* __restrict__ u_norm, const unsigned int* __restrict__ max_norm_bits,
-                                                 float eps_rel, int32_t K, int32_t* __restrict__ out_ids,
+                                                 float eps_rel, bool prove, int32_t K, int32_t* __restrict__ out_ids,
                                                  float* __restrict__ out_scores, int32_t* __restrict__ redo_rows,
                                                  int32_t* __restrict__ n_redo) {
   constexpr int PER = KC / 32;
@@ -519,14 +520,24 @@ __global__ void __launch_bounds__(256) k_rescore(const int64_t* __restrict__ use
     }
     if (rank[q] == K - 1) kth = sc[q];
   }
+  // real candidates: a user with fewer unseen items than the lists hold leaves (-FLT_MAX, INT32_MAX) slots, which
+  // all share one rank; with fewer than K real ones the columns past it are never written above
+  int n_real = 0;
+#pragma unroll
+  for (int q = 0; q < PER; ++q) n_real += __popc(__ballot_sync(0xffffffffu, id[q] != INT32_MAX));
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) kth = fmaxf(kth, __shfl_xor_sync(0xffffffffu, kth, o));
-  if (lane == 0 && redo_rows != nullptr) {
-    // proof of completeness: nothing outside the list can have an exact score >= kth
-    // approx score of the weakest kept candidate of either group: nothing outside the lists scores above it
-    const float thr = fmaxf(cand_thr[2 * r], cand_thr[2 * r + 1]);
-    const float eps = eps_rel * u_norm[r] * __uint_as_float(*max_norm_bits);
-    if (thr > -FLT_MAX && !(kth > thr + eps)) redo_rows[atomicAdd(n_redo, 1)] = int32_t(r);
+  if (lane == 0) {
+    // a short list goes to the exact redo, which ranks the train items after the unseen ones as the fp32 kernel does
+    bool redo = n_real < K;
+    if (!redo && prove) {
+      // proof of completeness: nothing outside the list can have an exact score >= kth
+      // approx score of the weakest kept candidate of either group: nothing outside the lists scores above it
+      const float thr = fmaxf(cand_thr[2 * r], cand_thr[2 * r + 1]);
+      const float eps = eps_rel * u_norm[r] * __uint_as_float(*max_norm_bits);
+      redo = thr > -FLT_MAX && !(kth > thr + eps);
+    }
+    if (redo) redo_rows[atomicAdd(n_redo, 1)] = int32_t(r);
   }
 }
 
@@ -704,8 +715,8 @@ template <int KC, int BC, int NG, int STRIDE>
 static int tc_launch(const __nv_bfloat16* Au, const __nv_bfloat16* Bi, const int64_t* users, int64_t n_users,
                      const float* f_u, const float* f_i, int32_t I, int32_t d, int Kp, int nkb, const int64_t* tr_indptr,
                      const int32_t* tr_idx, int32_t K, int32_t* cand, float* thr, const float* unorm,
-                     const unsigned int* scal, float eps_rel, int32_t* out_ids, float* out_scores, int32_t* redo_rows,
-                     int32_t* n_redo, cudaStream_t stream) {
+                     const unsigned int* scal, float eps_rel, bool prove, int32_t* out_ids, float* out_scores,
+                     int32_t* redo_rows, int32_t* n_redo, cudaStream_t stream) {
   const int S = tc_stages(TcConfig{KC, BC, NG, STRIDE}, Kp);
   const size_t smem = tc_smem(TcConfig{KC, BC, NG, STRIDE}, Kp, S);
   CGX_CUDA(cudaFuncSetAttribute(k_eval_umma<KC, BC, NG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -716,7 +727,7 @@ static int tc_launch(const __nv_bfloat16* Au, const __nv_bfloat16* Bi, const int
       int(option(CGX_OPT_EVAL_DEBUG) >> 1));
   CGX_LAUNCH_CHECK();
   k_rescore<STRIDE><<<(unsigned)ceil_div(n_users, 8), 256, 0, stream>>>(users, n_users, f_u, f_i, d, tr_indptr, tr_idx,
-                                                                       cand, thr, unorm, scal, eps_rel, K, out_ids,
+                                                                       cand, thr, unorm, scal, eps_rel, prove, K, out_ids,
                                                                        out_scores, redo_rows, n_redo);
   CGX_LAUNCH_CHECK();
   return CGX_OK;
@@ -752,10 +763,12 @@ int eval_topk_tc(const int64_t* users, int64_t n_users, const float* f_u, const 
   CGX_LAUNCH_CHECK();
   // bf16x3: dropped lo*lo term, bf16 rounding of lo, fp32 accumulation inside the MMA: 2^-13 |a||b| is a safe cap
   const float eps_rel = 1.0f / 8192.0f;
-  int32_t* redo_rows = precision == CGX_SCORE_BF16X3 ? redo : nullptr;
+  // bf16 selects without the proof (approximate ranking), but a row with fewer than K real candidates is redone for
+  // both precisions: its list cannot fill the K columns
+  const bool prove = precision == CGX_SCORE_BF16X3;
   int32_t* n_redo = reinterpret_cast<int32_t*>(scal + 1);
 #define CGX_TC_ARGS Au, Bi, users, n_users, f_u, f_i, I, d, Kp, nkb, tr_indptr, tr_idx, K, cand, thr, unorm, scal, eps_rel, \
-                    out_ids, out_scores, redo_rows, n_redo, stream
+                    prove, out_ids, out_scores, redo, n_redo, stream
   if (cfg.NG == 2) {
     CGX_TRY((tc_launch<24, 24, 2, 64>(CGX_TC_ARGS)));
   } else if (cfg.KC == 32) {
@@ -764,19 +777,18 @@ int eval_topk_tc(const int64_t* users, int64_t n_users, const float* f_u, const 
     CGX_TRY((tc_launch<64, 16, 1, 64>(CGX_TC_ARGS)));
   }
 #undef CGX_TC_ARGS
-  if (redo_rows != nullptr) {   // rows whose completeness proof failed: exact kernel, count read on device
-    const size_t er_smem = size_t(d) * 4 + size_t(K) * ER_THREADS * 8;
-    CGX_CUDA(cudaFuncSetAttribute(k_eval_redo_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)er_smem));
-    const int64_t er_grid = n_users < 148 * 2 ? n_users : 148 * 2;   // persistent over the device-side row list
-    k_eval_redo_rows<<<(unsigned)er_grid, ER_THREADS, er_smem, stream>>>(users, redo, n_redo, f_u, f_i, I, d, tr_indptr,
-                                                                        tr_idx, K, out_ids, out_scores);
-    CGX_LAUNCH_CHECK();
-    if (option(CGX_OPT_EVAL_DEBUG) & 1) {   // diagnostics only: synchronises
-      unsigned int h[2];
-      CGX_CUDA(cudaMemcpyAsync(h, scal, 8, cudaMemcpyDeviceToHost, stream));
-      CGX_CUDA(cudaStreamSynchronize(stream));
-      fprintf(stderr, "[cgx eval] rows=%lld redo=%u (%.3f %%)\n", (long long)n_users, h[1], 100.0 * h[1] / n_users);
-    }
+  // rows with a short list or a failed completeness proof: exact kernel, count read on device
+  const size_t er_smem = size_t(d) * 4 + size_t(K) * ER_THREADS * 8;
+  CGX_CUDA(cudaFuncSetAttribute(k_eval_redo_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)er_smem));
+  const int64_t er_grid = n_users < 148 * 2 ? n_users : 148 * 2;   // persistent over the device-side row list
+  k_eval_redo_rows<<<(unsigned)er_grid, ER_THREADS, er_smem, stream>>>(users, redo, n_redo, f_u, f_i, I, d, tr_indptr,
+                                                                      tr_idx, K, out_ids, out_scores);
+  CGX_LAUNCH_CHECK();
+  if (option(CGX_OPT_EVAL_DEBUG) & 1) {   // diagnostics only: synchronises
+    unsigned int h[2];
+    CGX_CUDA(cudaMemcpyAsync(h, scal, 8, cudaMemcpyDeviceToHost, stream));
+    CGX_CUDA(cudaStreamSynchronize(stream));
+    fprintf(stderr, "[cgx eval] rows=%lld redo=%u (%.3f %%)\n", (long long)n_users, h[1], 100.0 * h[1] / n_users);
   }
   return CGX_OK;
 }

@@ -54,7 +54,7 @@ class CFG:
     # credibility groups (lighgcn_cu_pop.py:74)
     cred_group_pct: float = 0.20
 
-    # which script's behaviour train_lightgcn() follows: "cu" | "v2" | "da" | "msg" | "me"
+    # which script's behaviour train_lightgcn() follows: "cu" | "v2" | "da" | "msg" | "me" | "raw"
     variant: str = "v2"
     # full-rank eval: "bf16x3" = tcgen05 candidate selection + exact fp32 re-scoring + completeness proof (the
     # SAME ids and score bits as "fp32", 6-7x faster); "fp32" = CUDA-core kernel; "bf16" = one approximate pass

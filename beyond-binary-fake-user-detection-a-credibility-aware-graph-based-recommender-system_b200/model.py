@@ -230,6 +230,13 @@ class _Base(torch.nn.Module):
         torch.nn.init.xavier_uniform_(self.user_emb.weight)
         torch.nn.init.xavier_uniform_(self.item_emb.weight)
 
+    def ego_tables(self):
+        """(user table, item table, user gradient, item gradient) as TrainStep updates them: the storage of the two
+        weights, and fresh [U, d] / [I, d] buffers installed as their .grad."""
+        eu, ei = self.user_emb.weight, self.item_emb.weight
+        eu.grad, ei.grad = torch.empty_like(eu), torch.empty_like(ei)
+        return eu.data, ei.data, eu.grad, ei.grad
+
     def _final(self):
         return _Propagate.apply(self.user_emb.weight, self.item_emb.weight, self.graph, self.num_layers, self.ORDER)
 
@@ -288,6 +295,7 @@ class RawLightGCN(torch.nn.Module):
     """Plain LightGCN of lightgcn.py:306-349 (the thesis' ablation baseline): ONE embedding table over
     users + items and the symmetric normalised adjacency; x <- A x on a bipartite graph is the Jacobi
     schedule on the two blocks of the table.  state_dict key: `emb.weight`."""
+    ORDER = "jacobi"
 
     def __init__(self, num_users, num_items, emb_dim, num_layers, norm_adj):
         super().__init__()
@@ -302,9 +310,16 @@ class RawLightGCN(torch.nn.Module):
         self.emb = torch.nn.Embedding(self.num_nodes, emb_dim)
         torch.nn.init.xavier_uniform_(self.emb.weight)
 
+    def ego_tables(self):
+        """(user table, item table, user gradient, item gradient) as TrainStep updates them: the row blocks [0, U) and
+        [U, U + I) of the one table's storage, and the same blocks of a fresh buffer installed as its .grad."""
+        w, U = self.emb.weight, self.num_users
+        w.grad = torch.empty_like(w)
+        return w.data[:U], w.data[U:], w.grad[:U], w.grad[U:]
+
     def propagate(self):
         w = self.emb.weight
-        fu, fi = _Propagate.apply(w[: self.num_users], w[self.num_users:], self.graph, self.num_layers, "jacobi")
+        fu, fi = _Propagate.apply(w[: self.num_users], w[self.num_users:], self.graph, self.num_layers, self.ORDER)
         return torch.cat([fu, fi], dim=0)
 
     def get_user_item_emb(self):
@@ -323,29 +338,37 @@ class RawLightGCN(torch.nn.Module):
 class FusedAdam:
     """torch.optim.Adam(params, lr) semantics (defaults: betas (0.9, 0.999), eps 1e-8; lightgcn_cu.py:587)
     for the two embedding tables, one kernel launch per step.  The step count lives on the device so
-    that a captured CUDA graph keeps advancing it."""
+    that a captured CUDA graph keeps advancing it.  `grads`, when given, are the two gradient buffers to read instead
+    of the weights' .grad: the tables may be the two row blocks of ONE parameter (RawLightGCN), which is then
+    torch.optim.Adam on that parameter, Adam being elementwise."""
 
-    def __init__(self, user_weight: torch.Tensor, item_weight: torch.Tensor, lr=1e-3, betas=(0.9, 0.999), eps=1e-8):
+    def __init__(self, user_weight: torch.Tensor, item_weight: torch.Tensor, lr=1e-3, betas=(0.9, 0.999), eps=1e-8,
+                 grads=None):
         self.params = (user_weight, item_weight)
+        self.grads = grads
         self.lr, self.betas, self.eps = float(lr), (float(betas[0]), float(betas[1])), float(eps)
         self.m = [torch.zeros_like(p) for p in self.params]
         self.v = [torch.zeros_like(p) for p in self.params]
         self.step_dev = torch.zeros(1, dtype=torch.int64, device=user_weight.device)   # steps taken so far
 
+    def _grads(self):
+        return self.grads if self.grads is not None else tuple(p.grad for p in self.params)
+
     def zero_grad(self, set_to_none: bool = False):
-        for p in self.params:
-            if p.grad is not None:
-                p.grad.zero_()
+        for g in self._grads():
+            if g is not None:
+                g.zero_()
 
     @torch.no_grad()
     def step(self):
         pu, pi = self.params
+        gu, gi = self._grads()
         dev = pu.device
         with torch.cuda.device(dev):
             st = stream_ptr(dev)
             check(lib().cgx_tick(ptr(self.step_dev), st))
-            check(lib().cgx_adam_step(ptr(pu.data), ptr(_f32c(pu.grad)), ptr(self.m[0]), ptr(self.v[0]), pu.numel(),
-                                      ptr(pi.data), ptr(_f32c(pi.grad)), ptr(self.m[1]), ptr(self.v[1]), pi.numel(),
+            check(lib().cgx_adam_step(ptr(pu.data), ptr(_f32c(gu)), ptr(self.m[0]), ptr(self.v[0]), pu.numel(),
+                                      ptr(pi.data), ptr(_f32c(gi)), ptr(self.m[1]), ptr(self.v[1]), pi.numel(),
                                       self.lr, self.betas[0], self.betas[1], self.eps, ptr(self.step_dev), 0, st))
 
     def state_dict(self):
@@ -356,7 +379,9 @@ class FusedAdam:
 class TrainStep:
     """One full training step on pre-allocated buffers.  Equivalent to lightgcn_cu.py:608-652 /
     lighgcn_cu_pop.py:826-863: one (user, pos, neg) triple per batch user, final embeddings, BPR (+fair) + L2
-    loss, backward, dense Adam.
+    loss, backward, dense Adam.  The model hands over its ego tables with `ego_tables()` and its layer order as
+    `ORDER`: the two weights of CredLightGCN / LightGCN, or the user and item row blocks of RawLightGCN's one table
+    (lightgcn.py's loop: Jacobi order, one Adam over `emb.weight`), whose gradient fills the same blocks of its .grad.
 
     `step(users)` samples on device and updates the parameters; `forward_backward(users, pos, neg)` runs
     on an injected triple list and leaves the gradients in `.grad` (parity tests).  `capture(batch)` records
@@ -375,13 +400,15 @@ class TrainStep:
     # free device memory that must remain after the deferred path's own forward workspace, else the step stays eager
     DEFER_HEADROOM = 2 << 30
 
-    def __init__(self, model: _Base, lr=1e-3, reg_weight=1e-4, fair_weight=0.0, pop=None, optimizer=None,
+    def __init__(self, model: _Base | RawLightGCN, lr=1e-3, reg_weight=1e-4, fair_weight=0.0, pop=None, optimizer=None,
                  sampler=None):
         self.model, self.graph = model, model.graph
         self.reg, self.fair = float(reg_weight), float(fair_weight)
-        dev = model.user_emb.weight.device
+        # the ego tables and their gradients: two parameters, or the two row blocks of RawLightGCN's one table
+        self._eu, self._ei, self._gu, self._gi = model.ego_tables()
+        eu, ei = self._eu, self._ei
+        dev = eu.device
         self.pop = None if pop is None else torch.as_tensor(pop, dtype=torch.float32, device=dev).contiguous()
-        eu, ei = model.user_emb.weight, model.item_emb.weight
         self._f_u, self._f_i = torch.empty_like(eu), torch.empty_like(ei)
         # dL/d(final tables): dense, but kept ALL-ZERO between steps -- the loss writes <= 3 * batch rows, flags them
         # for the adjoint (cgx_bpr_mark_rows) and the rows are zeroed again after use (cgx_bpr_clear_rows): no fill of
@@ -391,8 +418,7 @@ class TrainStep:
         self.nz_i = torch.zeros(ei.shape[0], dtype=torch.uint8, device=dev)
         self.front_i = torch.zeros(ei.shape[0], dtype=torch.uint8, device=dev)   # item frontier of the batch
         self.batch_u = torch.zeros(eu.shape[0], dtype=torch.uint8, device=dev)   # users of the batch
-        eu.grad, ei.grad = torch.empty_like(eu), torch.empty_like(ei)
-        self.opt = optimizer or FusedAdam(eu, ei, lr=lr)
+        self.opt = optimizer or FusedAdam(eu, ei, lr=lr, grads=(self._gu, self._gi))
         self.sampler = sampler
         self.phase_events = None      # set to a list to collect (start, fwd_end, loss_end, bwd_end) CUDA events
         self.side = torch.cuda.Stream(device=dev)     # plan (+ item frontier) overlap the forward
@@ -438,7 +464,7 @@ class TrainStep:
         if not self._pending:
             return
         m, g = self.model, self.graph
-        eu, ei = m.user_emb.weight, m.item_emb.weight
+        eu, ei = self._eu, self._ei
         d, K, order = eu.shape[1], m.num_layers, _lib.ORDERS[m.ORDER]
         dev = eu.device
         with torch.cuda.device(dev):
@@ -470,7 +496,7 @@ class TrainStep:
     @torch.no_grad()
     def forward_backward(self, users, pos, neg):
         m, g = self.model, self.graph
-        eu, ei = m.user_emb.weight, m.item_emb.weight
+        eu, ei = self._eu, self._ei
         d, K, order = eu.shape[1], m.num_layers, _lib.ORDERS[m.ORDER]
         ws = g.propagate_workspace(d, order)
         dev = eu.device
@@ -523,9 +549,9 @@ class TrainStep:
             self._mark(marks)
             check(lib().cgx_propagate_bwd_frontier(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(self.g_u),
                                                    ptr(self.g_i), ptr(self.nz_u), ptr(self.nz_i), ptr(front),
-                                                   ptr(eu.grad), ptr(ei.grad), ptr(ws), ws.numel(), st))
+                                                   ptr(self._gu), ptr(self._gi), ptr(ws), ws.numel(), st))
             self._mark(marks)
-            apply_ego(g, ego_rows, ego_coef, eu, ei, eu.grad, ei.grad)
+            apply_ego(g, ego_rows, ego_coef, eu, ei, self._gu, self._gi)
             check(lib().cgx_bpr_clear_rows(ptr(ego_rows), n_ent, g.num_users, d, ptr(self.g_u), ptr(self.g_i),
                                            ptr(self.nz_u), ptr(self.nz_i), st))
         if self.phase_events is not None:
@@ -562,15 +588,15 @@ class TrainStep:
         with torch.cuda.stream(warm):                       # warm-up outside capture (allocations, attributes)
             state = opt_state = None
             if preserve_state:
-                state = [p.detach().clone() for p in (self.model.user_emb.weight, self.model.item_emb.weight)]
+                state = [self._eu.clone(), self._ei.clone()]
                 opt_state = ([t.clone() for t in self.opt.m], [t.clone() for t in self.opt.v],
                              self.opt.step_dev.clone(), self.tick.clone()) if isinstance(self.opt, FusedAdam) else None
             for _ in range(2):
                 self._sampled_step(self._g_users)
             # the warm-up steps must not count: restore parameters, optimiser state and counters
             if state is not None:
-                self.model.user_emb.weight.data.copy_(state[0])
-                self.model.item_emb.weight.data.copy_(state[1])
+                self._eu.copy_(state[0])
+                self._ei.copy_(state[1])
             if opt_state is not None:
                 for dst, src in zip(self.opt.m, opt_state[0]):
                     dst.copy_(src)

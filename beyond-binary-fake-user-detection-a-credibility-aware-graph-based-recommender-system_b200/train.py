@@ -12,6 +12,10 @@ edges.  `cfg.variant` selects which script is reproduced:
     "me"  version_1/..._method-e         Gauss-Seidel, popularity-mixture negatives
     "da"  version_1/..._Degree-Aware     Gauss-Seidel, uniform negatives, alpha_i damping
     "v2"  Version-2/lighgcn_cu_pop       Gauss-Seidel, popularity-mixture negatives, extra metrics
+    "raw" lightgcn.py                    plain LightGCN: one table over users + items, the symmetric normalised
+                                         adjacency (build_norm_adj, Jacobi order), uniform negatives, no credibility
+                                         CSV, sampled or full eval, `best_model.pt` with the key `emb.weight`
+RAW's L2 weight is cfg.reg (1e-4, as in every script).  lightgcn-1.py is the same script with cfg.epochs = 200.
 """
 from __future__ import annotations
 
@@ -23,8 +27,8 @@ import numpy as np
 import torch
 
 from . import config, evaluate
-from .graph import build_graph
-from .model import CredLightGCN, LightGCN, TrainStep
+from .graph import build_graph, build_norm_adj
+from .model import CredLightGCN, LightGCN, RawLightGCN, TrainStep
 from .sampler import TripleSampler
 
 _GRAPH_VARIANT = {"cu": "cu", "v2": "v2", "msg": "v2", "me": "v2", "da": "da"}
@@ -100,13 +104,18 @@ def _print_metrics(tag, res, Ks, rich):
 
 
 def train_on_arrays(train_edges, val_edges, test_edges, num_users, num_items, cred_np, out_dir=None, cfg=None):
-    """The reference's training loop on in-memory edges.  Returns (model, test_results)."""
+    """The reference's training loop on in-memory edges.  Returns (model, test_results).  cred_np is not read for
+    cfg.variant == "raw" (None is fine)."""
     cfg = cfg or config.cfg
     variant = cfg.variant
     device = cfg.device
     print("Using device:", device)
 
-    graph = build_graph(train_edges, num_users, num_items, cred_np, _GRAPH_VARIANT[variant], device)
+    if variant == "raw":
+        norm_adj = build_norm_adj(train_edges, num_users, num_items, device)
+        graph = norm_adj.graph
+    else:
+        graph = build_graph(train_edges, num_users, num_items, cred_np, _GRAPH_VARIANT[variant], device)
     train_csr = graph.user_csr_numpy()
     val_csr = evaluate_csr(val_edges, num_users, num_items, device)
     test_csr = evaluate_csr(test_edges, num_users, num_items, device)
@@ -120,6 +129,9 @@ def train_on_arrays(train_edges, val_edges, test_edges, num_users, num_items, cr
         model = CredLightGCN(num_users, num_items, cfg.emb_dim, cfg.num_layers, graph.operator("C"),
                              graph.operator("A")).to(device)
         reg = cfg.lambda_reg
+    elif variant == "raw":
+        model = RawLightGCN(num_users, num_items, cfg.emb_dim, cfg.num_layers, norm_adj).to(device)
+        reg = cfg.reg
     else:
         model = LightGCN(num_users, num_items, cfg.emb_dim, cfg.num_layers, graph.operator("A"),
                          graph.operator("C")).to(device)
@@ -209,7 +221,7 @@ def train_lightgcn():
     num_users, num_items = len(user2idx), len(item2idx)
     print(f"Loaded edges. Users={num_users:,} Items={num_items:,} "
           f"Train={train_edges.shape[1]:,} Val={val_edges.shape[1]:,} Test={test_edges.shape[1]:,}")
-    cred_np = load_credibility_vector(cfg.cred_csv_path, user2idx)
+    cred_np = None if cfg.variant == "raw" else load_credibility_vector(cfg.cred_csv_path, user2idx)
     _, test_res = train_on_arrays(train_edges, val_edges, test_edges, num_users, num_items, cred_np, out, cfg)
     return test_res
 

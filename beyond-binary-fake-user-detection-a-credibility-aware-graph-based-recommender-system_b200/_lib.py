@@ -73,14 +73,14 @@ _SIGNATURES = {
     "cgx_propagate_fwd": (C.c_int, [_CSR, _CSR, C.c_int, C.c_int32, C.c_int32, _P, _P, _P, _P, _P,
                                     C.c_size_t, _P]),
     "cgx_propagate_fwd_layers": (C.c_int, [_CSR, _CSR, C.c_int, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32,
-                                           C.c_int32, _P, _P, _P, _P, C.c_size_t, _P]),
+                                           C.c_int32, C.c_int, _P, _P, _P, C.c_int64, _P, _P, _P, C.c_size_t, _P]),
     "cgx_propagate_bwd": (C.c_int, [_CSR, _CSR, C.c_int, C.c_int32, C.c_int32, _P, _P, _P, _P, _P,
                                     C.c_size_t, _P]),
     "cgx_propagate_bwd_flagged": (C.c_int, [_CSR, _CSR, C.c_int, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P,
                                             C.c_size_t, _P]),
     "cgx_propagate_bwd_frontier": (C.c_int, [_CSR, _CSR, C.c_int, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P,
                                              _P, _P, C.c_size_t, _P]),
-    "cgx_batch_frontier": (C.c_int, [_CSR, _P, _P, _P, C.c_int64, _P, _P, _P]),
+    "cgx_batch_frontier": (C.c_int, [_CSR, _P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "cgx_bpr_mark_rows": (C.c_int, [_P, C.c_int64, C.c_int32, _P, _P, _P]),
     "cgx_bpr_clear_rows": (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "cgx_bpr_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32, C.c_int32]),

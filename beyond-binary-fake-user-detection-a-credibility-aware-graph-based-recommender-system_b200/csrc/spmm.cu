@@ -78,6 +78,14 @@ __device__ __forceinline__ void ld256_rw(const float4* p, float4& a, float4& b) 
                  : "memory");
   }
 }
+__device__ __forceinline__ float4 ld128_rw(const float4* p) {
+  float4 a;
+  asm volatile("ld.global.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w) : "l"(p) : "memory");
+  return a;
+}
+__device__ __forceinline__ void st128(float4* p, const float4& a) {
+  asm volatile("st.global.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(a.x), "f"(a.y), "f"(a.z), "f"(a.w) : "memory");
+}
 template <int POL>
 __device__ __forceinline__ void st256(float4* p, const float4& a, const float4& b) {
   if (POL == POL_FIRST) {
@@ -194,10 +202,16 @@ struct SpmmPush {
 
 // acc_nz (nullable): acc_nz[row] == 0 promises that ACC_IN[row] is all zero, and it is then not read (the adjoint's
 // ACC_IN is the loss gradient: <= 3 * batch non-zero rows of millions).
+// ACC_PREV (nullable, with ACC_OUT): ACC_OUT[r] = acc_scale * ((ACC_IN[r] + ACC_PREV[r]) + y), the running sum of the
+// layer before folded in here instead of by that layer's own product -- the adds of the unfolded chain, in its order.
+// ACC_PREV may alias Y (Gauss-Seidel: the item product writes i_K over i_{K-1}), so it is read coherently, and Y is
+// stored after ACC_OUT, whose value waits for that load: a store issued while a load of the same bytes is still in
+// flight stalls the SM's memory pipeline (measured on C4: the completing item product 9.3 -> 14.5 ms).
 template <int G, int V, bool STREAM>
 __device__ __forceinline__ void epilogue(int64_t row, int lane, const float4 (&y)[V], float4* __restrict__ Y,
                                          const float4* ACC_IN, float4* ACC_OUT, float acc_scale,
-                                         const uint8_t* __restrict__ acc_nz, const SpmmPush ps) {
+                                         const uint8_t* __restrict__ acc_nz, const SpmmPush ps,
+                                         const float4* ACC_PREV = nullptr) {
   constexpr int ROW4 = G * V;
   constexpr int POL = STREAM ? POL_FIRST : POL_NORMAL;
   const int64_t o = row * ROW4 + lane * V;
@@ -210,6 +224,16 @@ __device__ __forceinline__ void epilogue(int64_t row, int lane, const float4 (&y
 #pragma unroll
       for (int v = 0; v < V; ++v) a[v] = ACC_IN[o + v];
     }
+  }
+  if (ACC_PREV != nullptr) {
+    float4 p[V];
+    if constexpr (V == 2) ld256_rw<POL>(ACC_PREV + o, p[0], p[1]);
+    else {
+#pragma unroll
+      for (int v = 0; v < V; ++v) p[v] = ld128_rw(ACC_PREV + o + v);
+    }
+#pragma unroll
+    for (int v = 0; v < V; ++v) a[v] = add4(a[v], p[v]);
   }
   if (ps.rows_per > 0) {
     const int owner = int(row / ps.rows_per);
@@ -224,7 +248,8 @@ __device__ __forceinline__ void epilogue(int64_t row, int lane, const float4 (&y
       for (int v = 0; v < V; ++v) ypush[v] = y[v];
     }
   }
-  if (Y != nullptr) {
+  const bool y_late = ACC_PREV != nullptr;
+  if (Y != nullptr && !y_late) {
     if constexpr (V == 2) st256<POL>(Y + o, y[0], y[1]);
     else {
 #pragma unroll
@@ -238,6 +263,13 @@ __device__ __forceinline__ void epilogue(int64_t row, int lane, const float4 (&y
     else {
 #pragma unroll
       for (int v = 0; v < V; ++v) ACC_OUT[o + v] = a[v];
+    }
+  }
+  if (Y != nullptr && y_late) {
+    if constexpr (V == 2) st256<POL>(Y + o, y[0], y[1]);
+    else {
+#pragma unroll
+      for (int v = 0; v < V; ++v) st128(Y + o + v, y[v]);
     }
   }
 }
@@ -259,13 +291,16 @@ __global__ void __launch_bounds__(SP_THREADS, MINB) k_spmm(const int32_t* __rest
                                                            const float* __restrict__ val, int64_t n_items,
                                                            SpmmSched sc, const float4* __restrict__ X,
                                                            float4* __restrict__ Y, const float4* ACC_IN,
-                                                           float4* ACC_OUT, float acc_scale, float4* partial,
+                                                           float4* ACC_OUT, const float4* ACC_PREV,
+                                                           float acc_scale, float4* partial,
                                                            const uint8_t* __restrict__ nz,
                                                            const uint8_t* __restrict__ acc_nz,
                                                            const uint8_t* __restrict__ out_rows,
                                                            const int4* __restrict__ work, const SpmmPush ps_in) {
   // PUSH = false: a compile-time "off", so that the ordinary instantiations carry no trace of the push path
   const SpmmPush ps = PUSH ? ps_in : SpmmPush{0ull, 0, 0};
+  // ACC_PREV only in the masked instantiations, which the last layer uses: the others run at the 64-register cap
+  const float4* acc_prev = NZ && !PUSH ? ACC_PREV : nullptr;
   constexpr int ROW4 = G * V;
   // Programmatic dependent launch: let the next kernel of the stream start its own prologue now, and run
   // THIS kernel's prologue (descriptor, first batch of column ids / values -- graph constants) while the
@@ -302,7 +337,7 @@ __global__ void __launch_bounds__(SP_THREADS, MINB) k_spmm(const int32_t* __rest
   if (item >= sc.n_chunks) {
     // (loading ACC_IN[row] before the gathers, to take it off the dependency chain, was measured SLOWER: the
     // four extra live registers spill at the 64-register cap -- C2 0.514 -> 0.553 ms, C4 155 -> 160 ms)
-    epilogue<G, V, HOT>(wd.w, lane, acc, Y, ACC_IN, ACC_OUT, acc_scale, acc_nz, ps);
+    epilogue<G, V, HOT>(wd.w, lane, acc, Y, ACC_IN, ACC_OUT, acc_scale, acc_nz, ps, acc_prev);
     return;
   }
   const int32_t k = wd.w;
@@ -323,7 +358,7 @@ __global__ void __launch_bounds__(SP_THREADS, MINB) k_spmm(const int32_t* __rest
 #pragma unroll
     for (int v = 0; v < V; ++v) acc[v] = add4(acc[v], __ldcg(partial + int64_t(c) * ROW4 + lane * V + v));
   }
-  epilogue<G, V, HOT>(int64_t(__ldg(sc.perm + k)), lane, acc, Y, ACC_IN, ACC_OUT, acc_scale, acc_nz, ps);
+  epilogue<G, V, HOT>(int64_t(__ldg(sc.perm + k)), lane, acc, Y, ACC_IN, ACC_OUT, acc_scale, acc_nz, ps, acc_prev);
   if (lane == 0) sc.arrive[k] = 0;       // self-resetting for the next launch
 }
 
@@ -331,8 +366,8 @@ __global__ void __launch_bounds__(SP_THREADS, MINB) k_spmm(const int32_t* __rest
 template <int G, int V>
 __global__ void __launch_bounds__(SP_THREADS) k_spmm_finish(SpmmSched sc, const float4* __restrict__ partial,
                                                             float4* __restrict__ Y, const float4* ACC_IN,
-                                                            float4* ACC_OUT, float acc_scale,
-                                                            const uint8_t* __restrict__ acc_nz,
+                                                            float4* ACC_OUT, const float4* ACC_PREV,
+                                                            float acc_scale, const uint8_t* __restrict__ acc_nz,
                                                             const uint8_t* __restrict__ out_rows, const SpmmPush ps) {
   constexpr int GROUPS = SP_THREADS / G;
   constexpr int ROW4 = G * V;
@@ -358,8 +393,96 @@ __global__ void __launch_bounds__(SP_THREADS) k_spmm_finish(SpmmSched sc, const 
       for (int g = 1; g < GROUPS; ++g) s = add4(s, red[g][lane * V + v]);
       acc[v] = s;
     }
-    epilogue<G, V, false>(int64_t(__ldg(sc.perm + k)), lane, acc, Y, ACC_IN, ACC_OUT, acc_scale, acc_nz, ps);
+    epilogue<G, V, false>(int64_t(__ldg(sc.perm + k)), lane, acc, Y, ACC_IN, ACC_OUT, acc_scale, acc_nz, ps,
+                          ACC_PREV);
   }
+}
+
+__device__ __forceinline__ int64_t clamp_row(int64_t x, int64_t n) { return (x < 0 || x >= n) ? 0 : x; }
+
+// Output rows named by a list instead of a row mask (SpmmList): one CTA per entry t computes row r = rows[t] (ids out
+// of range count as 0, as in cgx_bpr_plan) when owner[r] == t, so a repeated row is computed once (the epilogue adds
+// into ACC_OUT in place).  The row is cut into the schedule's chunks (cgx_row_schedule_work) and the chunk sums are
+// added in the order of k_spmm: a row up to CGX_LONG_ROW in one piece, a long row's chunks in chunk order (as its
+// last-arriving chunk adds them), a huge row's as k_spmm_finish does (group g sums chunks g, g + GROUPS, ..., then the
+// groups in order).  The gathers are the masked k_spmm's (NZ, gather flags nz), so every output row has its bits.
+// The grid is the list, not every work item of the table: B rows cost B CTAs, not a pass over 10 M descriptors.
+template <int G, int V, int UNR>
+__global__ void __launch_bounds__(SP_THREADS) k_spmm_list(const int64_t* __restrict__ indptr,
+                                                          const int32_t* __restrict__ idx,
+                                                          const float* __restrict__ val, int64_t n_rows,
+                                                          const int64_t* __restrict__ rows,
+                                                          const int32_t* __restrict__ owner,
+                                                          const float4* __restrict__ X, float4* __restrict__ Y,
+                                                          const float4* ACC_IN, float4* ACC_OUT,
+                                                          const float4* ACC_PREV, float acc_scale,
+                                                          const uint8_t* __restrict__ nz,
+                                                          const uint8_t* __restrict__ acc_nz) {
+  constexpr int GROUPS = SP_THREADS / G;
+  constexpr int ROW4 = G * V;
+  __shared__ float4 red[GROUPS][ROW4];
+  const int64_t t = blockIdx.x;
+  const int64_t row = clamp_row(__ldg(rows + t), n_rows);
+  if (__ldg(owner + row) != int32_t(t)) return;   // the whole CTA: another entry owns the row
+  const int lane = threadIdx.x & (G - 1), grp = threadIdx.x / G;
+  const unsigned mask = group_mask<G>();
+  const int64_t begin = __ldg(indptr + row), len = __ldg(indptr + row + 1) - begin;
+  const bool chunked = len > CGX_LONG_ROW, huge = len > CGX_HUGE_ROW;
+  if (!chunked && grp != 0) return;
+  const int64_t n_pieces = chunked ? (len + CGX_CHUNK - 1) / CGX_CHUNK : 1;
+  float4 run[V];
+#pragma unroll
+  for (int v = 0; v < V; ++v) run[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int64_t c0 = 0; c0 < n_pieces; c0 += GROUPS) {   // uniform over the CTA when chunked
+    const int64_t c = c0 + grp;
+    float4 p[V];
+#pragma unroll
+    for (int v = 0; v < V; ++v) p[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (c < n_pieces) {
+      const int64_t b = begin + c * CGX_CHUNK;
+      const int32_t n = int32_t(chunked ? (len - c * CGX_CHUNK < CGX_CHUNK ? len - c * CGX_CHUNK : CGX_CHUNK) : len);
+      int32_t cf = 0;
+      float wf = 0.f;
+      if (lane < n) {
+        cf = ld_idx<false>(idx + b + lane);
+        wf = ld_val<false>(val + b + lane);
+      }
+      gather_batches<G, V, UNR, true, false>(idx + b, val + b, n, X, lane, mask, cf, wf, p, nz);
+#pragma unroll
+      for (int v = 0; v < V; ++v) {      // (a whole row is the sum itself: 0 + (-0) would not keep its bits)
+        if (!chunked) run[v] = p[v];
+        else if (huge) run[v] = add4(run[v], p[v]);
+      }
+    }
+    if (chunked && !huge) {               // chunk order: group 0 adds this round's chunks one by one
+#pragma unroll
+      for (int v = 0; v < V; ++v) red[grp][lane * V + v] = p[v];
+      __syncthreads();
+      if (grp == 0) {
+        const int64_t m = n_pieces - c0 < GROUPS ? n_pieces - c0 : GROUPS;
+        for (int g = 0; g < m; ++g) {
+#pragma unroll
+          for (int v = 0; v < V; ++v) run[v] = add4(run[v], red[g][lane * V + v]);
+        }
+      }
+      __syncthreads();
+    }
+  }
+  if (huge) {                             // k_spmm_finish's reduction over the groups
+#pragma unroll
+    for (int v = 0; v < V; ++v) red[grp][lane * V + v] = run[v];
+    __syncthreads();
+    if (grp != 0) return;
+#pragma unroll
+    for (int v = 0; v < V; ++v) {
+      float4 s = red[0][lane * V + v];
+      for (int g = 1; g < GROUPS; ++g) s = add4(s, red[g][lane * V + v]);
+      run[v] = s;
+    }
+  } else if (grp != 0) {
+    return;
+  }
+  epilogue<G, V, false>(row, lane, run, Y, ACC_IN, ACC_OUT, acc_scale, acc_nz, SpmmPush{0ull, 0, 0}, ACC_PREV);
 }
 
 __global__ void k_scale(const float4* __restrict__ in, float4* __restrict__ out, int64_t n4, float s) {
@@ -384,11 +507,29 @@ static int row_flags(const float* X, int64_t n_rows, int32_t d, uint8_t* flags, 
   return CGX_OK;
 }
 
+// Output rows of a product given as a list (k_spmm_list) instead of a row mask: rows[0 .. n), owner[r] = the entry
+// that computes row r.  n = 0: off.
+struct SpmmList {
+  const int64_t* rows;
+  const int32_t* owner;
+  int64_t n;
+};
+
 template <int G, int V, int UNR, int MINB, bool NZ, bool PUSH, bool HOT>
 static int launch_spmm(const cgx_csr* m, const float* val, const float* X, float* Y, const float* ACC_IN,
-                       float* ACC_OUT, float acc_scale, void* workspace, size_t workspace_bytes,
-                       cudaStream_t stream, const uint8_t* nz, const uint8_t* acc_nz, const uint8_t* out_rows,
-                       const SpmmPush ps) {
+                       float* ACC_OUT, const float* ACC_PREV, float acc_scale, void* workspace,
+                       size_t workspace_bytes, cudaStream_t stream, const uint8_t* nz, const uint8_t* acc_nz,
+                       const uint8_t* out_rows, const SpmmPush ps, const SpmmList ls) {
+  if constexpr (NZ && !PUSH && !HOT) {
+    if (ls.n > 0) {
+      k_spmm_list<G, V, UNR><<<(unsigned)ls.n, SP_THREADS, 0, stream>>>(
+          m->indptr, m->idx, val, m->n_rows, ls.rows, ls.owner, reinterpret_cast<const float4*>(X),
+          reinterpret_cast<float4*>(Y), reinterpret_cast<const float4*>(ACC_IN), reinterpret_cast<float4*>(ACC_OUT),
+          reinterpret_cast<const float4*>(ACC_PREV), acc_scale, nz, acc_nz);
+      CGX_LAUNCH_CHECK();
+      return CGX_OK;
+    }
+  }
   constexpr int GROUPS = SP_THREADS / G;
   float4* partial = nullptr;
   if (m->n_long > 0) {
@@ -411,19 +552,21 @@ static int launch_spmm(const cgx_csr* m, const float* val, const float* X, float
   cfg.numAttrs = 1;
   CGX_CUDA(cudaLaunchKernelEx(&cfg, k_spmm<G, V, UNR, MINB, NZ, PUSH, HOT>, HOT ? m->idx_hint : m->idx, val, items, sc,
                               reinterpret_cast<const float4*>(X), reinterpret_cast<float4*>(Y),
-                              reinterpret_cast<const float4*>(ACC_IN), reinterpret_cast<float4*>(ACC_OUT), acc_scale,
-                              partial, nz, acc_nz, out_rows, static_cast<const int4*>(m->work), ps));
+                              reinterpret_cast<const float4*>(ACC_IN), reinterpret_cast<float4*>(ACC_OUT),
+                              reinterpret_cast<const float4*>(ACC_PREV), acc_scale, partial, nz, acc_nz, out_rows,
+                              static_cast<const int4*>(m->work), ps));
   CGX_LAUNCH_CHECK();
   if (m->n_huge > 0) {
     k_spmm_finish<G, V><<<(unsigned)m->n_huge, SP_THREADS, 0, stream>>>(
         sc, partial, reinterpret_cast<float4*>(Y), reinterpret_cast<const float4*>(ACC_IN),
-        reinterpret_cast<float4*>(ACC_OUT), acc_scale, acc_nz, out_rows, ps);
+        reinterpret_cast<float4*>(ACC_OUT), reinterpret_cast<const float4*>(ACC_PREV), acc_scale, acc_nz, out_rows,
+        ps);
     CGX_LAUNCH_CHECK();
   }
   return CGX_OK;
 }
 
-#define CGX_SPMM_ARGS m, val, X, Y, ACC_IN, ACC_OUT, acc_scale, ws, ws_bytes, stream, nz, acc_nz, out_rows, ps
+#define CGX_SPMM_ARGS m, val, X, Y, ACC_IN, ACC_OUT, ACC_PREV, acc_scale, ws, ws_bytes, stream, nz, acc_nz, out_rows, ps, ls
 
 // Group geometry by regime (profiles/r1_spmm_variants.txt; the sweep itself lives in the round-1 history).
 // Gathered table in L2 (C2/C3: latency-bound): d/4 lanes per row, one float4 per lane, 8 gathers in flight.
@@ -433,9 +576,9 @@ static int launch_spmm(const cgx_csr* m, const float* val, const float* X, float
 // when the graph carries hot-row hints (cgx_hot_hints), per-row L2 eviction priorities.
 template <int G, int V, int UNR>
 static int spmm_flavour(const cgx_csr* m, const float* val, const float* X, float* Y, const float* ACC_IN,
-                        float* ACC_OUT, float acc_scale, void* ws, size_t ws_bytes, cudaStream_t stream,
-                        const uint8_t* nz, const uint8_t* acc_nz, const uint8_t* out_rows, const SpmmPush ps,
-                        bool hot) {
+                        float* ACC_OUT, const float* ACC_PREV, float acc_scale, void* ws, size_t ws_bytes,
+                        cudaStream_t stream, const uint8_t* nz, const uint8_t* acc_nz, const uint8_t* out_rows,
+                        const SpmmPush ps, const SpmmList ls, bool hot) {
   const bool push = ps.rows_per > 0;
   if constexpr (V == 2) {
     if (hot && nz == nullptr) {
@@ -451,18 +594,25 @@ static int spmm_flavour(const cgx_csr* m, const float* val, const float* X, floa
   return launch_spmm<G, V, UNR, 4, false, false, false>(CGX_SPMM_ARGS);
 }
 
-#define CGX_FLAVOUR_ARGS m, val, X, Y, ACC_IN, ACC_OUT, acc_scale, ws, ws_bytes, stream, nz, acc_nz, out_rows, ps, hot
+#define CGX_FLAVOUR_ARGS \
+  m, val, X, Y, ACC_IN, ACC_OUT, ACC_PREV, acc_scale, ws, ws_bytes, stream, nz, acc_nz, out_rows, ps, ls, hot
 
 static int spmm_dispatch(const cgx_csr* m, int use_bwd, int32_t d, const float* X, float* Y, const float* ACC_IN,
                          float* ACC_OUT, float acc_scale, void* ws, size_t ws_bytes, cudaStream_t stream,
                          const uint8_t* nz = nullptr, const SpmmPush ps = SpmmPush{0ull, 0, 0},
-                         const uint8_t* acc_nz = nullptr, const uint8_t* out_rows = nullptr) {
+                         const uint8_t* acc_nz = nullptr, const uint8_t* out_rows = nullptr,
+                         const float* ACC_PREV = nullptr, const SpmmList ls = SpmmList{nullptr, nullptr, 0}) {
   CGX_REQUIRE(m && m->perm && m->work && (m->nnz == 0 || (m->idx && m->val_fwd && m->val_bwd)) && X, CGX_ERR_ARG,
               "spmm: NULL pointer (cgx_csr needs idx, both value arrays and the cgx_row_schedule* outputs)");
   CGX_REQUIRE(m->n_long == 0 || (m->chunk_ptr && m->arrive), CGX_ERR_ARG, "spmm: chunk tables missing");
   CGX_REQUIRE(Y || ACC_OUT || ps.rows_per > 0, CGX_ERR_ARG, "spmm: no output requested");
   CGX_REQUIRE(out_rows == nullptr || (nz != nullptr && ps.rows_per == 0), CGX_ERR_ARG,
               "spmm: an output-row mask needs gather flags and no push mode");
+  // the masked instantiations are the ones that carry ACC_PREV (k_spmm) and the row list
+  CGX_REQUIRE((ACC_PREV == nullptr || (ACC_OUT != nullptr && (out_rows != nullptr || ls.n > 0))) &&
+                  (ls.n == 0 || (out_rows == nullptr && nz != nullptr && ps.rows_per == 0 && ls.rows && ls.owner &&
+                                 m->indptr && ls.n < (int64_t(1) << 31))),
+              CGX_ERR_ARG, "spmm: ACC_PREV needs an output-row mask or list; a row list needs gather flags");
   const float* val = use_bwd ? m->val_bwd : m->val_fwd;
   if (m->n_rows == 0) return CGX_OK;
   const bool beyond_l2 = int64_t(m->n_cols) * int64_t(d) * 4 > option(CGX_OPT_L2_TABLE_BYTES);
@@ -581,14 +731,14 @@ extern "C" int cgx_row_flags(const float* X, int64_t n_rows, int32_t d, uint8_t*
 }
 
 // Item frontier of a triple batch: flags[i] = 1 for i in pos, neg and the by_user rows of the batch users, and
-// (flags_u nullable) flags_u[u] = 1 for the batch users.  One warp per triple; duplicate users walk their row twice
-// (the stores are idempotent).  Out-of-range ids are clamped to 0, as cgx_bpr_plan does, so the frontier covers every
-// row that cgx_bpr_mark_rows flags.
-__device__ __forceinline__ int64_t clamp_row(int64_t x, int64_t n) { return (x < 0 || x >= n) ? 0 : x; }
+// (flags_u nullable) flags_u[u] = 1 for the batch users, (owner_u nullable) owner_u[u] = one of the t with
+// users[t] = u.  One warp per triple; duplicate users walk their row twice (the stores are idempotent).  Out-of-range
+// ids are clamped to 0, as cgx_bpr_plan does, so the frontier covers every row that cgx_bpr_mark_rows flags.
 __global__ void k_batch_frontier(const int64_t* __restrict__ indptr, const int32_t* __restrict__ idx,
                                  const int64_t* __restrict__ users, const int64_t* __restrict__ pos,
                                  const int64_t* __restrict__ neg, int64_t B, int32_t U, int32_t I,
-                                 uint8_t* __restrict__ flags, uint8_t* __restrict__ flags_u) {
+                                 uint8_t* __restrict__ flags, uint8_t* __restrict__ flags_u,
+                                 int32_t* __restrict__ owner_u) {
   const int64_t t = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) / 32;
   const int lane = threadIdx.x & 31;
   if (t >= B) return;
@@ -597,6 +747,7 @@ __global__ void k_batch_frontier(const int64_t* __restrict__ indptr, const int32
     flags[clamp_row(pos[t], I)] = 1;
     flags[clamp_row(neg[t], I)] = 1;
     if (flags_u != nullptr) flags_u[u] = 1;
+    if (owner_u != nullptr) owner_u[u] = int32_t(t);   // any writer wins; only batch entries are ever read
   }
   const int64_t end = indptr[u + 1];
   for (int64_t j = indptr[u] + lane; j < end; j += 32) flags[idx[j]] = 1;
@@ -604,7 +755,7 @@ __global__ void k_batch_frontier(const int64_t* __restrict__ indptr, const int32
 
 extern "C" int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64_t* pos,
                                   const int64_t* neg, int64_t B, uint8_t* flags_i, uint8_t* flags_u,
-                                  void* stream_) {
+                                  int32_t* owner_u, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(by_user && by_user->indptr && (by_user->nnz == 0 || by_user->idx) && users && pos && neg && flags_i,
               CGX_ERR_ARG, "batch_frontier: NULL pointer");
@@ -613,7 +764,7 @@ extern "C" int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, 
   CGX_CUDA(cudaMemsetAsync(flags_i, 0, size_t(by_user->n_cols), stream));
   if (flags_u != nullptr) CGX_CUDA(cudaMemsetAsync(flags_u, 0, size_t(by_user->n_rows), stream));
   k_batch_frontier<<<(unsigned)ceil_div(B * 32, 256), 256, 0, stream>>>(
-      by_user->indptr, by_user->idx, users, pos, neg, B, by_user->n_rows, by_user->n_cols, flags_i, flags_u);
+      by_user->indptr, by_user->idx, users, pos, neg, B, by_user->n_rows, by_user->n_cols, flags_i, flags_u, owner_u);
   CGX_LAUNCH_CHECK();
   return CGX_OK;
 }
@@ -641,22 +792,27 @@ extern "C" size_t cgx_propagate_workspace_bytes_for(const cgx_csr* by_user, cons
 extern "C" int cgx_propagate_fwd(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t K, int32_t d,
                                  const float* e0_u, const float* e0_i, float* out_u, float* out_i,
                                  void* workspace, size_t workspace_bytes, void* stream) {
-  return cgx_propagate_fwd_layers(by_user, by_item, order, K, d, e0_u, e0_i, out_u, out_i, 0, K, nullptr, nullptr,
-                                  nullptr, workspace, workspace_bytes, stream);
+  return cgx_propagate_fwd_layers(by_user, by_item, order, K, d, e0_u, e0_i, out_u, out_i, 0, K, 0, nullptr, nullptr,
+                                  nullptr, 0, nullptr, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int cgx_propagate_fwd_layers(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t K,
                                         int32_t d, const float* e0_u, const float* e0_i, float* out_u, float* out_i,
-                                        int32_t layer_begin, int32_t layer_end, const uint8_t* rows_u,
-                                        const uint8_t* rows_i, const uint8_t* all_rows, void* workspace,
+                                        int32_t layer_begin, int32_t layer_end, int fold, const uint8_t* rows_u,
+                                        const uint8_t* rows_i, const int64_t* list_u, int64_t n_list_u,
+                                        const int32_t* owner_u, const uint8_t* all_rows, void* workspace,
                                         size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(by_user && by_item && e0_u && e0_i && out_u && out_i, CGX_ERR_ARG, "propagate_fwd: NULL pointer");
   CGX_REQUIRE(K >= 1, CGX_ERR_ARG, "propagate_fwd: num_layers must be >= 1");
   CGX_REQUIRE(0 <= layer_begin && layer_begin <= layer_end && layer_end <= K, CGX_ERR_ARG,
               "propagate_fwd: layers [%d, %d) outside [0, %d)", layer_begin, layer_end, K);
-  CGX_REQUIRE((rows_u == nullptr && rows_i == nullptr) || all_rows != nullptr, CGX_ERR_ARG,
+  CGX_REQUIRE((rows_u == nullptr && rows_i == nullptr && list_u == nullptr) || all_rows != nullptr, CGX_ERR_ARG,
               "propagate_fwd: output-row masks need all_rows");
+  CGX_REQUIRE(list_u == nullptr || (rows_u == nullptr && owner_u != nullptr && n_list_u > 0), CGX_ERR_ARG,
+              "propagate_fwd: a user row list needs owner_u and no user row mask");
+  CGX_REQUIRE(!fold || (K >= 3 && (layer_end < K || ((rows_u != nullptr || list_u != nullptr) && rows_i != nullptr))),
+              CGX_ERR_ARG, "propagate_fwd: folding needs num_layers >= 3 and output-row masks on the last layer");
   CGX_REQUIRE(order == CGX_ORDER_JACOBI || order == CGX_ORDER_GS, CGX_ERR_ARG, "propagate_fwd: bad order");
   CGX_REQUIRE(by_user->n_rows == by_item->n_cols && by_user->n_cols == by_item->n_rows, CGX_ERR_ARG,
               "propagate_fwd: operator shapes disagree");
@@ -676,12 +832,18 @@ extern "C" int cgx_propagate_fwd_layers(const cgx_csr* by_user, const cgx_csr* b
   CGX_REQUIRE(ws.ok, CGX_ERR_WORKSPACE, "propagate_fwd: workspace too small");
   const float s = 1.0f / float(K + 1);
   const SpmmPush nops{0ull, 0, 0};
-  // The last layer writes only the output rows its masks flag (rows_u / rows_i, nullable).  A mask needs the
-  // row-sparse instantiation (spmm_dispatch); its gather flags are all_rows, all ones, so no entry is dropped and the
-  // sum is the unmasked one.  Layer k - 1's buffers are what layer k gathers, and the last layer writes no user
-  // buffer (and, in Jacobi order, no item buffer): a later call for the rows left out finds its inputs intact.
+  // The last layer writes only the output rows its masks flag (rows_u / rows_i, nullable), or the user rows of list_u.
+  // A mask or list needs the row-sparse instantiation (spmm_dispatch); its gather flags are all_rows, all ones, so no
+  // entry is dropped and the sum is the unmasked one.  Layer k - 1's buffers are what layer k gathers, and the last
+  // layer writes no user buffer (and, in Jacobi order, no item buffer): a later call for the rows left out finds its
+  // inputs intact.
+  // fold: layer K - 1 writes its buffers only, and the last layer adds them to the running sum of layers 0 .. K - 2
+  // (epilogue, ACC_PREV): out = s ((out + l_{K-1}) + l_K), the adds of the unfolded chain (1.0f (x) is exact), without
+  // a pass of the running sums over the whole tables for layer K - 1.  Layer K - 1's buffers are still l_{K-1} when
+  // the last layer reads them: in Gauss-Seidel order its item product writes i_K over i_{K-1} only at the row it has
+  // just read in the same epilogue (and writes no user buffer); in Jacobi order it writes no buffer.
   for (int k = layer_begin; k < layer_end; ++k) {
-    const bool first = k == 0, last = k == K - 1;
+    const bool first = k == 0, last = k == K - 1, folded = fold && k == K - 2;
     const float* cu = first ? e0_u : ub[(k - 1) & 1];   // layer k tables
     const float* ci = first ? e0_i : ib[(k - 1) & 1];
     float* nu = ub[k & 1];
@@ -689,14 +851,18 @@ extern "C" int cgx_propagate_fwd_layers(const cgx_csr* by_user, const cgx_csr* b
     const float sc = last ? s : 1.0f;
     const uint8_t* mu = last ? rows_u : nullptr;
     const uint8_t* mi = last ? rows_i : nullptr;
+    const SpmmList lu = last && list_u ? SpmmList{list_u, owner_u, n_list_u} : SpmmList{nullptr, nullptr, 0};
+    float* acc_i = folded ? nullptr : out_i;
+    float* acc_u = folded ? nullptr : out_u;
     // item side: i_{k+1} = C u_k
     const bool need_ni = !last || order == CGX_ORDER_GS;
-    CGX_TRY(spmm_dispatch(by_item, 0, d, cu, need_ni ? ni : nullptr, first ? e0_i : out_i, out_i, sc, lw, lws,
-                          stream, mi ? all_rows : nullptr, nops, nullptr, mi));
+    CGX_TRY(spmm_dispatch(by_item, 0, d, cu, need_ni ? ni : nullptr, first ? e0_i : acc_i, acc_i, sc, lw, lws,
+                          stream, mi ? all_rows : nullptr, nops, nullptr, mi, fold && last ? ci : nullptr));
     // user side: u_{k+1} = A i_k (Jacobi) or A i_{k+1} (Gauss-Seidel)
     const float* src = order == CGX_ORDER_JACOBI ? ci : ni;
-    CGX_TRY(spmm_dispatch(by_user, 0, d, src, last ? nullptr : nu, first ? e0_u : out_u, out_u, sc, lw, lws,
-                          stream, mu ? all_rows : nullptr, nops, nullptr, mu));
+    CGX_TRY(spmm_dispatch(by_user, 0, d, src, last ? nullptr : nu, first ? e0_u : acc_u, acc_u, sc, lw, lws,
+                          stream, mu || lu.n ? all_rows : nullptr, nops, nullptr, mu, fold && last ? cu : nullptr,
+                          lu));
   }
   return CGX_OK;
 }

@@ -102,17 +102,17 @@ def bpr_plan(graph: CredGraph, users, pos, neg, plan=None):
     return plan
 
 
-def batch_frontier(graph: CredGraph, users, pos, neg, flags=None, flags_u=None):
+def batch_frontier(graph: CredGraph, users, pos, neg, flags=None, flags_u=None, owner_u=None):
     """uint8[I]: 1 on the items of pos, neg and the train rows of the batch users (cgx_batch_frontier), the only
     rows where the first item-side adjoint of the batch's loss can be non-zero.  flags_u (uint8[U], optional) is
-    set to 1 on the batch users."""
+    set to 1 on the batch users, and owner_u (int32[U], optional) to one batch position of each batch user."""
     dev = graph.device
     users, pos, neg = _i64c(users, dev), _i64c(pos, dev), _i64c(neg, dev)
     if flags is None:
         flags = torch.empty(graph.num_items, dtype=torch.uint8, device=dev)
     with torch.cuda.device(dev):
         check(lib().cgx_batch_frontier(graph.by_user.ref(), ptr(users), ptr(pos), ptr(neg), users.numel(), ptr(flags),
-                                       ptr(flags_u), stream_ptr(dev)))
+                                       ptr(flags_u), ptr(owner_u), stream_ptr(dev)))
     return flags
 
 
@@ -392,7 +392,9 @@ class TrainStep:
     the pos / neg rows of f_i, so when the item table is beyond L2 (the SpMM's regime switch), num_layers >= 2 and
     the device has room for a second forward workspace ((U + I) d floats) with DEFER_HEADROOM to spare, the step
     computes the last layer's products only on the batch users and on the item frontier (pos, neg and the
-    batch users' train items: all that the batch users' last-layer rows gather).  The first read of `f_u` or `f_i`
+    batch users' train items: all that the batch users' last-layer rows gather), the user rows from the batch list
+    itself; with num_layers >= 3 it also adds layer K - 1 into the final tables only there (cgx_propagate_fwd_layers,
+    fold).  The first read of `f_u` or `f_i`
     after a step computes the other rows, on the current stream, with the same bits as an eager forward.  The
     properties return the same tensor objects every time: a reference held across a later step() is not completed
     by it; read the attribute again."""
@@ -428,7 +430,7 @@ class TrainStep:
         # Deferred last layer: decided by the first forward (_defers_final).  Its layer buffers must survive the
         # backward, which overwrites the graph's shared workspace, so the deferred path owns a forward workspace.
         self._defer_final = None
-        self._fws = self._all_rows = None
+        self._fws = self._all_rows = self._owner_u = None
         self._pending = False         # f_u / f_i lack the rows outside the last step's masks
         self._final_error = None      # a failed completion: f_u / f_i are unusable until the next step
 
@@ -472,9 +474,9 @@ class TrainStep:
             rest_i = torch.eq(self.front_i, 0).view(torch.uint8)
             try:
                 check(lib().cgx_propagate_fwd_layers(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
-                                                     ptr(self._f_u), ptr(self._f_i), K - 1, K, ptr(rest_u),
-                                                     ptr(rest_i), ptr(self._all_rows), ptr(self._fws),
-                                                     self._fws.numel(), stream_ptr(dev)))
+                                                     ptr(self._f_u), ptr(self._f_i), K - 1, K, int(K >= 3),
+                                                     ptr(rest_u), ptr(rest_i), None, 0, None, ptr(self._all_rows),
+                                                     ptr(self._fws), self._fws.numel(), stream_ptr(dev)))
             except _lib.CgxError as e:
                 # part of the rows may have been added already, so a retry could add them twice: every read raises
                 # until the next step recomputes the tables
@@ -512,6 +514,8 @@ class TrainStep:
             self._fws = workspace(lib().cgx_propagate_workspace_bytes_for(g.by_user.ref(), g.by_item.ref(), d, order),
                                   dev)
             self._all_rows = torch.ones(max(g.num_users, g.num_items), dtype=torch.uint8, device=dev)
+            self._owner_u = torch.empty(g.num_users, dtype=torch.int32, device=dev)
+        fold = int(defer and K >= 3)       # K = 2: folding layer 1 would need E^0 after Adam
         front = self.front_i if beyond_l2 or defer else None
         marks = []
         self._pending, self._final_error = False, None
@@ -522,19 +526,20 @@ class TrainStep:
             with torch.cuda.stream(self.side):
                 bpr_plan(g, users, pos, neg, plan)      # scatter plan: beside the forward
                 if front is not None:
-                    batch_frontier(g, users, pos, neg, front, self.batch_u if defer else None)
+                    batch_frontier(g, users, pos, neg, front, *((self.batch_u, self._owner_u) if defer else ()))
             st = stream_ptr(dev)
             if defer:
-                # layers 1..K-1 beside the plan and frontier, then layer K on the rows the loss reads
+                # layers 1..K-1 beside the plan and frontier, then layer K on the rows the loss reads: the item
+                # frontier, and the batch users straight from the batch list (a grid of B blocks)
                 fws = self._fws
                 check(lib().cgx_propagate_fwd_layers(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
-                                                     ptr(self._f_u), ptr(self._f_i), 0, K - 1, None, None, None,
-                                                     ptr(fws), fws.numel(), st))
+                                                     ptr(self._f_u), ptr(self._f_i), 0, K - 1, fold, None, None, None,
+                                                     0, None, None, ptr(fws), fws.numel(), st))
                 main.wait_stream(self.side)
                 check(lib().cgx_propagate_fwd_layers(g.by_user.ref(), g.by_item.ref(), order, K, d, ptr(eu), ptr(ei),
-                                                     ptr(self._f_u), ptr(self._f_i), K - 1, K, ptr(self.batch_u),
-                                                     ptr(self.front_i), ptr(self._all_rows), ptr(fws), fws.numel(),
-                                                     st))
+                                                     ptr(self._f_u), ptr(self._f_i), K - 1, K, fold, None,
+                                                     ptr(self.front_i), ptr(users), users.numel(), ptr(self._owner_u),
+                                                     ptr(self._all_rows), ptr(fws), fws.numel(), st))
                 self._mark(marks)
                 self._pending = True
             else:

@@ -230,12 +230,19 @@ int cgx_propagate_fwd(const cgx_csr* by_user, const cgx_csr* by_item, int order,
  * running sum of layers 0..K-1.  Masked rows can be computed later by a call for layer K-1 alone with the
  * complementary masks on the same workspace: the last layer's inputs are not overwritten by it, and the final
  * tables then carry the bits of cgx_propagate_fwd.  all_rows: uint8[max(U, I)], every entry 1, needed with a mask.
+ * list_u int64[n_list_u] (nullable, instead of rows_u): the last layer's user product computes the rows list_u[t]
+ * (ids out of range count as 0) whose owner_u[list_u[t]] == t -- cgx_batch_frontier writes owner_u -- with a grid
+ * of n_list_u blocks; every other user row is left as rows_u would leave an unflagged one.
  * (The last layer adds into out_* in place: computing a row twice adds it twice.)  The completing call picks its
  * SpMM geometry from the options current when it runs (CGX_OPT_L2_TABLE_BYTES): change none between the two calls,
- * or the completed rows may differ from cgx_propagate_fwd in the last bits. */
+ * or the completed rows may differ from cgx_propagate_fwd in the last bits.
+ * fold != 0 (num_layers >= 3; every call of one forward passes the same value, and the last layer has masks):
+ * layer num_layers - 1 does not add into out_*, and the last layer adds it in its epilogue instead, with the same
+ * bits -- the running sums of that layer are not streamed over the whole tables. */
 int cgx_propagate_fwd_layers(const cgx_csr* by_user, const cgx_csr* by_item, int order, int32_t num_layers,
                              int32_t d, const float* e0_u, const float* e0_i, float* out_u, float* out_i,
-                             int32_t layer_begin, int32_t layer_end, const uint8_t* rows_u, const uint8_t* rows_i,
+                             int32_t layer_begin, int32_t layer_end, int fold, const uint8_t* rows_u,
+                             const uint8_t* rows_i, const int64_t* list_u, int64_t n_list_u, const int32_t* owner_u,
                              const uint8_t* all_rows, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Backward: (g_u, g_i) = dL/d(out_u, out_i) dense -> (d_e0_u, d_e0_i).  SURVEY.md appendix C. */
@@ -263,10 +270,11 @@ int cgx_propagate_bwd_frontier(const cgx_csr* by_user, const cgx_csr* by_item, i
  * loss.backward(), CU:651 / V2:862, can make non-zero): flags_i uint8[num_items] is zeroed, then set for pos[t],
  * neg[t] and every column of by_user row users[t], t < batch.  users / pos / neg int64[batch] (device); ids out of
  * range count as 0, as in cgx_bpr_plan.  flags_u uint8[num_users] (nullable) is zeroed and set for users[t]: the
- * user rows the loss reads.  Depends on the indices only: it can run on a side stream beside the forward
- * propagation, as cgx_bpr_plan does. */
+ * user rows the loss reads.  owner_u int32[num_users] (nullable; not zeroed): owner_u[users[t]] = one t of each
+ * batch user, for the user row list of cgx_propagate_fwd_layers.  Depends on the indices only: it can run on a side
+ * stream beside the forward propagation, as cgx_bpr_plan does. */
 int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64_t* pos, const int64_t* neg,
-                       int64_t batch, uint8_t* flags_i, uint8_t* flags_u, void* stream);
+                       int64_t batch, uint8_t* flags_i, uint8_t* flags_u, int32_t* owner_u, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * BPR + L2 (+ fairness) on a batch of (user, pos, neg) triples.  Replaces score / l2_reg / the loss

@@ -3,7 +3,7 @@
     python profiles/frontier.py stats OUT.json [--batches N]        (GPU)  |F|, its edges and its hot-set share
     python profiles/frontier.py kernels OUT.json [--tree DIR]       (GPU)  torch.profiler times of one eager C4 step
     python profiles/frontier.py reads OUT.json                      (GPU)  what reading TrainStep.f_u costs; C2 deferral
-    python profiles/frontier.py traffic STATS.json                  (CPU)  rewrite launches 5 - 8 of r2_traffic.json
+    python profiles/frontier.py traffic STATS.json                  (CPU)  rewrite launches 3 - 8 of r2_traffic.json
 
 The frontier F of a batch is pos + neg + the train items of the batch users (cgx_batch_frontier): the only rows where
 the first item-side adjoint bi' = g_i + A^T g_u can be non-zero.  `stats` builds the C4 graph and the sampler exactly
@@ -197,17 +197,28 @@ def traffic(args):
     # gathers u_{K-1} along the edges of F's rows: it is charged the captured launch's DRAM bytes per edge net of its
     # streams (descriptors, three d-wide row streams), times the edges of F; plus every descriptor, the first batch of
     # column ids / values of the rows outside F, F's three row streams, and the flag arrays (all-ones gather flags
-    # over users, the mask over items).  Launch 6: every descriptor, the first batch of every row outside the batch,
-    # the batch rows' idx + val, gathered rows and two row streams (ACC_IN, ACC_OUT), and the flag arrays.
+    # over users, the mask over items).  Since r6 launch 5 also reads layer K - 1's rows of F (the folded running
+    # sum: four row streams), and launch 6 runs over the batch list (k_spmm_list): per batch user its indptr pair,
+    # owner entry and list entry (a 32-byte sector each), its idx + val, gathered rows and three row streams (ACC_IN,
+    # layer K - 1, ACC_OUT), and the gather flags of its edges -- no descriptor of any other row.
+    # Launches 3 and 4 (layer K - 1 = 2), r6: the layer writes its buffers only, so each is charged its capture net of
+    # the running-sum streams it no longer reads and writes (2 d floats per output row).
     l5_cap = c4["launches"][4].get("captured_before_frontier", c4["launches"][4])
     desc_i = 16 * (st["item_chunks"] + I - st["item_rows_long"])
-    desc_u = 16 * (st["user_chunks"] + U - st["user_rows_long"])
     per_edge = (l5_cap["gb"] * 1e9 - desc_i - 3 * row * I) / E
-    l5 = desc_i + 64 * out_items + per_edge * m["front_edges"] + 3 * row * m["front_items"] + U + I
+    l5 = desc_i + 64 * out_items + per_edge * m["front_edges"] + 4 * row * m["front_items"] + U + I
     bu_edges = B * E / U
-    l6 = desc_u + 64 * (U - B) + (8 + row) * bu_edges + 2 * row * B + U + I
+    l6 = 3 * 32 * B + (8 + row) * bu_edges + 3 * row * B + 8 * B + bu_edges
+    for i, rows in ((2, I), (3, U)):
+        old = c4["launches"][i]
+        cap = old.get("captured_before_fold", old)
+        c4["launches"][i] = dict(kernel=old["kernel"], gb=round((cap["gb"] * 1e9 - 2 * row * rows) / 1e9, 3),
+                                 computed=True, what="layer K - 1: layer buffers only (running sum folded into "
+                                 "layer K)", source="capture net of the running-sum streams (frontier.py traffic)",
+                                 captured_before_fold=dict(ms=cap.get("ms"), gb=cap["gb"],
+                                                           l2_hit_pct=cap.get("l2_hit_pct")))
     for i, gb, kind in ((4, l5, "last forward hop: item rows masked by the batch's item frontier F"),
-                        (5, l6, "last forward hop: user rows masked by the batch users"),
+                        (5, l6, "last forward hop: the batch users' rows from the batch list"),
                         (6, l7, "item rows masked by the batch's item frontier F"),
                         (7, l8, "user rows gathering only the rows of F")):
         old = c4["launches"][i]
@@ -218,14 +229,19 @@ def traffic(args):
                                  if "captured_before_frontier" not in old else old["captured_before_frontier"])
     for i in range(4, 8):
         c4["launches"][i]["kernel"] = "k_spmm<16, 2, 4, 4, 1, 0, 0>"
+    c4["launches"][5]["kernel"] = "k_spmm_list<16, 2, 4>"
     c4["bytes_per_step"] = sum(l["gb"] for l in c4["launches"]) * 1e9
     c4["source"] = ("computed: ncu --set full of bench.py's eager step (profiles/r2_ncu_spmm_c4.txt) for launches "
-                    f"1-4 and 9-12, bytes computed from the measured item frontier ({src}) for launches 5-8")
-    c4["note"] = ("launches 5 and 6 (the last forward hop) and 7 and 8 (the Gauss-Seidel adjoint at k = 0) are "
-                  "computed, not captured: they now touch only the batch's item frontier (and, launch 6, the batch "
-                  "users); their capture before that change is kept under captured_before_frontier")
+                    f"1-2 and 9-12, net of the folded running sums for launches 3-4, bytes computed from the measured "
+                    f"item frontier ({src}) for launches 5-8")
+    c4["note"] = ("launches 3 and 4 (layer K - 1, r6: buffers only) are their capture net of the running-sum "
+                  "streams, kept under captured_before_fold; launches 5 and 6 (the last forward hop) and 7 and 8 "
+                  "(the Gauss-Seidel adjoint at k = 0) are computed, not captured: they now touch only the batch's "
+                  "item frontier (and, launch 6, the batch users from the batch list); their capture before that "
+                  "change is kept under captured_before_frontier")
     path.write_text(json.dumps(data, indent=1))
-    print(f"launch 5: {l5 / 1e9:.3f} GB, launch 6: {l6 / 1e9:.3f} GB, launch 7: {l7 / 1e9:.3f} GB, "
+    print(f"launches 3 / 4: {c4['launches'][2]['gb']:.3f} / {c4['launches'][3]['gb']:.3f} GB, "
+          f"launch 5: {l5 / 1e9:.3f} GB, launch 6: {l6 / 1e9:.3f} GB, launch 7: {l7 / 1e9:.3f} GB, "
           f"launch 8: {l8 / 1e9:.3f} GB, step: {c4['bytes_per_step'] / 1e9:.1f} GB")
 
 

@@ -80,20 +80,21 @@ _SIGNATURES = {
                                             C.c_size_t, _P]),
     "cgx_propagate_bwd_frontier": (C.c_int, [_CSR, _CSR, C.c_int, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P,
                                              _P, _P, C.c_size_t, _P]),
-    "cgx_batch_frontier": (C.c_int, [_CSR, _P, _P, _P, C.c_int64, _P, _P, _P, _P]),
+    "cgx_batch_frontier": (C.c_int, [_CSR, _P, _P, _P, C.c_int64, _P, _P, _P, _P, _P]),
     "cgx_bpr_mark_rows": (C.c_int, [_P, C.c_int64, C.c_int32, _P, _P, _P]),
     "cgx_bpr_clear_rows": (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "cgx_bpr_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32, C.c_int32]),
     "cgx_bpr_plan_workspace_bytes": (C.c_size_t, [C.c_int64]),
-    "cgx_bpr_plan": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P, C.c_size_t, _P]),
+    "cgx_bpr_plan": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P, C.c_size_t, _P, _P]),
     "cgx_bpr_fwd_bwd": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P,
                                   _P, _P,
-                                  C.c_float, C.c_float, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
+                                  C.c_float, C.c_float, _P, _P, _P, _P, _P, _P, C.c_size_t, _P, _P, _P]),
     "cgx_bpr_apply_ego": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "cgx_sampler_build_workspace_bytes": (C.c_size_t, [C.c_int32]),
     "cgx_sampler_build": (C.c_int, [_P, C.c_int32, C.c_double, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
     "cgx_sample_triples": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int32, _P, _P, _P, _P, _P, C.c_float,
-                                     C.c_int32, C.c_uint64, C.c_uint64, _P, _P, _P, _P]),
+                                     C.c_int32, C.c_uint64, C.c_uint64, _P, _P, _P, _P, _P, _P]),
+    "cgx_batch_select": (C.c_int, [_P, C.c_int64, _P, C.c_int64, C.c_int64, C.c_int64, _P, _P, _P, _P, _P]),
     "cgx_tick": (C.c_int, [_P, _P]),
     "cgx_adam_step": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_int64, C.c_float, C.c_float,
                                 C.c_float, C.c_float, _P, C.c_int64, _P]),
@@ -118,7 +119,8 @@ _SIGNATURES = {
     "cgx_eval_topk": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int32, C.c_int32, _P, _P, C.c_int32, C.c_int, _P,
                                 _P, _P, C.c_size_t, _P]),
     "cgx_score_candidates": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, _P]),
-    "cgx_eval_candidates": (C.c_int, [_P, C.c_int64, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_uint64, _P, _P]),
+    "cgx_eval_candidates": (C.c_int, [_P, C.c_int64, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_uint64, _P, _P,
+                                      C.c_int64]),
     "cgx_rank_candidates": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, _P]),
     "cgx_eval_topk_uses_tensor_cores": (C.c_int, [C.c_int32, C.c_int32, C.c_int]),
     "cgx_eval_metrics_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),

@@ -40,21 +40,24 @@ __device__ __forceinline__ float dot4(const float4& a, const float4& b) {
 
 __device__ __forceinline__ int64_t clamp_id(int64_t x, int64_t n) { return (x < 0 || x >= n) ? 0 : x; }
 
-// key of entry e (0..3B): row in the high bits (items offset by U), entry id in the low bits
+// key of entry e (0..3B): row in the high bits (items offset by U), entry id in the low bits; an entry of a triple
+// t >= cnt (absent) gets the row U + I, behind every real row
 __device__ __forceinline__ uint64_t plan_key(const int64_t* __restrict__ users, const int64_t* __restrict__ pos,
-                                             const int64_t* __restrict__ neg, int64_t B, int32_t U, int32_t I,
-                                             int entry_bits, int64_t e) {
+                                             const int64_t* __restrict__ neg, int64_t B, int64_t cnt, int32_t U,
+                                             int32_t I, int entry_bits, int64_t e) {
   const int type = int(e / B);
   const int64_t t = e - int64_t(type) * B;
-  const int64_t row = type == 0 ? clamp_id(users[t], U) : int64_t(U) + clamp_id(type == 1 ? pos[t] : neg[t], I);
+  const int64_t row = t >= cnt ? int64_t(U) + I
+                    : type == 0 ? clamp_id(users[t], U) : int64_t(U) + clamp_id(type == 1 ? pos[t] : neg[t], I);
   return (uint64_t(row) << entry_bits) | uint64_t(e);
 }
 
 __global__ void k_plan_keys(const int64_t* __restrict__ users, const int64_t* __restrict__ pos,
-                            const int64_t* __restrict__ neg, int64_t B, int32_t U, int32_t I, int entry_bits,
-                            uint64_t* __restrict__ keys) {
+                            const int64_t* __restrict__ neg, int64_t B, const int64_t* __restrict__ count, int32_t U,
+                            int32_t I, int entry_bits, uint64_t* __restrict__ keys) {
   const int64_t e = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (e < 3 * B) keys[e] = plan_key(users, pos, neg, B, U, I, entry_bits, e);
+  const int64_t cnt = count != nullptr ? *count : B;
+  if (e < 3 * B) keys[e] = plan_key(users, pos, neg, B, cnt, U, I, entry_bits, e);
 }
 
 // ---- single-CTA stable radix sort of up to PS_MAX keys on the row bits -------------------------
@@ -65,7 +68,8 @@ constexpr int PS_MAX = PS_THREADS * PS_STEPS;  // 12288 keys = 3 * 4096
 
 __global__ void __launch_bounds__(PS_THREADS, 1) k_plan_small(const int64_t* __restrict__ users,
                                                               const int64_t* __restrict__ pos,
-                                                              const int64_t* __restrict__ neg, int64_t B, int32_t U,
+                                                              const int64_t* __restrict__ neg, int64_t B,
+                                                              const int64_t* __restrict__ count, int32_t U,
                                                               int32_t I, int entry_bits, int row_bits,
                                                               uint64_t* __restrict__ sorted) {
   extern __shared__ __align__(16) unsigned char ps_smem[];
@@ -76,7 +80,8 @@ __global__ void __launch_bounds__(PS_THREADS, 1) k_plan_small(const int64_t* __r
   const int n = int(3 * B);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint32_t lt = (1u << lane) - 1u;
-  for (int e = threadIdx.x; e < n; e += PS_THREADS) buf0[e] = plan_key(users, pos, neg, B, U, I, entry_bits, e);
+  const int64_t n_real = count != nullptr ? *count : B;
+  for (int e = threadIdx.x; e < n; e += PS_THREADS) buf0[e] = plan_key(users, pos, neg, B, n_real, U, I, entry_bits, e);
   __syncthreads();
   uint64_t* src = buf0;
   uint64_t* dst = buf1;
@@ -149,6 +154,8 @@ struct BprArgs {
   const int64_t* neg;
   int64_t B;
   int64_t B_total;   // denominator of the means (== B unless the batch is sharded over ranks)
+  const int64_t* count;      // nullable: triples t >= *count are absent (padding of a sharded batch)
+  const int64_t* total_dev;  // nullable: the denominator read from the device instead of B_total
   int32_t U, I;
   const float4* f_u;
   const float4* f_i;
@@ -157,6 +164,11 @@ struct BprArgs {
   const float* pop;
   float reg, fair;
 };
+
+__device__ __forceinline__ int64_t bpr_count(const BprArgs& a) { return a.count != nullptr ? *a.count : a.B; }
+__device__ __forceinline__ float bpr_total(const BprArgs& a) {
+  return float(a.total_dev != nullptr ? *a.total_dev : a.B_total);
+}
 
 // per triple: scores, loss term, coefficients
 template <int G, int V>
@@ -168,6 +180,10 @@ __global__ void __launch_bounds__(BP_THREADS) k_bpr_triple(BprArgs a, float* __r
   const int lane = threadIdx.x & (G - 1);
   const int64_t t = (int64_t(blockIdx.x) * BP_THREADS + threadIdx.x) / G;
   if (t >= a.B) return;
+  if (t >= bpr_count(a)) {                 // absent: no term, no index check
+    if ((threadIdx.x & (G - 1)) == 0) loss_term[t] = 0.f;
+    return;
+  }
   const unsigned mask = bp_group_mask<G>();
   int64_t u = a.users[t], p = a.pos[t], n = a.neg[t];
   if (u < 0 || u >= a.U || p < 0 || p >= a.I || n < 0 || n >= a.I) {
@@ -192,7 +208,7 @@ __global__ void __launch_bounds__(BP_THREADS) k_bpr_triple(BprArgs a, float* __r
   yn = group_sum<G>(yn, mask);
   l2 = group_sum<G>(l2, mask);
   if (lane == 0) {
-    const float invB = 1.0f / float(a.B_total);
+    const float invB = 1.0f / bpr_total(a);
     const float x = yp - yn;
     const float sig = 1.0f / (1.0f + expf(-x));
     const float term = -logf(sig + 1e-12f);                      // lightgcn_cu.py:637 (epsilon form)
@@ -228,6 +244,10 @@ __global__ void __launch_bounds__(BP_THREADS) k_bpr_scatter(BprArgs a, int entry
   const int64_t k = (int64_t(blockIdx.x) * BP_THREADS + threadIdx.x) / G;
   const int64_t n = 3 * a.B;
   if (k >= n) return;
+  if (k >= 3 * bpr_count(a)) {             // absent entries sort last: no row
+    if (lane == 0) ego_rows[k] = -1;
+    return;
+  }
   const uint64_t emask = (uint64_t(1) << entry_bits) - 1;
   const uint64_t key = keys[k];
   const int64_t row = int64_t(key >> entry_bits);
@@ -313,7 +333,7 @@ __global__ void __launch_bounds__(BP_THREADS) k_bpr_scatter(BprArgs a, int entry
     for (int v = 0; v < V; ++v) dst[v * G + lane] = acc[v];
     if (lane == 0) {
       ego_rows[k] = int32_t(row);
-      ego_coef[k] = float(mult) * 2.0f * a.reg / float(a.B_total);
+      ego_coef[k] = float(mult) * 2.0f * a.reg / bpr_total(a);
     }
     return;
   }
@@ -381,7 +401,7 @@ __global__ void __launch_bounds__(BP_THREADS) k_bpr_combine(BprArgs a, int entry
   for (int v = 0; v < V; ++v) dst[v * G + lane] = acc[v];
   if (lane == 0) {
     ego_rows[k] = int32_t(row);
-    ego_coef[k] = float(mult) * 2.0f * a.reg / float(a.B_total);
+    ego_coef[k] = float(mult) * 2.0f * a.reg / bpr_total(a);
   }
 }
 
@@ -495,14 +515,16 @@ using namespace cgx;
 extern "C" size_t cgx_bpr_plan_workspace_bytes(int64_t batch) { return plan_ws(batch); }
 
 extern "C" int cgx_bpr_plan(const int64_t* users, const int64_t* pos, const int64_t* neg, int64_t batch, int32_t U,
-                            int32_t I, uint64_t* plan, void* workspace, size_t workspace_bytes, void* stream_) {
+                            int32_t I, uint64_t* plan, void* workspace, size_t workspace_bytes, void* stream_,
+                            const int64_t* count) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(users && pos && neg && plan, CGX_ERR_ARG, "bpr_plan: NULL pointer");
   CGX_REQUIRE(batch > 0 && batch < (int64_t(1) << 29), CGX_ERR_ARG, "bpr_plan: bad batch size %lld",
               (long long)batch);
   CGX_REQUIRE(workspace_bytes >= plan_ws(batch), CGX_ERR_WORKSPACE, "bpr_plan: workspace too small");
   const int64_t n = 3 * batch;
-  const int entry_bits = bits_for(n), row_bits = bits_for(int64_t(U) + I);
+  // with a count, absent entries take the row U + I
+  const int entry_bits = bits_for(n), row_bits = bits_for(int64_t(U) + I + (count != nullptr ? 1 : 0));
   if (n <= PS_MAX) {
     const size_t smem = plan_small_smem();
     // the shared-memory opt-in is a per-DEVICE attribute: set it once per device (a bit per ordinal), which also
@@ -515,7 +537,7 @@ extern "C" int cgx_bpr_plan(const int64_t* users, const int64_t* pos, const int6
       CGX_CUDA(cudaFuncSetAttribute(k_plan_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       attr_set.fetch_or(bit, std::memory_order_release);
     }
-    k_plan_small<<<1, PS_THREADS, smem, stream>>>(users, pos, neg, batch, U, I, entry_bits, row_bits, plan);
+    k_plan_small<<<1, PS_THREADS, smem, stream>>>(users, pos, neg, batch, count, U, I, entry_bits, row_bits, plan);
     CGX_LAUNCH_CHECK();
     return CGX_OK;
   }
@@ -524,7 +546,7 @@ extern "C" int cgx_bpr_plan(const int64_t* users, const int64_t* pos, const int6
   size_t sort_bytes = radix_sort_temp_bytes(n);
   void* sort_tmp = ws.take<char>(sort_bytes);
   CGX_REQUIRE(ws.ok, CGX_ERR_WORKSPACE, "bpr_plan: workspace too small");
-  k_plan_keys<<<(unsigned)ceil_div(n, 256), 256, 0, stream>>>(users, pos, neg, batch, U, I, entry_bits, plan);
+  k_plan_keys<<<(unsigned)ceil_div(n, 256), 256, 0, stream>>>(users, pos, neg, batch, count, U, I, entry_bits, plan);
   CGX_LAUNCH_CHECK();
   uint64_t* sorted = plan;
   CGX_TRY(radix_sort_u64(plan, alt, n, entry_bits + row_bits, sort_tmp, sort_bytes, stream, &sorted));
@@ -540,14 +562,14 @@ extern "C" int cgx_bpr_fwd_bwd(const int64_t* users, const int64_t* pos, const i
                                const float* f_i, const float* e0_u, const float* e0_i, const float* pop,
                                float reg_weight, float fair_weight, float* loss_out, float* g_u, float* g_i,
                                int32_t* ego_rows, float* ego_coef, void* workspace, size_t workspace_bytes,
-                               void* stream_) {
+                               void* stream_, const int64_t* count, const int64_t* batch_total_dev) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(users && pos && neg && plan && f_u && f_i && e0_u && e0_i && loss_out && g_u && g_i && ego_rows &&
                   ego_coef,
               CGX_ERR_ARG, "bpr: NULL pointer");
   CGX_REQUIRE(batch > 0 && batch < (int64_t(1) << 29), CGX_ERR_ARG, "bpr: bad batch size %lld", (long long)batch);
   CGX_REQUIRE(workspace_bytes >= bpr_ws(batch), CGX_ERR_WORKSPACE, "bpr: workspace too small");
-  BprArgs a{users, pos, neg, batch, batch_total > 0 ? batch_total : batch, U, I,
+  BprArgs a{users, pos, neg, batch, batch_total > 0 ? batch_total : batch, count, batch_total_dev, U, I,
             reinterpret_cast<const float4*>(f_u),
             reinterpret_cast<const float4*>(f_i), reinterpret_cast<const float4*>(e0_u),
             reinterpret_cast<const float4*>(e0_i), pop, reg_weight, fair_weight};

@@ -61,22 +61,27 @@ __global__ void __launch_bounds__(SM_THREADS) k_sample(const int64_t* __restrict
                                                        SamplerTables tb, float mix_pop, int32_t max_tries,
                                                        uint64_t seed, uint64_t offset,
                                                        const unsigned long long* __restrict__ offset_dev,
+                                                       const int64_t* __restrict__ slots,
+                                                       const int64_t* __restrict__ count,
                                                        int64_t* __restrict__ pos_out, int64_t* __restrict__ neg_out) {
-  const int64_t t = int64_t(blockIdx.x) * SM_THREADS + threadIdx.x;
-  if (t >= B) return;
+  const int64_t i = int64_t(blockIdx.x) * SM_THREADS + threadIdx.x;
+  if (i >= B || (count != nullptr && i >= *count)) return;   // past the device count: absent, nothing written
+  // the Philox stream of an entry is keyed by its slot of the (global) batch: a rank holding part of a batch draws
+  // exactly what a whole-batch call draws for the same user
+  const int64_t t = slots != nullptr ? slots[i] : i;
   if (offset_dev != nullptr) offset += *offset_dev;   // device-side step counter (CUDA-graph replay)
   const Philox rng{uint32_t(seed), uint32_t(seed >> 32)};
   const uint32_t o_lo = uint32_t(offset), o_hi = uint32_t(offset >> 32);
   // counter = (slot, draw index, offset.lo, offset.hi); draw 0 is the positive
-  const int64_t u = users[t];
+  const int64_t u = users[i];
   const int64_t lo = __ldg(indptr + u), hi = __ldg(indptr + u + 1);
   if (hi <= lo) {  // caller contract: batch users own >= 1 train item (lightgcn_cu.py:592)
-    pos_out[t] = -1;
-    neg_out[t] = -1;
+    pos_out[i] = -1;
+    neg_out[i] = -1;
     return;
   }
   uint4 r = rng(uint32_t(t), 0u, o_lo, o_hi ^ uint32_t(t >> 32));
-  pos_out[t] = int64_t(__ldg(idx + lo + int64_t(bounded(u64_of(r.x, r.y), uint64_t(hi - lo)))));
+  pos_out[i] = int64_t(__ldg(idx + lo + int64_t(bounded(u64_of(r.x, r.y), uint64_t(hi - lo)))));
   const bool popmix = mix_pop >= 0.f;
   const int32_t D = popmix ? __ldg(tb.n_classes) : 0;
   int32_t item = 0;
@@ -93,7 +98,7 @@ __global__ void __launch_bounds__(SM_THREADS) k_sample(const int64_t* __restrict
     }
     if (!row_has(idx, lo, hi, item)) break;
   }
-  neg_out[t] = int64_t(item);
+  neg_out[i] = int64_t(item);
 }
 
 // ---- sampled-evaluation candidates: 1 test positive + n_neg negatives outside test U train ----------
@@ -103,13 +108,14 @@ __global__ void __launch_bounds__(SM_THREADS) k_eval_candidates(const int64_t* _
                                                                 const int32_t* __restrict__ tr_idx,
                                                                 const int64_t* __restrict__ te_indptr,
                                                                 const int32_t* __restrict__ te_idx, int32_t I,
-                                                                int32_t n_cand, uint64_t seed,
+                                                                int32_t n_cand, uint64_t seed, int64_t row_base,
                                                                 int64_t* __restrict__ cand) {
   const int64_t t = int64_t(blockIdx.x) * SM_THREADS + threadIdx.x;
   if (t >= n_users * n_cand) return;
-  const int64_t r = t / n_cand;
-  const int slot = int(t - r * n_cand);
-  const int64_t u = users[r];
+  const int64_t rl = t / n_cand;
+  const int slot = int(t - rl * n_cand);
+  const int64_t u = users[rl];
+  const int64_t r = row_base + rl;   // streams are keyed by the row of the whole list
   const Philox rng{uint32_t(seed), uint32_t(seed >> 32)};
   const int64_t te_lo = __ldg(te_indptr + u), te_hi = __ldg(te_indptr + u + 1);
   if (slot == 0) {   // the positive: uniform over the user's test items (callers pass users with >= 1 test item)
@@ -125,6 +131,66 @@ __global__ void __launch_bounds__(SM_THREADS) k_eval_candidates(const int64_t* _
     if (!row_has(te_idx, te_lo, te_hi, item) && !row_has(tr_idx, tr_lo, tr_hi, item)) break;
   }
   cand[t] = int64_t(item);
+}
+
+// ---- batch selection of a user-sharded epoch: one CTA per batch ---------------------------------------------------
+// Global batch s is perm[s B, min((s + 1) B, n_train)).  The entries whose user lies in [lo, hi) are compacted in
+// batch order (a block-wide exclusive scan of per-thread counts), rebased to local ids, and given their slot in the
+// global batch -- the slot keys the sampler's Philox stream.
+constexpr int BS_THREADS = 1024;
+constexpr int BS_PER = 4;
+constexpr int64_t BS_MAX = int64_t(BS_THREADS) * BS_PER;
+
+__global__ void __launch_bounds__(BS_THREADS) k_batch_select(const int64_t* __restrict__ perm, int64_t n_train,
+                                                             const unsigned long long* __restrict__ step, int64_t B,
+                                                             int64_t lo, int64_t hi, int64_t* __restrict__ users,
+                                                             int64_t* __restrict__ slots, int64_t* __restrict__ count,
+                                                             int64_t* __restrict__ total) {
+  __shared__ int warp_tot[BS_THREADS / 32];
+  const int64_t start = int64_t(*step) * B;
+  const int64_t rem = n_train - start;
+  const int64_t n = rem <= 0 ? 0 : (rem < B ? rem : B);
+  const int j0 = threadIdx.x * BS_PER;
+  int64_t u[BS_PER];
+  int c = 0;
+#pragma unroll
+  for (int q = 0; q < BS_PER; ++q) {
+    u[q] = j0 + q < n ? perm[start + j0 + q] : -1;
+    if (u[q] >= lo && u[q] < hi) ++c;
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int inc = c;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int v = __shfl_up_sync(0xffffffffu, inc, o);
+    if (lane >= o) inc += v;
+  }
+  if (lane == 31) warp_tot[warp] = inc;
+  __syncthreads();
+  if (warp == 0) {
+    const int w = warp_tot[lane];
+    int wi = w;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int v = __shfl_up_sync(0xffffffffu, wi, o);
+      if (lane >= o) wi += v;
+    }
+    warp_tot[lane] = wi - w;
+  }
+  __syncthreads();
+  int p = warp_tot[warp] + inc - c;
+#pragma unroll
+  for (int q = 0; q < BS_PER; ++q) {
+    if (u[q] >= lo && u[q] < hi) {
+      users[p] = u[q] - lo;
+      slots[p] = j0 + q;
+      ++p;
+    }
+  }
+  if (threadIdx.x == BS_THREADS - 1) {
+    *count = p;
+    *total = n;
+  }
 }
 
 // ---- table build -------------------------------------------------------------------------------
@@ -237,7 +303,7 @@ extern "C" int cgx_sample_triples(const int64_t* users, int64_t batch, const int
                                   const int32_t* class_start, const float* class_prob, const int32_t* class_alias,
                                   const int32_t* n_classes, float mix_pop, int32_t max_tries, uint64_t seed,
                                   uint64_t offset, const uint64_t* offset_dev, int64_t* pos_out, int64_t* neg_out,
-                                  void* stream_) {
+                                  void* stream_, const int64_t* slots, const int64_t* count) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(users && samp_indptr && samp_idx && pos_out && neg_out && batch > 0 && num_items > 0, CGX_ERR_ARG,
               "sample_triples: bad argument");
@@ -247,21 +313,37 @@ extern "C" int cgx_sample_triples(const int64_t* users, int64_t batch, const int
   SamplerTables tb{items_by_deg, class_start, class_prob, class_alias, n_classes};
   k_sample<<<(unsigned)ceil_div(batch, SM_THREADS), SM_THREADS, 0, stream>>>(
       users, batch, samp_indptr, samp_idx, num_items, tb, mix_pop, max_tries, seed, offset,
-      reinterpret_cast<const unsigned long long*>(offset_dev), pos_out, neg_out);
+      reinterpret_cast<const unsigned long long*>(offset_dev), slots, count, pos_out, neg_out);
   CGX_LAUNCH_CHECK();
   return CGX_OK;
 }
 
 extern "C" int cgx_eval_candidates(const int64_t* users, int64_t n_users, const int64_t* train_indptr,
                                    const int32_t* train_idx, const int64_t* test_indptr, const int32_t* test_idx,
-                                   int32_t num_items, int32_t n_neg, uint64_t seed, int64_t* cand, void* stream_) {
+                                   int32_t num_items, int32_t n_neg, uint64_t seed, int64_t* cand, void* stream_,
+                                   int64_t row_base) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(users && train_indptr && train_idx && test_indptr && test_idx && cand && n_users > 0 && num_items > 0 &&
-                  n_neg >= 0,
+                  n_neg >= 0 && row_base >= 0,
               CGX_ERR_ARG, "eval_candidates: bad argument");
   const int64_t n = n_users * (1 + n_neg);
   k_eval_candidates<<<(unsigned)ceil_div(n, SM_THREADS), SM_THREADS, 0, stream>>>(
-      users, n_users, train_indptr, train_idx, test_indptr, test_idx, num_items, 1 + n_neg, seed, cand);
+      users, n_users, train_indptr, train_idx, test_indptr, test_idx, num_items, 1 + n_neg, seed, row_base, cand);
+  CGX_LAUNCH_CHECK();
+  return CGX_OK;
+}
+
+extern "C" int cgx_batch_select(const int64_t* perm, int64_t n_train, const uint64_t* step, int64_t batch, int64_t lo,
+                                int64_t hi, int64_t* users_out, int64_t* slots_out, int64_t* count_out,
+                                int64_t* total_out, void* stream_) {
+  CGX_REQUIRE(perm && step && users_out && slots_out && count_out && total_out, CGX_ERR_ARG,
+              "batch_select: NULL pointer");
+  CGX_REQUIRE(n_train > 0 && batch > 0 && batch <= BS_MAX && lo >= 0 && hi >= lo, CGX_ERR_ARG,
+              "batch_select: bad argument (n_train %lld, batch %lld <= %lld, range [%lld, %lld))", (long long)n_train,
+              (long long)batch, (long long)BS_MAX, (long long)lo, (long long)hi);
+  k_batch_select<<<1, BS_THREADS, 0, static_cast<cudaStream_t>(stream_)>>>(
+      perm, n_train, reinterpret_cast<const unsigned long long*>(step), batch, lo, hi, users_out, slots_out, count_out,
+      total_out);
   CGX_LAUNCH_CHECK();
   return CGX_OK;
 }

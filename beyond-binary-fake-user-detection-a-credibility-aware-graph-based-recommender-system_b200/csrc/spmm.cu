@@ -738,10 +738,10 @@ __global__ void k_batch_frontier(const int64_t* __restrict__ indptr, const int32
                                  const int64_t* __restrict__ users, const int64_t* __restrict__ pos,
                                  const int64_t* __restrict__ neg, int64_t B, int32_t U, int32_t I,
                                  uint8_t* __restrict__ flags, uint8_t* __restrict__ flags_u,
-                                 int32_t* __restrict__ owner_u) {
+                                 int32_t* __restrict__ owner_u, const int64_t* __restrict__ count) {
   const int64_t t = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) / 32;
   const int lane = threadIdx.x & 31;
-  if (t >= B) return;
+  if (t >= B || (count != nullptr && t >= *count)) return;   // absent triples flag nothing
   const int64_t u = clamp_row(users[t], U);
   if (lane == 0) {
     flags[clamp_row(pos[t], I)] = 1;
@@ -755,7 +755,7 @@ __global__ void k_batch_frontier(const int64_t* __restrict__ indptr, const int32
 
 extern "C" int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64_t* pos,
                                   const int64_t* neg, int64_t B, uint8_t* flags_i, uint8_t* flags_u,
-                                  int32_t* owner_u, void* stream_) {
+                                  int32_t* owner_u, void* stream_, const int64_t* count) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   CGX_REQUIRE(by_user && by_user->indptr && (by_user->nnz == 0 || by_user->idx) && users && pos && neg && flags_i,
               CGX_ERR_ARG, "batch_frontier: NULL pointer");
@@ -764,7 +764,8 @@ extern "C" int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, 
   CGX_CUDA(cudaMemsetAsync(flags_i, 0, size_t(by_user->n_cols), stream));
   if (flags_u != nullptr) CGX_CUDA(cudaMemsetAsync(flags_u, 0, size_t(by_user->n_rows), stream));
   k_batch_frontier<<<(unsigned)ceil_div(B * 32, 256), 256, 0, stream>>>(
-      by_user->indptr, by_user->idx, users, pos, neg, B, by_user->n_rows, by_user->n_cols, flags_i, flags_u, owner_u);
+      by_user->indptr, by_user->idx, users, pos, neg, B, by_user->n_rows, by_user->n_cols, flags_i, flags_u, owner_u,
+      count);
   CGX_LAUNCH_CHECK();
   return CGX_OK;
 }

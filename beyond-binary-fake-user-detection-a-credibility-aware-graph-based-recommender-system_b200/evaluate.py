@@ -270,15 +270,18 @@ def sampled_candidates(train_csr, test_csr, num_items: int, n_neg: int, seed: in
     return users, cands
 
 
-def sampled_candidates_device(train_csr_dev, test_csr_dev, users, num_items: int, n_neg: int, seed: int):
-    """Candidate lists of the sampled protocol drawn by one kernel (cgx_eval_candidates)."""
+def sampled_candidates_device(train_csr_dev, test_csr_dev, users, num_items: int, n_neg: int, seed: int,
+                              row_base: int = 0):
+    """Candidate lists of the sampled protocol drawn by one kernel (cgx_eval_candidates).  row_base: the rows of
+    this call are rows row_base.. of a whole list (a shard gets the lists the whole call gives the same rows)."""
     dev = train_csr_dev[0].device
     users = torch.as_tensor(users, device=dev).to(torch.int64).contiguous()
     cand = torch.empty(users.numel(), 1 + n_neg, dtype=torch.int64, device=dev)
     with torch.cuda.device(dev):
         check(lib().cgx_eval_candidates(ptr(users), users.numel(), ptr(train_csr_dev[0]), ptr(train_csr_dev[1]),
                                         ptr(test_csr_dev[0]), ptr(test_csr_dev[1]), num_items, n_neg,
-                                        (int(seed) + 999) & 0xFFFFFFFFFFFFFFFF, ptr(cand), stream_ptr(dev)))
+                                        (int(seed) + 999) & 0xFFFFFFFFFFFFFFFF, ptr(cand), stream_ptr(dev),
+                                        int(row_base)))
     return cand
 
 

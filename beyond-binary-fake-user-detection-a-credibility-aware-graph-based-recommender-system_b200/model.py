@@ -88,8 +88,9 @@ def spmm_sparse_rows(csr, x, flags=None, use_bwd_values=False):
     return y
 
 
-def bpr_plan(graph: CredGraph, users, pos, neg, plan=None):
-    """Sorted (row, entry) keys of a triple batch: the scatter plan of the fused loss (indices only)."""
+def bpr_plan(graph: CredGraph, users, pos, neg, plan=None, count=None):
+    """Sorted (row, entry) keys of a triple batch: the scatter plan of the fused loss (indices only).
+    count: optional int64[1] device tensor -- triples at or past it are absent (padding; see bpr_fused)."""
     dev = graph.device
     users, pos, neg = _i64c(users, dev), _i64c(pos, dev), _i64c(neg, dev)
     B = users.numel()
@@ -98,35 +99,39 @@ def bpr_plan(graph: CredGraph, users, pos, neg, plan=None):
     ws = workspace(lib().cgx_bpr_plan_workspace_bytes(B), dev)
     with torch.cuda.device(dev):
         check(lib().cgx_bpr_plan(ptr(users), ptr(pos), ptr(neg), B, graph.num_users, graph.num_items, ptr(plan),
-                                 ptr(ws), ws.numel(), stream_ptr(dev)))
+                                 ptr(ws), ws.numel(), stream_ptr(dev), ptr(count)))
     return plan
 
 
-def batch_frontier(graph: CredGraph, users, pos, neg, flags=None, flags_u=None, owner_u=None):
+def batch_frontier(graph: CredGraph, users, pos, neg, flags=None, flags_u=None, owner_u=None, count=None):
     """uint8[I]: 1 on the items of pos, neg and the train rows of the batch users (cgx_batch_frontier), the only
     rows where the first item-side adjoint of the batch's loss can be non-zero.  flags_u (uint8[U], optional) is
-    set to 1 on the batch users, and owner_u (int32[U], optional) to one batch position of each batch user."""
+    set to 1 on the batch users, and owner_u (int32[U], optional) to one batch position of each batch user.
+    count (int64[1] device tensor, optional): triples at or past it are absent."""
     dev = graph.device
     users, pos, neg = _i64c(users, dev), _i64c(pos, dev), _i64c(neg, dev)
     if flags is None:
         flags = torch.empty(graph.num_items, dtype=torch.uint8, device=dev)
     with torch.cuda.device(dev):
         check(lib().cgx_batch_frontier(graph.by_user.ref(), ptr(users), ptr(pos), ptr(neg), users.numel(), ptr(flags),
-                                       ptr(flags_u), ptr(owner_u), stream_ptr(dev)))
+                                       ptr(flags_u), ptr(owner_u), stream_ptr(dev), ptr(count)))
     return flags
 
 
 def bpr_fused(graph: CredGraph, f_u, f_i, e0_u, e0_i, users, pos, neg, reg_weight, fair_weight=0.0, pop=None,
-              g_u=None, g_i=None, plan=None, bufs=None, batch_total=0):
+              g_u=None, g_i=None, plan=None, bufs=None, batch_total=0, count=None, total=None):
     """Loss value + gradients w.r.t. the propagated tables + compact ego (L2) gradient.
     g_u / g_i, when given, must be zero-filled [U,d] / [I,d] buffers; `plan` = bpr_plan(...) of the
-    same batch (built here when absent); `bufs` = reusable (loss, ego_rows, ego_coef, ws)."""
+    same batch (built here when absent); `bufs` = reusable (loss, ego_rows, ego_coef, ws).
+    count (int64[1] device tensor, optional; the plan must be built with the same): triples at or past it are absent
+    -- no loss term, no gradient row, ego_rows -1, no range check.  total (int64[1] device tensor, optional): the
+    mean's denominator, read on the device instead of batch_total."""
     dev = f_u.device
     f_u, f_i, e0_u, e0_i = _f32c(f_u), _f32c(f_i), _f32c(e0_u), _f32c(e0_i)
     users, pos, neg = _i64c(users, dev), _i64c(pos, dev), _i64c(neg, dev)
     B, d = users.numel(), f_u.shape[1]
     if plan is None:
-        plan = bpr_plan(graph, users, pos, neg)
+        plan = bpr_plan(graph, users, pos, neg, count=count)
     if g_u is None:
         g_u = torch.zeros_like(f_u)
     if g_i is None:
@@ -140,7 +145,7 @@ def bpr_fused(graph: CredGraph, f_u, f_i, e0_u, e0_i, users, pos, neg, reg_weigh
                                     graph.num_items,
                                     d, ptr(f_u), ptr(f_i), ptr(e0_u), ptr(e0_i), ptr(pop_t), float(reg_weight),
                                     float(fair_weight), ptr(loss), ptr(g_u), ptr(g_i), ptr(ego_rows),
-                                    ptr(ego_coef), ptr(ws), ws.numel(), stream_ptr(dev)))
+                                    ptr(ego_coef), ptr(ws), ws.numel(), stream_ptr(dev), ptr(count), ptr(total)))
     return loss, g_u, g_i, ego_rows, ego_coef
 
 

@@ -79,14 +79,18 @@ class TripleSampler:
                                               ptr(self.n_classes), ptr(ws), ws.numel(), stream_ptr(dev)))
             self.tables = (self.items_by_deg, self.class_start, self.class_prob, self.class_alias, self.n_classes)
 
-    def sample(self, users: torch.Tensor, offset: int | None = None, offset_dev: torch.Tensor | None = None):
+    def sample(self, users: torch.Tensor, offset: int | None = None, offset_dev: torch.Tensor | None = None,
+               slots: torch.Tensor | None = None, count: torch.Tensor | None = None, out=None):
         """users: int64 CUDA tensor of batch users, each with >= 1 train item.  Returns (pos, neg).
-        offset_dev: int64[1] device counter added to the offset (CUDA-graph replay)."""
+        offset_dev: int64[1] device counter added to the offset (CUDA-graph replay).
+        slots: int64[B] device tensor -- entry k draws the triple of global batch slot slots[k] (a sharded rank's part
+        of a batch draws what the whole-batch call draws for those users); count: int64[1] device tensor -- entries at
+        or past it are absent and their outputs are left untouched; out: (pos, neg) buffers to write."""
         g, dev = self.graph, self.graph.device
         users = torch.as_tensor(users, device=dev).to(torch.int64).contiguous()
         B = users.numel()
-        pos = torch.empty(B, dtype=torch.int64, device=dev)
-        neg = torch.empty(B, dtype=torch.int64, device=dev)
+        pos, neg = out if out is not None else (torch.empty(B, dtype=torch.int64, device=dev),
+                                                torch.empty(B, dtype=torch.int64, device=dev))
         if offset is None:
             offset = self.calls
         self.calls += 1
@@ -96,5 +100,5 @@ class TripleSampler:
                                            ptr(t[0]), ptr(t[1]), ptr(t[2]), ptr(t[3]), ptr(t[4]),
                                            -1.0 if self.mix_pop is None else float(self.mix_pop), self.max_tries,
                                            int(self.seed) & 0xFFFFFFFFFFFFFFFF, int(offset), ptr(offset_dev),
-                                           ptr(pos), ptr(neg), stream_ptr(dev)))
+                                           ptr(pos), ptr(neg), stream_ptr(dev), ptr(slots), ptr(count)))
         return pos, neg

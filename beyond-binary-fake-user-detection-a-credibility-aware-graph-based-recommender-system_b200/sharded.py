@@ -531,20 +531,25 @@ def item_gradient_block_floats(B: int, d: int) -> int:
     return 2 * B * (d + 2) + 4
 
 
-def pack_item_gradient(ego_rows, ego_coef, gi_local, loss, B: int, Bm: int, U: int, d: int) -> torch.Tensor:
+def pack_item_gradient(ego_rows, ego_coef, gi_local, loss, B: int, Bm: int, U: int, d: int, count=None) -> torch.Tensor:
     """One rank's block.  ego_rows int32[3B] / ego_coef float[3B] come from cgx_bpr_fwd_bwd: entry k names the row of
     the k-th position of the scatter plan when that position starts a run (users < U, items offset by U), else -1; the
-    plan is sorted by row with the B user entries first, so the item runs live in positions [B, 3B).  gi_local [I, d]
-    holds the gradient rows the loss wrote.  Blocks have the size of Bm = max_batch on every rank (ranks may hold
-    different batch sizes): unused slots carry row id -1 and zeros."""
+    plan is sorted by row with the B user entries first, so the item runs live in positions [B, 3B) -- or, when the
+    batch has a device count c (int64[1] tensor `count`: triples at or past it are padding), in [c, 3c), the absent
+    entries sorting last.  gi_local [I, d] holds the gradient rows the loss wrote.  Blocks have the size of
+    Bm = max_batch on every rank (ranks may hold different batch sizes): unused slots carry row id -1 and zeros."""
     dev = gi_local.device
-    er = ego_rows[B:]
+    if count is None:
+        er, ec = ego_rows[B:], ego_coef[B:]
+    else:                                   # positions c .. c + 2B - 1 (clamped; those past 3c hold -1)
+        at = (torch.arange(2 * B, device=dev) + count).clamp_(max=3 * B - 1)
+        er, ec = ego_rows[at], ego_coef[at]
     valid = er >= U
     rows = torch.where(valid, er - U, torch.zeros_like(er)).to(torch.int64)
     block = torch.zeros(item_gradient_block_floats(Bm, d), dtype=torch.float32, device=dev)
     block[: 2 * B * d].view(2 * B, d).copy_(torch.where(valid[:, None], gi_local[rows], 0.0))
     o_coef, o_rows, o_loss = 2 * Bm * d, 2 * Bm * (d + 1), 2 * Bm * (d + 2)
-    block[o_coef: o_coef + 2 * B] = torch.where(valid, ego_coef[B:], 0.0)   # (non-head slots are uninitialised)
+    block[o_coef: o_coef + 2 * B] = torch.where(valid, ec, 0.0)   # (non-head slots are uninitialised)
     rid_local = torch.full((2 * Bm,), -1, dtype=torch.int32, device=dev)
     rid_local[: 2 * B] = torch.where(valid, rows, torch.full_like(rows, -1)).to(torch.int32)
     block[o_rows: o_rows + 2 * Bm] = rid_local.view(torch.float32)
@@ -586,7 +591,9 @@ class ShardedTrainStep:
 
     def __init__(self, graph: CredGraph, user_emb: torch.Tensor, item_emb: torch.Tensor, num_layers, order,
                  lr=1e-3, reg_weight=1e-4, mix_pop=0.7, gamma=0.75, max_tries=50, seed=42, group=None,
-                 exchange: str = "p2p", max_batch: int = 4096):
+                 exchange: str = "p2p", max_batch: int = 4096, fair_weight: float = 0.0, pop=None):
+        """fair_weight / pop: the fairness term of lightgcn_cu.py (pop: float[I], deg_i / max(deg_i) of the GLOBAL
+        item degrees); its gradient rides in the loss gradient the step exchanges."""
         self.graph, self.group = graph, group
         self.eu = torch.nn.Parameter(user_emb.contiguous())
         self.ei = torch.nn.Parameter(item_emb.contiguous())
@@ -617,7 +624,8 @@ class ShardedTrainStep:
         graph.set_emb_dim(d)          # hot-row hints of the SpMMs for this width
         self.prop = ShardedPropagation(CudaBackend(graph), num_layers, order, group, self.ex)
         self.sampler = TripleSampler(graph, mix_pop, gamma, max_tries, seed)
-        self.reg = float(reg_weight)
+        self.reg, self.fair = float(reg_weight), float(fair_weight)
+        self.pop = None if pop is None else torch.as_tensor(pop, dtype=torch.float32, device=dev).contiguous()
         self.eu.grad, self.ei.grad = torch.zeros_like(self.eu), torch.zeros_like(self.ei)
         self.opt = FusedAdam(self.eu, self.ei, lr=lr)
         # dense gradient tables kept ZERO outside the rows of the current batch (flagged for the adjoint by
@@ -632,6 +640,8 @@ class ShardedTrainStep:
         self._ego_u = None          # dense form only: user L2 gradient buffer
         self._bufs = {}
         self._graph = None
+        self._sel = None            # device-side batch selection of an epoch (plan_epochs)
+        self._g_selected = False    # the captured graph is the epoch step (capture(selected=True))
 
     # Tables of 256 MB and more whose item rows are short (C5 shards: 10 non-zeros per row -- the pushed form makes
     # the product NVLink-bound there).  Measured on 8 B200s, C5, ms per step: pushed 134.5, pull kernel 97.6, NCCL 85.8,
@@ -659,31 +669,39 @@ class ShardedTrainStep:
         return item_gradient_block_floats(B, d)
 
     @torch.no_grad()
-    def __call__(self, users_local: torch.Tensor, batch_total: int | None = None, triples=None):
+    def __call__(self, users_local: torch.Tensor, batch_total: int | None = None, triples=None, count=None,
+                 total=None, slots=None):
         """batch_total: global batch size (default: every rank holds a batch of this size).
-        triples: optional injected (pos, neg) for users_local instead of sampling (parity tests)."""
+        triples: optional injected (pos, neg) for users_local instead of sampling (parity tests).
+        count / total / slots: int64 device tensors of a padded batch (cgx_batch_select): entries at or past count[0]
+        are absent, total[0] is the global batch size, slots the entries' positions in the global batch (their
+        sampler streams)."""
         g, dev = self.graph, self.eu.device
         B = users_local.numel()
         world = _world(self.group)
-        B_total = int(batch_total) if batch_total is not None else B * world
+        B_total = 0 if total is not None else int(batch_total) if batch_total is not None else B * world
         U, (I, d) = g.num_users, self.ei.shape
         if B not in self._bufs:
-            self._bufs[B] = (torch.empty(3 * B, dtype=torch.int64, device=dev), bpr_buffers(g, B, dev))
-        plan, bufs = self._bufs[B]
+            self._bufs[B] = (torch.empty(3 * B, dtype=torch.int64, device=dev), bpr_buffers(g, B, dev),
+                             (torch.zeros(B, dtype=torch.int64, device=dev), torch.zeros(B, dtype=torch.int64,
+                                                                                           device=dev)))
+        plan, bufs, pn = self._bufs[B]
         if hasattr(self.ex, "begin_step"):
             self.ex.begin_step()
         with torch.cuda.device(dev):
             check(lib().cgx_tick(ptr(self.tick), stream_ptr(dev)))
         if triples is None:
-            pos, neg = self.sampler.sample(users_local, offset=0, offset_dev=self.tick)
+            pos, neg = self.sampler.sample(users_local, offset=0, offset_dev=self.tick, slots=slots, count=count,
+                                           out=pn)
         else:
             pos, neg = (torch.as_tensor(t, device=dev).to(torch.int64) for t in triples)
-        bpr_plan(g, users_local, pos, neg, plan)
+        bpr_plan(g, users_local, pos, neg, plan, count=count)
         f_u, f_i = self.prop.forward(self.eu.data, self.ei.data)
         if not self.compact:
-            return self._finish_dense(users_local, pos, neg, plan, bufs, f_u, f_i, B_total)
+            return self._finish_dense(users_local, pos, neg, plan, bufs, f_u, f_i, B_total, count, total)
         loss, _, _, ego_rows, ego_coef = bpr_fused(g, f_u, f_i, self.eu.data, self.ei.data, users_local, pos, neg,
-                                                   self.reg, 0.0, None, self.g_u, self.gi_local, plan, bufs, B_total)
+                                                   self.reg, self.fair, self.pop, self.g_u, self.gi_local, plan, bufs,
+                                                   B_total, count=count, total=total)
         with torch.cuda.device(dev):
             check(lib().cgx_bpr_mark_rows(ptr(ego_rows), ego_rows.numel(), U, ptr(self.nz_u), ptr(self.nz_i_local),
                                           stream_ptr(dev)))
@@ -691,7 +709,7 @@ class ShardedTrainStep:
         Bm = self.max_batch
         if B > Bm:
             raise _lib.CgxError(f"ShardedTrainStep: batch of {B} users exceeds max_batch={Bm}")
-        block = pack_item_gradient(ego_rows, ego_coef, self.gi_local, loss, B, Bm, U, d)
+        block = pack_item_gradient(ego_rows, ego_coef, self.gi_local, loss, B, Bm, U, d, count)
         blocks = self.ex.allgather(block)                                   # [world, n], rank order
         vals, coef, rows_all, ok, total_loss = unpack_item_gradient(blocks, Bm, d, I)
         for r in range(world):                                              # rank order: same bits on every rank
@@ -723,7 +741,7 @@ class ShardedTrainStep:
             self.ei.grad.index_fill_(0, flat_c, 0.0)
         return total_loss
 
-    def _finish_dense(self, users_local, pos, neg, plan, bufs, f_u, f_i, B_total):
+    def _finish_dense(self, users_local, pos, neg, plan, bufs, f_u, f_i, B_total, count=None, total=None):
         """Loss, adjoint and Adam with ONE dense exchange of [item gradient seed ; item L2 gradient ; loss] -- the
         small-table form of the step (2 I d + 4 floats through the same exchange as the item tables)."""
         g, dev = self.graph, self.eu.device
@@ -737,7 +755,8 @@ class ShardedTrainStep:
         self._ego_u.zero_()
         bufs = (red[2 * n: 2 * n + 1],) + tuple(bufs[1:])
         _, _, _, ego_rows, ego_coef = bpr_fused(g, f_u, f_i, self.eu.data, self.ei.data, users_local, pos, neg,
-                                                self.reg, 0.0, None, self.g_u, gi2[0], plan, bufs, B_total)
+                                                self.reg, self.fair, self.pop, self.g_u, gi2[0], plan, bufs, B_total,
+                                                count=count, total=total)
         apply_ego(g, ego_rows, ego_coef, self.eu.data, self.ei.data, self._ego_u, gi2[1])
         # cloned: the exchange's output region is recycled two exchanges later, the seed is needed by every layer
         red = self.ex.reduce(red).clone()
@@ -748,33 +767,87 @@ class ShardedTrainStep:
         self.opt.step()
         return red[2 * n: 2 * n + 1]
 
-    def capture(self, batch: int):
+    def capture(self, batch: int, selected: bool = False):
         """Record the whole sharded step as one CUDA graph.  Only with the peer-memory exchange: every launch
         of the step is then a kernel of this library or a torch elementwise op, and the exchange epochs are
-        device-side counters.  (Capturing the NCCL variant hung on this stack: torch 2.11 / NCCL 2.28.9.)"""
+        device-side counters.  (Capturing the NCCL variant hung on this stack: torch 2.11 / NCCL 2.28.9.)
+        selected=True records the epoch step of plan_epochs() instead -- batch selection on the device, then the step
+        over the padded local batch of capacity max_batch -- which step_selected() replays: every batch of an epoch,
+        the tail batch included, runs the same graph with no host work."""
         if not isinstance(self.ex, P2PExchange):
             raise _lib.CgxError("ShardedTrainStep.capture needs exchange='p2p'")
+        if selected and self._sel is None:
+            raise _lib.CgxError("ShardedTrainStep.capture(selected=True) needs plan_epochs() first")
         dev = self.eu.device
         self._g_users = torch.zeros(batch, dtype=torch.int64, device=dev)
+        run = self._selected_step if selected else (lambda: self(self._g_users))
         state = (self.eu.data, self.ei.data, self.opt.m[0], self.opt.m[1], self.opt.v[0], self.opt.v[1],
-                 self.opt.step_dev, self.tick)
+                 self.opt.step_dev, self.tick) + ((self._sel["step"],) if selected else ())
         warm = torch.cuda.Stream(device=dev)
         warm.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(warm):
             keep = [t.clone() for t in state]
             for _ in range(2):                     # every rank runs the same two steps: exchanges stay matched
-                self(self._g_users)
+                run()
             for dst, src in zip(state, keep):
                 dst.copy_(src)
         torch.cuda.current_stream(dev).wait_stream(warm)
         torch.cuda.synchronize(dev)
         self._graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._graph):
-            self._g_loss = self(self._g_users)
+            self._g_loss = run()
+        self._g_selected = selected
         return self
 
+    # ---- epochs with device-side batch selection (train_on_arrays_sharded) ----------------------------------------
+    def plan_epochs(self, n_train: int, lo: int, hi: int):
+        """Buffers of the epoch step: the epoch's permutation of the n_train GLOBAL train users (begin_epoch), a device
+        batch counter, and the selection outputs of capacity max_batch.  This rank owns the users [lo, hi)."""
+        dev = self.eu.device
+        i64 = dict(dtype=torch.int64, device=dev)
+        self._sel = dict(perm=torch.zeros(int(n_train), **i64), n_train=int(n_train), lo=int(lo), hi=int(hi),
+                         step=torch.zeros(1, **i64), users=torch.zeros(self.max_batch, **i64),
+                         slots=torch.zeros(self.max_batch, **i64), count=torch.zeros(1, **i64),
+                         total=torch.zeros(1, **i64))
+        return self
+
+    def begin_epoch(self, perm):
+        """Upload the epoch's permutation of the global train users (identical on every rank) and restart at batch 0."""
+        sel = self._sel
+        p = torch.as_tensor(np.ascontiguousarray(perm, dtype=np.int64) if not isinstance(perm, torch.Tensor) else perm)
+        if p.numel() != sel["n_train"]:
+            raise _lib.CgxError(f"begin_epoch: permutation of {p.numel()} users, planned {sel['n_train']}")
+        sel["perm"].copy_(p.to(torch.int64))
+        sel["step"].zero_()
+
+    def _selected_step(self):
+        sel, dev = self._sel, self.eu.device
+        with torch.cuda.device(dev):
+            st = stream_ptr(dev)
+            check(lib().cgx_batch_select(ptr(sel["perm"]), sel["n_train"], ptr(sel["step"]), self.max_batch,
+                                         sel["lo"], sel["hi"], ptr(sel["users"]), ptr(sel["slots"]), ptr(sel["count"]),
+                                         ptr(sel["total"]), st))
+            check(lib().cgx_tick(ptr(sel["step"]), st))
+        return self(sel["users"], count=sel["count"], total=sel["total"], slots=sel["slots"])
+
+    def step_selected(self):
+        """The next batch of the epoch (begin_epoch): the captured graph when capture(..., selected=True) ran, else
+        the same launches eagerly.  Returns the global loss of the batch (float[1] device tensor)."""
+        if self._graph is not None and self._g_selected:
+            self._graph.replay()
+            return self._g_loss
+        return self._selected_step()
+
+    def last_batch(self):
+        """(global users, global slots, pos, neg) of this rank's part of the last selected batch (host NumPy)."""
+        sel = self._sel
+        c = int(sel["count"].item())
+        pos, neg = self._bufs[self.max_batch][2]
+        return ((sel["users"][:c] + sel["lo"]).cpu().numpy(), sel["slots"][:c].cpu().numpy(),
+                pos[:c].cpu().numpy(), neg[:c].cpu().numpy())
+
     def step(self, users):
-        if self._graph is not None and users.numel() == self._g_users.numel():
+        if self._graph is not None and not self._g_selected and users.numel() == self._g_users.numel():
             self._g_users.copy_(users, non_blocking=True)
             self._graph.replay()
             return self._g_loss
@@ -844,16 +917,249 @@ def evaluate_full_ranking_sharded(f_u_local, f_i, graph: CredGraph, test_edges_l
         ids = torch.zeros(0, K, dtype=torch.int32, device=dev)
     sums, bitmaps = ev.metrics_sums_device(ids, users_dev, te, num_items, ks, pop_dev, total_train, flags_dev,
                                            with_coverage=extra)
+    sums, cover = _reduce_metric_sums(sums, bitmaps, num_items, group)
+    return ev.metrics_result(Ks, ks, sums, cover, n, num_items, "full", groups)
+
+
+def _reduce_metric_sums(sums, bitmaps, num_items, group):
+    """Per-rank metric sums -> global sums (all-reduce) and, with bitmaps, the global coverage counts (host)."""
+    from . import evaluate as ev
+    world = _world(group)
     if world > 1:
         dist.all_reduce(sums, group=group)
-        if extra:   # NCCL has no bitwise-OR reduction: gather the (small) bitmaps and OR them here
+        if bitmaps is not None:   # NCCL has no bitwise-OR reduction: gather the (small) bitmaps and OR them here
             parts = [torch.empty_like(bitmaps) for _ in range(world)]
             dist.all_gather(parts, bitmaps, group=group)
             for p in parts[1:]:
                 parts[0] |= p
             bitmaps = parts[0]
-    cover = ev.coverage_counts_device(bitmaps, num_items).cpu().numpy() if extra else None
-    return ev.metrics_result(Ks, ks, sums.cpu().numpy(), cover, n, num_items, "full", groups)
+    cover = ev.coverage_counts_device(bitmaps, num_items).cpu().numpy() if bitmaps is not None else None
+    return sums.cpu().numpy(), cover
+
+
+@torch.no_grad()
+def evaluate_sampled_sharded(f_u_local, f_i, graph: CredGraph, lo: int, hi: int, train_csr, test_csr, num_items,
+                             Ks=(10, 20), n_neg=99, seed=42, on_device=False, item_pop=None, total_train=0, cred=None,
+                             group_pct=0.20, group=None):
+    """The sampled protocol (1 test positive + n_neg negatives per test user, lightgcn_cu.py:487-546) over user
+    shards: every rank scores and ranks the candidate lists of ITS test users against the replicated item table,
+    and only metric sums cross ranks.  train_csr / test_csr: host CSRs (indptr, indices) of the WHOLE graph;
+    `graph` is the rank's local CredGraph (users [lo, hi)); cred: the GLOBAL credibility vector (None: no
+    popularity / credibility metrics).  Candidates: on_device=False draws the reference's PCG64 list over all test
+    users -- identical on every rank -- and keeps the rank's rows; on_device=True draws the rank's rows with
+    cgx_eval_candidates keyed by their row in the whole list.  Either way each user ranks the candidates the
+    single-GPU evaluate_sampled gives it, and the credibility groups are percentiles of the global order."""
+    from . import evaluate as ev
+    from .graph import user_csr_device
+    dev = f_u_local.device
+    te_ip = np.asarray(test_csr[0])
+    users_all = np.flatnonzero(np.diff(te_ip) > 0).astype(np.int64)
+    if users_all.size == 0:
+        raise RuntimeError("No users with test interactions.")
+    first, last = np.searchsorted(users_all, lo), np.searchsorted(users_all, hi)
+    users = users_all[first:last]
+    if on_device:
+        te_loc = user_csr_device(np.stack([np.repeat(np.arange(hi - lo), np.diff(te_ip[lo:hi + 1])),
+                                           np.asarray(test_csr[1])[te_ip[lo]:te_ip[hi]]]), hi - lo, num_items, dev)
+        cands_dev = (ev.sampled_candidates_device((graph.samp_indptr, graph.samp_idx), te_loc, users - lo, num_items,
+                                                  n_neg, seed, row_base=int(first)) if users.size else None)
+    else:
+        _, cands = ev.sampled_candidates(train_csr, test_csr, num_items, n_neg, seed)
+        cands_dev = torch.from_numpy(np.ascontiguousarray(cands[first:last])).to(dev) if users.size else None
+    ks = sorted(set(int(k) for k in Ks))
+    extra = item_pop is not None and cred is not None
+    pop_dev = flags_dev = groups = None
+    if extra:
+        hi_g, lo_g = ev.make_cred_groups(users_all, cred, group_pct)
+        in_hi, in_lo = np.isin(users, hi_g), np.isin(users, lo_g)
+        flags_dev = torch.from_numpy(in_hi.astype(np.uint8) + 2 * in_lo.astype(np.uint8)).to(dev)
+        pop_dev = torch.as_tensor(np.asarray(item_pop, dtype=np.int64)).to(dev)
+        groups = (len(hi_g), len(lo_g), np.asarray(cred, np.float64)[users_all].mean())
+    users_dev = torch.from_numpy(users - lo).to(dev)
+    if users.size:
+        scores = ev.score_candidates_device(f_u_local, f_i, users_dev, cands_dev)
+        ranked = ev.rank_candidates_device(scores, cands_dev)
+        gt = cands_dev[:, 0]
+    else:
+        ranked = torch.zeros(0, 1 + n_neg, dtype=torch.int64, device=dev)
+        gt = None
+    sums, bitmaps = ev.metrics_sums_device(ranked, users_dev, None, num_items, ks, pop_dev, total_train, flags_dev,
+                                           gt_single_dev=gt, with_coverage=extra)
+    sums, cover = _reduce_metric_sums(sums, bitmaps, num_items, group)
+    return ev.metrics_result(Ks, ks, sums, cover, int(users_all.size), num_items, "sampled(1pos+neg)", groups,
+                             extra_keys={"negatives": n_neg})
+
+
+# ------------------------------------------------------------------------------------------
+# the reference's training loop over user shards (train_lightgcn() under torchrun)
+# ------------------------------------------------------------------------------------------
+def initial_tables(variant: str, num_users: int, num_items: int, emb_dim: int):
+    """The initial (user, item) tables of the single-GPU model, drawn from torch's CPU generator in the same order as
+    the model's constructor draws them (nn.Embedding's normal_ fill, then xavier_uniform_): RawLightGCN's one
+    (U + I) x d table, or the two tables of CredLightGCN / LightGCN."""
+    if variant == "raw":
+        w = torch.empty(num_users + num_items, emb_dim)
+        torch.nn.init.normal_(w)
+        torch.nn.init.xavier_uniform_(w)
+        return w[:num_users], w[num_users:]
+    eu, ei = torch.empty(num_users, emb_dim), torch.empty(num_items, emb_dim)
+    torch.nn.init.normal_(eu)
+    torch.nn.init.normal_(ei)
+    torch.nn.init.xavier_uniform_(eu)
+    torch.nn.init.xavier_uniform_(ei)
+    return eu, ei
+
+
+def _gather_users(eu_local: torch.Tensor, bounds, group) -> torch.Tensor:
+    """The user shards of all ranks in rank order (every rank takes part; the result is used on rank 0)."""
+    world = _world(group)
+    if world == 1:
+        return eu_local.clone()
+    rows = int(max(bounds[r + 1] - bounds[r] for r in range(world)))
+    pad = torch.zeros(rows, eu_local.shape[1], dtype=eu_local.dtype, device=eu_local.device)
+    pad[: eu_local.shape[0]] = eu_local
+    parts = [torch.empty_like(pad) for _ in range(world)]
+    dist.all_gather(parts, pad, group=group)
+    return torch.cat([parts[r][: int(bounds[r + 1] - bounds[r])] for r in range(world)])
+
+
+def train_on_arrays_sharded(train_edges, val_edges, test_edges, num_users, num_items, cred_np, out_dir=None, cfg=None,
+                            group=None, on_step=None):
+    """train.train_on_arrays over the users of `group`'s ranks (one process per GPU, the current CUDA device): the
+    same model, batches and triples as the single-GPU loop -- losses, metrics and tables agree up to the order of
+    floating-point sums -- for every cfg.variant.
+
+    Every rank computes the same train users and the same default_rng(cfg.seed) shuffle per epoch and runs
+    ceil(n_train / batch_size) steps; the ShardedTrainStep selects each global batch's entries of the rank's users
+    on the device (cgx_batch_select), samples the triple of each entry from the stream of its slot in the global
+    batch, and divides by the global batch size, so the tail batch needs nothing special.  Evaluation follows
+    cfg.eval_mode (full-rank: evaluate_full_ranking_sharded at cfg.score_precision; sampled:
+    evaluate_sampled_sharded), with only metric sums crossing ranks.  Prints come from rank 0.  The best-validation
+    checkpoint (same file name and keys as the single-GPU loop: the user shards in rank order and the item table)
+    is written by rank 0 and restored on every rank before the test evaluation.  on_step(step, epoch, s): optional
+    callback after every step (e.g. ShardedTrainStep.last_batch()).
+    Returns (state_dict on rank 0 / None on the other ranks, test results -- identical on every rank)."""
+    from pathlib import Path
+
+    from . import config
+    from . import evaluate as ev
+    from .train import _GRAPH_VARIANT, _POPMIX, _print_metrics, evaluate_csr
+    cfg = cfg or config.cfg
+    variant = cfg.variant
+    world = _world(group)
+    rank = dist.get_rank(group) if world > 1 else 0
+    dev = torch.device("cuda", torch.cuda.current_device())
+    say = print if rank == 0 else (lambda *a, **k: None)
+    say("Using device:", dev, f"(user-sharded over {world} ranks)")
+
+    train_edges = np.asarray(train_edges)
+    U, I = int(num_users), int(num_items)
+    deg_u = np.bincount(train_edges[0].astype(np.int64), minlength=U)
+    bounds = partition_users(deg_u, world)
+    lo, hi = int(bounds[rank]), int(bounds[rank + 1])
+    raw = variant == "raw"
+    cred = np.ones(U, dtype=np.float32) if raw else np.asarray(cred_np, dtype=np.float32)
+    gl = build_local_graph(shard_edges(train_edges, bounds, rank), hi - lo, I, cred[lo:hi],
+                           "cu" if raw else _GRAPH_VARIANT[variant], dev, group)
+    rich = variant == "v2"
+    item_pop, total_train = ev.compute_item_popularity(train_edges, I) if rich else (None, 0)
+    train_users = np.flatnonzero(deg_u > 0)
+    if len(train_users) == 0:
+        raise RuntimeError("No train users with interactions. Check your threshold/split.")
+
+    pop_fair = None
+    if variant == "cu" and cfg.lambda_fair:
+        deg_i = gl.deg_i_float()
+        pop_fair = (deg_i / max(float(deg_i.max()), 1.0)).astype(np.float32)      # lightgcn_cu.py:583
+    popmix = variant in _POPMIX
+    if popmix:
+        item_deg = gl.deg_i.cpu().numpy().astype(np.float64)
+        p10, p50, p90, p99 = np.percentile(item_deg, [10, 50, 90, 99])
+        say(f"[NEG-E] item_deg percentiles: p10={p10:.0f} p50={p50:.0f} p90={p90:.0f} p99={p99:.0f} "
+            f"max={item_deg.max():.0f}")
+        say(f"[NEG-E] mix_pop={cfg.neg_mix_pop} gamma={cfg.neg_pop_gamma}")
+    eu0, ei0 = initial_tables(variant, U, I, cfg.emb_dim)
+    step = ShardedTrainStep(gl, eu0[lo:hi].to(dev), ei0.to(dev), cfg.num_layers,
+                            "jacobi" if variant in ("cu", "raw") else "gs", lr=cfg.lr,
+                            reg_weight=cfg.lambda_reg if variant == "cu" else cfg.reg,
+                            mix_pop=cfg.neg_mix_pop if popmix else None, gamma=cfg.neg_pop_gamma,
+                            max_tries=cfg.neg_max_tries, seed=cfg.seed, group=group, exchange="auto",
+                            max_batch=cfg.batch_size, fair_weight=cfg.lambda_fair if variant == "cu" else 0.0,
+                            pop=pop_fair)
+    del eu0, ei0
+    n_train, B = len(train_users), int(cfg.batch_size)
+    steps = -(-n_train // B)
+    step.plan_epochs(n_train, lo, hi)
+
+    full = cfg.eval_mode == "full" and variant != "cu"
+    train_csr_host = None if full else evaluate_csr(train_edges, U, I, dev)    # the reference's candidate draw
+
+    def run_eval(edges):
+        f_u, f_i = step.prop.forward(step.eu.data, step.ei.data)
+        f_u, f_i = f_u.contiguous(), f_i.contiguous()
+        if full:
+            return evaluate_full_ranking_sharded(f_u, f_i, gl, shard_edges(np.asarray(edges), bounds, rank), I,
+                                                 cfg.Ks, item_pop, total_train, cred[lo:hi] if rich else None,
+                                                 cfg.cred_group_pct, group, cfg.score_precision)
+        return evaluate_sampled_sharded(f_u, f_i, gl, lo, hi, train_csr_host, evaluate_csr(edges, U, I, dev), I, cfg.Ks,
+                                        cfg.sampled_negatives, cfg.seed, cfg.sampled_eval_on_device, item_pop,
+                                        total_train, cred if rich else None, cfg.cred_group_pct, group)
+
+    def state_dict():
+        eu_all = _gather_users(step.eu.data, bounds, group)
+        if rank != 0:
+            return None
+        if raw:
+            return {"emb.weight": torch.cat([eu_all, step.ei.data.clone()])}
+        return {"user_emb.weight": eu_all, "item_emb.weight": step.ei.data.clone()}
+
+    best_val, best = -1.0, None
+    best_path = None
+    if out_dir is not None:
+        best_path = Path(out_dir) / "model" / ("best_model_cred.pt" if variant == "cu" else "best_model.pt")
+        if rank == 0:
+            best_path.parent.mkdir(parents=True, exist_ok=True)
+
+    rng = np.random.default_rng(cfg.seed)
+    captured = False
+    for epoch in range(1, cfg.epochs + 1):
+        rng.shuffle(train_users)
+        step.begin_epoch(train_users)
+        if not captured and isinstance(step.ex, P2PExchange):
+            step.capture(B, selected=True)       # every rank: the exchange kind is agreed on by all ranks
+            captured = True
+        losses = []
+        for s in range(steps):
+            losses.append(step.step_selected().clone())
+            if on_step is not None:
+                on_step(step, epoch, s)
+        avg_loss = float(torch.stack(losses).mean().item()) if losses else 0.0
+        say(f"Epoch {epoch:03d} | loss={avg_loss:.6f}" if variant == "cu" else f"Epoch {epoch:02d} | loss={avg_loss:.6f}")
+
+        if epoch % cfg.eval_every == 0:
+            val_res = run_eval(val_edges)
+            selK = max(cfg.Ks)
+            if rank == 0:
+                _print_metrics("VAL metrics:", val_res, cfg.Ks, rich)
+            if val_res[selK]["recall"] > best_val:
+                best_val = val_res[selK]["recall"]
+                best = (step.eu.data.clone(), step.ei.data.clone())
+                sd = state_dict()
+                if best_path is not None and rank == 0:
+                    torch.save(sd, best_path)
+                    print(f"  ✅ Saved best model to {best_path} (val Recall@{selK}={best_val:.4f})")
+    step.check()
+    if best is not None:
+        step.eu.data.copy_(best[0])
+        step.ei.data.copy_(best[1])
+    test_res = run_eval(test_edges)
+    if rank == 0:
+        _print_metrics("\nTEST metrics:", test_res, cfg.Ks, rich)
+    sd = state_dict()
+    if world > 1:
+        dist.barrier(group=group)
+    step.close()
+    return sd, test_res
 
 
 # ------------------------------------------------------------------------------------------

@@ -19,7 +19,10 @@ RAW's L2 weight is cfg.reg (1e-4, as in every script).  lightgcn-1.py is the sam
 """
 from __future__ import annotations
 
+import contextlib
 import csv
+import io
+import os
 import pickle
 from pathlib import Path
 
@@ -207,9 +210,19 @@ def evaluate_csr(edges, num_users, num_items, device):
     return indptr.cpu().numpy(), idx.cpu().numpy().astype(np.int64)
 
 
+def _sharded_world():
+    import torch.distributed as dist
+    return dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
+
+
 def train_lightgcn():
-    """Reference entry point: everything comes from the module-global cfg and cfg.out_dir."""
+    """Reference entry point: everything comes from the module-global cfg and cfg.out_dir.  Under an initialised
+    torch.distributed process group of more than one rank (torchrun, see main()) it trains user-sharded over the
+    ranks (sharded.train_on_arrays_sharded: the same batches, triples and results as one GPU), printing on rank 0."""
+    import torch.distributed as dist
     cfg = config.cfg
+    world = _sharded_world()
+    quiet = world > 1 and dist.get_rank() != 0
     out = Path(cfg.out_dir)
     train_edges = np.load(out / "npy" / "train_edges.npy")
     val_edges = np.load(out / "npy" / "val_edges.npy")
@@ -219,21 +232,49 @@ def train_lightgcn():
     with open(out / "model" / "item2idx.pkl", "rb") as f:
         item2idx = pickle.load(f)
     num_users, num_items = len(user2idx), len(item2idx)
-    print(f"Loaded edges. Users={num_users:,} Items={num_items:,} "
-          f"Train={train_edges.shape[1]:,} Val={val_edges.shape[1]:,} Test={test_edges.shape[1]:,}")
-    cred_np = None if cfg.variant == "raw" else load_credibility_vector(cfg.cred_csv_path, user2idx)
+    with contextlib.redirect_stdout(io.StringIO()) if quiet else contextlib.nullcontext():
+        print(f"Loaded edges. Users={num_users:,} Items={num_items:,} "
+              f"Train={train_edges.shape[1]:,} Val={val_edges.shape[1]:,} Test={test_edges.shape[1]:,}")
+        cred_np = None if cfg.variant == "raw" else load_credibility_vector(cfg.cred_csv_path, user2idx)
+    if world > 1:
+        from .sharded import train_on_arrays_sharded
+        _, test_res = train_on_arrays_sharded(train_edges, val_edges, test_edges, num_users, num_items, cred_np, out,
+                                              cfg)
+        return test_res
     _, test_res = train_on_arrays(train_edges, val_edges, test_edges, num_users, num_items, cred_np, out, cfg)
     return test_res
 
 
 def main():
     """The reference's main() (lightgcn_cu.py:690-703): build the graph files if they are missing, then train.
-    Unlike the reference, the raw JSONL is only required when the graph files do not exist yet."""
+    Unlike the reference, the raw JSONL is only required when the graph files do not exist yet.
+    Started by `torchrun --nproc-per-node N` (WORLD_SIZE > 1), every process takes the GPU of its LOCAL_RANK, joins
+    an NCCL process group and trains user-sharded (train_lightgcn); rank 0 builds missing graph files.  Without
+    WORLD_SIZE, or with WORLD_SIZE=1, nothing of this happens."""
+    import torch.distributed as dist
     from . import ingest
-    set_seed(config.cfg.seed)
-    if not (Path(config.cfg.out_dir) / "npy" / "train_edges.npy").exists():
-        print("Graph files not found. Building graph first...")
-        ingest.build_graph_from_jsonl()
-    else:
-        print("Graph files exist. Skipping construction.")
-    train_lightgcn()
+    own_group = False
+    if int(os.environ.get("WORLD_SIZE", "1")) > 1 and not dist.is_initialized():
+        dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
+        torch.cuda.set_device(dev)
+        dist.init_process_group("nccl", device_id=dev)
+        own_group = True
+    try:
+        rank0 = _sharded_world() == 1 or dist.get_rank() == 0
+        set_seed(config.cfg.seed)
+        if rank0:
+            if not (Path(config.cfg.out_dir) / "npy" / "train_edges.npy").exists():
+                print("Graph files not found. Building graph first...")
+                ingest.build_graph_from_jsonl()
+            else:
+                print("Graph files exist. Skipping construction.")
+        if _sharded_world() > 1:
+            dist.barrier()
+        train_lightgcn()
+    finally:
+        if own_group:
+            dist.destroy_process_group()
+
+
+if __name__ == "__main__":
+    main()

@@ -272,9 +272,11 @@ int cgx_propagate_bwd_frontier(const cgx_csr* by_user, const cgx_csr* by_item, i
  * range count as 0, as in cgx_bpr_plan.  flags_u uint8[num_users] (nullable) is zeroed and set for users[t]: the
  * user rows the loss reads.  owner_u int32[num_users] (nullable; not zeroed): owner_u[users[t]] = one t of each
  * batch user, for the user row list of cgx_propagate_fwd_layers.  Depends on the indices only: it can run on a side
- * stream beside the forward propagation, as cgx_bpr_plan does. */
+ * stream beside the forward propagation, as cgx_bpr_plan does.  count int64[1] (device, nullable): triples
+ * t >= *count are absent and flag nothing (their ids are not read). */
 int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64_t* pos, const int64_t* neg,
-                       int64_t batch, uint8_t* flags_i, uint8_t* flags_u, int32_t* owner_u, void* stream);
+                       int64_t batch, uint8_t* flags_i, uint8_t* flags_u, int32_t* owner_u, void* stream,
+                       const int64_t* count);
 
 /* ------------------------------------------------------------------------------------------
  * BPR + L2 (+ fairness) on a batch of (user, pos, neg) triples.  Replaces score / l2_reg / the loss
@@ -292,13 +294,19 @@ int cgx_batch_frontier(const cgx_csr* by_user, const int64_t* users, const int64
  *   loss_out float[1]      NaN if any index of the batch was out of range
  *   batch_total            the mean's denominator: `batch`, or -- when the batch is sharded over ranks -- the
  *                          global batch size (the rank losses then add up to the global loss)
+ *   count int64[1]         (device, nullable; pass the same to cgx_bpr_plan) triples t >= *count are ABSENT --
+ *                          the padding of a fixed-capacity batch: they draw no loss term, write no gradient row,
+ *                          are not range-checked (garbage ids are harmless) and their plan entries sort behind
+ *                          every real row; ego_rows is -1 at those positions.  Loss, rows, ego_rows and ego_coef of
+ *                          positions < 3 * count then carry the bits of a call on the first count triples.
+ *   batch_total_dev int64[1] (device, nullable) the denominator read from the device instead of batch_total
  * ------------------------------------------------------------------------------------------ */
 /* Scatter plan: the 3B (row, entry) keys of a batch sorted by row, uint64[3B] (device).  Depends on
  * the indices only -- build it on a side stream while the forward propagation runs. */
 size_t cgx_bpr_plan_workspace_bytes(int64_t batch);
 int cgx_bpr_plan(const int64_t* users, const int64_t* pos, const int64_t* neg, int64_t batch,
                  int32_t num_users, int32_t num_items, uint64_t* plan,
-                 void* workspace, size_t workspace_bytes, void* stream);
+                 void* workspace, size_t workspace_bytes, void* stream, const int64_t* count);
 size_t cgx_bpr_workspace_bytes(int64_t batch, int32_t num_users, int32_t num_items);
 int cgx_bpr_fwd_bwd(const int64_t* users, const int64_t* pos, const int64_t* neg, int64_t batch,
                     int64_t batch_total, const uint64_t* plan, int32_t num_users, int32_t num_items, int32_t d,
@@ -306,7 +314,8 @@ int cgx_bpr_fwd_bwd(const int64_t* users, const int64_t* pos, const int64_t* neg
                     const float* pop, float reg_weight, float fair_weight,
                     float* loss_out, float* g_u, float* g_i,
                     int32_t* ego_rows, float* ego_coef,
-                    void* workspace, size_t workspace_bytes, void* stream);
+                    void* workspace, size_t workspace_bytes, void* stream, const int64_t* count,
+                    const int64_t* batch_total_dev);
 int cgx_bpr_apply_ego(const int32_t* ego_rows, const float* ego_coef, int64_t n_entries,
                       int32_t num_users, int32_t d, const float* e0_u, const float* e0_i,
                       float* d_e0_u, float* d_e0_i, void* stream);
@@ -340,13 +349,27 @@ int cgx_sampler_build(const int32_t* deg_i, int32_t num_items, double gamma,
  * mix_pop < 0 selects the uniform sampler of CU:295-299 (tables may then be NULL).
  * After max_tries rejected proposals the kernel falls back to uniform proposals (V2:373-376).
  * offset_dev (nullable): device counter added to `offset`, so that a captured CUDA graph draws new
- * triples on every replay (advance it with cgx_tick). */
+ * triples on every replay (advance it with cgx_tick).
+ * slots int64[batch] (nullable): entry k draws the stream of batch slot slots[k] instead of k -- a rank holding
+ * part of a batch (cgx_batch_select) then draws the triples a whole-batch call draws for the same users.
+ * count int64[1] (device, nullable): entries k >= *count are absent: nothing is read or written for them. */
 int cgx_sample_triples(const int64_t* users, int64_t batch, const int64_t* samp_indptr,
                        const int32_t* samp_idx, int32_t num_items,
                        const int32_t* items_by_deg, const int32_t* class_start,
                        const float* class_prob, const int32_t* class_alias, const int32_t* n_classes,
                        float mix_pop, int32_t max_tries, uint64_t seed, uint64_t offset,
-                       const uint64_t* offset_dev, int64_t* pos_out, int64_t* neg_out, void* stream);
+                       const uint64_t* offset_dev, int64_t* pos_out, int64_t* neg_out, void* stream,
+                       const int64_t* slots, const int64_t* count);
+
+/* Batch selection of a user-sharded epoch (run inside the captured step, one CTA): global batch s = *step is
+ * perm[s * batch, min((s + 1) * batch, n_train)) of the epoch's permutation perm int64[n_train] of global user ids.
+ * users_out int64[batch] receives, in batch order, the entries with lo <= user < hi rebased to local ids (user - lo),
+ * slots_out int64[batch] their positions in the global batch, count_out int64[1] how many there are, total_out
+ * int64[1] the size of global batch s (batch except in the tail batch; 0 past the epoch).  Entries past the count
+ * are not written.  batch <= 4096.  step is read, not advanced (cgx_tick). */
+int cgx_batch_select(const int64_t* perm, int64_t n_train, const uint64_t* step, int64_t batch, int64_t lo,
+                     int64_t hi, int64_t* users_out, int64_t* slots_out, int64_t* count_out, int64_t* total_out,
+                     void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Optimiser.  Replaces torch.optim.Adam(lr).step() (CU:587,652; V2:793,863; torch defaults) on the two
@@ -447,10 +470,13 @@ int cgx_score_candidates(const int64_t* users, const int64_t* cand, int64_t n_us
 
 /* Candidate lists of the sampled protocol drawn on device (CU:505-521): cand int64[n, 1 + n_neg]; column 0
  * is one of the user's test items (uniform), the others are uniform items outside test U train (rejection by
- * binary search in both sorted rows).  users must each own >= 1 test item.  Philox streams per (user, slot). */
+ * binary search in both sorted rows).  users must each own >= 1 test item.  Philox streams per (row, slot); row
+ * r of this call is row row_base + r of the streams, so that the rows of one shard get the lists a whole-list
+ * call gives the same rows. */
 int cgx_eval_candidates(const int64_t* users, int64_t n_users, const int64_t* train_indptr,
                         const int32_t* train_idx, const int64_t* test_indptr, const int32_t* test_idx,
-                        int32_t num_items, int32_t n_neg, uint64_t seed, int64_t* cand, void* stream);
+                        int32_t num_items, int32_t n_neg, uint64_t seed, int64_t* cand, void* stream,
+                        int64_t row_base);
 
 /* ranked[r] = cand[r] reordered by descending score, ties keeping candidate order (np.argsort(-scores),
  * CU:527, made stable). */
